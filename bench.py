@@ -59,7 +59,10 @@ def parse():
                                                          "the path a C++ host takes; --clouds is per GPU; timed by wall clock (the member GPUs run on their own streams)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-sample-clouds", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (rank 0) as DIR/<name>.npy, float64")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
     if args.graph < 0:
         args.graph = 1 if args.workload in ("table1", "grid512", "approach") else 0
     return args
@@ -92,6 +95,23 @@ def workload_config(args):
     if args.workload == "grid512":  # BASELINE.json configs[3]
         return dict(grid=512, rmax=190, step=15, area=(362.0, 362.0), r=2.56, n_clouds=1, n_points=1000000)
     return dict(grid=56, rmax=190, step=15, area=(32.0, 44.0), r=0.28, n_clouds=1, n_points=0)
+
+
+def dump_outputs(out_dir, arrays):
+    """one DIR/<name>.npy per array, float64 (exact for the int32 and float32 fields the library returns)"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
+
+
+# the answer fields of haf_best (n_guard / reserved describe how the answer was computed, not the answer)
+BEST_FIELDS = ("row", "col", "roll", "tilt", "approach_idx", "topval", "eval", "roll_rad", "M", "rolls_done", "n_windows_scored")
+
+
+def best_arrays(best):
+    """haf_best records of a batch -> {best_<field>: [n_clouds] or [n_clouds, 16] array}"""
+    return {"best_" + f: [list(getattr(b, f)) if f == "M" else getattr(b, f) for b in best] for f in BEST_FIELDS}
 
 
 def make_clouds(args, wc, rank):
@@ -313,8 +333,11 @@ def run_approach(args):
             return res["per_roll_top"][0][rb:re]
         return evaluate
 
+    last = {}
+
     def step(buf):
-        return hd.sharded_goal_search(evaluate_on(buf), A, R, [0] * A, [119] * A, rank, world)
+        last["result"] = hd.sharded_goal_search(evaluate_on(buf), A, R, [0] * A, [119] * A, rank, world)
+        return last["result"]
 
     ref = gs.search(dev, [h.make_request(area=wc["area"], approach=a) for a in approaches], outputs=False)
     per, overall, tops = step(dev)
@@ -354,6 +377,9 @@ def run_approach(args):
     ms_dev, w_dev = timed(dev, args.steps)
     launches = gs.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else {}
+    if args.dump_outputs and rank == 0:
+        per, overall, tops = last["result"]
+        dump_outputs(args.dump_outputs, {"per_request_best": per, "overall_best": overall, "unit_tops": tops})
     for _ in range(3):          # the host-memory path has its own staging buffer (and, with graphs on, its own captures)
         step(host.numpy())
     ms_e2e, w_e2e = timed(host.numpy(), args.steps)
@@ -440,12 +466,15 @@ def run_ours(args):
     rec_dev = torch.zeros((n_clouds, 8), dtype=torch.int32, device="cuda")
     gathered = torch.zeros((world * n_clouds, 8), dtype=torch.int32, device="cuda") if world > 1 else None
 
+    last = {}
+
     def step(buf):
         best = gs.search_batch_packed(buf, offsets, rq)
         if world > 1:
             gs.pack_best_records(best, rec_host)
             rec_dev.copy_(rec_host, non_blocking=True)
             dist.all_gather_into_tensor(gathered, rec_dev)
+        last["best"] = best
         return best
 
     def timed(buf, steps):
@@ -493,6 +522,8 @@ def run_ours(args):
     sampler.mark_begin()
     ms_dev, wall_dev, acc = timed(dev, args.steps)
     clocks = sampler.stop() if rank == 0 else {}
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, best_arrays(last["best"]))
     graph_replays = int(gs.timing().graph_replays)
     accs, ms_dev_prof = acc, ms_dev      # where the stage times come from
     if not prof_in_timed:

@@ -10,7 +10,6 @@ if ROOT not in sys.path:
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 FEATURES = os.path.join(GOLDEN, "refdata", "Features.txt")
 RANGE = os.path.join(GOLDEN, "refdata", "range21062012_allfeatures")
-REFERENCE_DATA = "/root/reference/data"
 
 
 def pytest_configure(config):

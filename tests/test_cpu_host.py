@@ -10,7 +10,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from conftest import FEATURES, GOLDEN, RANGE, REFERENCE_DATA, ROOT
+from conftest import FEATURES, GOLDEN, RANGE, ROOT
 
 
 def test_decimal_round_emulation_matches_glibc(tmp_path):
@@ -113,17 +113,21 @@ def test_best_key_orders_like_the_reference_rule():
     assert L.haf_best_key(-1000, 0) < L.haf_best_key(0, 100)
 
 
-def test_pcd_reader_on_reference_files():
-    if not os.path.isdir(REFERENCE_DATA):
-        pytest.skip("reference data not on this box")
+def _reference_pcd_file(tmp_path, name):
+    """one of the reference's bundled PCD files, written back from its committed bytes (tests/golden/pcd_files.npz)"""
+    path = tmp_path / (name + ".pcd")
+    path.write_bytes(np.load(os.path.join(GOLDEN, "pcd_files.npz"))[name].tobytes())
+    return str(path)
+
+
+def test_pcd_reader_on_reference_files(tmp_path):
     from haf_grasping_b200.pcd import read_pcd
     clouds = np.load(os.path.join(GOLDEN, "clouds.npz"))
-    a = read_pcd(os.path.join(REFERENCE_DATA, "pcd4.pcd"))
+    a = read_pcd(_reference_pcd_file(tmp_path, "pcd4"))
     assert a.shape == (200, 3)  # POINTS 200 although the file carries 208 lines
     assert a.tobytes() == clouds["pcd4"].tobytes()
-    t = read_pcd(os.path.join(REFERENCE_DATA, "table1_mult_obj_rcs_1428580506606673.pcd"))
+    t = read_pcd(_reference_pcd_file(tmp_path, "table1"))
     assert t.tobytes() == clouds["table1"].tobytes()
-    assert os.path.islink(os.path.join(REFERENCE_DATA, "objects_1.pcd"))
 
 
 def test_pcd_roundtrip_formats(tmp_path):
@@ -218,12 +222,11 @@ def test_cpp_pcd_reader_all_formats(tmp_path):
         assert py.tobytes() == pts.tobytes(), name
         out = subprocess.run([cli, "--pcd", str(f), "--dump-pcd"], capture_output=True, text=True, check=True).stdout.split()
         assert int(out[0]) == 53 and int(out[1]) == _fnv1a(pts.tobytes()), name
-    if os.path.isdir(REFERENCE_DATA):
-        for name in ("pcd5.pcd", "table2_mult_obj_rcs_1428580941635676.pcd"):
-            path = os.path.join(REFERENCE_DATA, name)
-            out = subprocess.run([cli, "--pcd", path, "--dump-pcd"], capture_output=True, text=True, check=True).stdout.split()
-            py = read_pcd(path)
-            assert int(out[0]) == len(py) and int(out[1]) == _fnv1a(py.tobytes())
+    for name in ("pcd5", "table2"):
+        path = _reference_pcd_file(tmp_path, name)
+        out = subprocess.run([cli, "--pcd", path, "--dump-pcd"], capture_output=True, text=True, check=True).stdout.split()
+        py = read_pcd(path)
+        assert int(out[0]) == len(py) and int(out[1]) == _fnv1a(py.tobytes())
 
 
 def test_bench_stage_roofline_and_clock_sampler_parsing(tmp_path):
@@ -259,3 +262,20 @@ def test_bench_stage_roofline_and_clock_sampler_parsing(tmp_path):
     s.t_begin = now - 1.0
     out = s.stop()
     assert out["samples"] == 2 and out["sm_mhz"] == 1850.0 and out["reasons"] == ["sw_power_cap"] and out["window"] == "timed region"
+
+
+def test_bench_dump_outputs_writes_every_answer_field_of_the_batch_records(tmp_path):
+    """bench.py --dump-outputs: one float64 .npy per answer field of the haf_best records, values exact."""
+    import importlib.util
+    from haf_grasping_b200 import api
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    b = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(b)
+    best = (api.haf_best * 3)()
+    best[1].row, best[2].topval, best[0].roll_rad, best[2].M[3] = 7, -1000, np.float32(0.1), 0.5
+    b.dump_outputs(str(tmp_path / "out"), b.best_arrays(best))
+    assert sorted(os.listdir(tmp_path / "out")) == sorted("best_%s.npy" % f for f in b.BEST_FIELDS)
+    load = lambda f: np.load(tmp_path / "out" / ("best_%s.npy" % f))  # noqa: E731
+    assert all(load(f).dtype == np.float64 for f in b.BEST_FIELDS)
+    assert load("row").tolist() == [0, 7, 0] and load("topval").tolist() == [0, 0, -1000]
+    assert load("roll_rad")[0] == np.float32(0.1) and load("M").shape == (3, 16) and load("M")[2, 3] == 0.5

@@ -1,7 +1,9 @@
 """libsvm front ends (SURVEY 8f-3): svm-scale-b200 / svm-predict-b200 and the haf_svm_* / haf_scale_* C ABI they bind.
 
 Parity here is pinned against the REFERENCE'S OWN PROGRAMS: oracle/_ref/svm-scale and oracle/_ref/svm-predict are
-libsvm-3.12 compiled unmodified from /root/reference; the GPU tests compare output files byte for byte.
+libsvm-3.12 compiled unmodified from the reference's sources; the GPU tests compare output files byte for byte.  Where
+oracle/_ref is not built, the GPU tests compare with the restatements of tests/libsvm_programs.py instead, pinned first to
+the committed outputs of those programs (tests/golden/svm_cli).
 """
 import os
 import subprocess
@@ -9,6 +11,7 @@ import subprocess
 import numpy as np
 import pytest
 
+import libsvm_programs
 from conftest import FEATURES, RANGE, ROOT
 
 LIBDIR = os.path.join(ROOT, "haf_grasping_b200", "lib")
@@ -156,10 +159,11 @@ def test_front_ends_reproduce_the_committed_reference_outputs(tools, tmp_path, t
 # ---------------------------------------------------------------- GPU: byte-exact against the reference's programs
 @pytest.fixture(scope="module")
 def roll_files(oracle_lib, tmp_path_factory, tmp_models):
-    """/tmp/features.txt of one roll of pcd2 written by the reference's own feature class, plus the reference programs'
-    outputs for the trained and the synthetic model."""
+    """/tmp/features.txt of roll 3 of pcd2 as the reference's feature class writes it ("-1 k:%.4g ..."), and the file
+    svm-scale -r makes of it ("%g" of every non-zero value, a blank after each pair), both written from the oracle's
+    values.  Their first 20 rows must equal the committed output of the reference's own class and svm-scale
+    (tests/golden/svm_cli); the rest rely on the oracle's text pinned by test_oracle_vs_ref.py."""
     import gzip
-    _ref_bins(oracle_lib)
     from conftest import GOLDEN
     wd = tmp_path_factory.mktemp("rollfiles")
     trained = str(wd / "trained.model")
@@ -168,10 +172,43 @@ def roll_files(oracle_lib, tmp_path_factory, tmp_models):
     clouds = np.load(os.path.join(GOLDEN, "clouds.npz"))
     o = oracle_lib.Oracle(FEATURES, RANGE, trained)
     ores = o.search(clouds["pcd2"], oracle_lib.make_request())
-    ref = oracle_lib.Ref(FEATURES, RANGE, trained)
-    ref.roll_file_exact(ores["integral"][3], ores["mask"][3], workdir=str(wd))
-    return {"dir": wd, "features": str(wd / "features.txt"), "scaled": str(wd / "features.txt.scale"),
-            "out_trained": str(wd / "output_calc_gp.txt"), "trained": trained, "synth": tmp_models(256)}
+    feats, _ = o.calc_featurevectors(ores["integral"][3], ores["mask"][3])
+    rows = ["-1" + "".join(" %d:%.4g" % (k + 1, v) for k, v in enumerate(f)) + "\n" for f in feats]
+    scaled = ["-1 " + "".join("%d:%g " % (k + 1, v) for k, v in enumerate(s) if v != 0) + "\n" for s in o.scale(feats)]
+    for lines, committed in ((rows, "features.txt"), (scaled, "scaled_ref.txt")):
+        with open(os.path.join(GOLDEN_CLI, committed)) as fh:
+            assert "".join(lines[:20]) == fh.read(), committed
+    files = {"features": str(wd / "features.txt"), "scaled": str(wd / "features.txt.scale")}
+    for key, lines in (("features", rows), ("scaled", scaled)):
+        with open(files[key], "w") as fh:
+            fh.write("".join(lines))
+    return dict(files, dir=wd, trained=trained, synth=tmp_models(256))
+
+
+@pytest.fixture(scope="module")
+def programs(oracle_lib, roll_files, tmp_path_factory):
+    """(scale_fit(args, src, range_out) -> (stdout, stderr), predict(src, model, out) -> (returncode, stdout, stderr)):
+    the reference's own svm-scale / svm-predict where oracle/_ref holds them, else the restatements, pinned first to the
+    committed outputs of the reference programs"""
+    if not oracle_lib.ref_available():
+        libsvm_programs.check_against_committed_outputs(oracle_lib, {k: roll_files[k] for k in ("trained", "synth")},
+                                                        tmp_path_factory.mktemp("restated"))
+        return libsvm_programs.svm_scale_fit, lambda src, model, out: libsvm_programs.svm_predict(src, model, out, oracle_lib)
+    ref_scale, ref_predict = _ref_bins(oracle_lib)
+
+    def scale_fit(args, src, range_out):
+        r = subprocess.run([ref_scale] + args + ["-s", range_out, src], capture_output=True, check=True)
+        return r.stdout, r.stderr
+
+    def predict(src, model, out):
+        r = subprocess.run([ref_predict, src, model, out], capture_output=True)
+        return r.returncode, r.stdout, r.stderr
+    return scale_fit, predict
+
+
+def test_restated_programs_reproduce_the_committed_reference_outputs(oracle_lib, tmp_path, tmp_models):
+    """the stand-ins of the reference programs (used where oracle/_ref is absent) print what the programs printed"""
+    libsvm_programs.check_against_committed_outputs(oracle_lib, _golden_models(tmp_path, tmp_models), tmp_path)
 
 
 @pytest.mark.gpu
@@ -184,10 +221,9 @@ def test_svm_scale_restore_mode_is_byte_identical_to_the_reference_program(tools
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("args", [[], ["-l", "0", "-u", "1"], ["-y", "-3", "5"], ["-l", "-2.5", "-u", "0.75", "-y", "0", "1"]])
-def test_svm_scale_fit_and_save_mode_matches_the_reference_program(tools, roll_files, oracle_lib, tmp_path, args):
+def test_svm_scale_fit_and_save_mode_matches_the_reference_program(tools, roll_files, programs, tmp_path, args):
     """No -r: min / max come from the data (pass 2 on the GPU, absent entries = 0); the saved range file and the scaled
     text must both equal the reference program's."""
-    ref_scale, _ = _ref_bins(oracle_lib)
     # a sparser, smaller file: drop every value with |v| < 0.02 and keep 60 rows -> absent entries matter
     rows = []
     for k, ln in enumerate(open(roll_files["features"]).read().split("\n")[:60]):
@@ -197,48 +233,47 @@ def test_svm_scale_fit_and_save_mode_matches_the_reference_program(tools, roll_f
         rows.append(" ".join([str(k % 3 - 1)] + [a for a in t[1:] if abs(float(a.split(":")[1])) >= 0.02]))
     src = tmp_path / "sparse.txt"
     src.write_text("\n".join(rows) + "\n")
-    a = subprocess.run([ref_scale] + args + ["-s", str(tmp_path / "ref.range"), str(src)], capture_output=True, check=True)
+    a_stdout, a_stderr = programs[0](args, str(src), str(tmp_path / "ref.range"))
     b = subprocess.run([tools[1]] + args + ["-s", str(tmp_path / "mine.range"), str(src)], capture_output=True, check=True)
     assert open(tmp_path / "ref.range", "rb").read() == open(tmp_path / "mine.range", "rb").read()
-    assert a.stdout == b.stdout
-    assert a.stderr == b.stderr     # the "#nonzeros" warning
+    assert a_stdout == b.stdout
+    assert a_stderr == b.stderr     # the "#nonzeros" warning
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("svm_mode", [0, 1, 2])
 @pytest.mark.parametrize("which", ["trained", "synth"])
-def test_svm_predict_output_file_is_byte_identical_to_the_reference_program(tools, roll_files, oracle_lib, tmp_path, svm_mode, which):
-    _, ref_predict = _ref_bins(oracle_lib)
+def test_svm_predict_output_file_is_byte_identical_to_the_reference_program(tools, roll_files, programs, tmp_path, svm_mode, which):
     model = roll_files[which]
     ref_out, my_out = tmp_path / "ref.out", tmp_path / "mine.out"
-    a = subprocess.run([ref_predict, roll_files["scaled"], model, str(ref_out)], capture_output=True, check=True)
+    a_rc, a_stdout, _ = programs[1](roll_files["scaled"], model, str(ref_out))
     b = subprocess.run([tools[0], "--svm-mode", str(svm_mode), roll_files["scaled"], model, str(my_out)], capture_output=True, check=True)
+    assert a_rc == 0
     assert open(ref_out, "rb").read() == open(my_out, "rb").read()
-    assert a.stdout == b.stdout     # "Accuracy = ...% (c/n) (classification)"
+    assert a_stdout == b.stdout     # "Accuracy = ...% (c/n) (classification)"
 
 
 @pytest.mark.gpu
-def test_svm_predict_stops_at_a_malformed_line_like_the_reference_program(tools, roll_files, oracle_lib, tmp_path):
-    _, ref_predict = _ref_bins(oracle_lib)
+def test_svm_predict_stops_at_a_malformed_line_like_the_reference_program(tools, roll_files, programs, tmp_path):
     lines = open(roll_files["scaled"]).read().split("\n")[:20]
     lines[12] = lines[12].replace(" 7:", " 7;")
     src = tmp_path / "broken.txt"
     src.write_text("\n".join(lines) + "\n")
-    a = subprocess.run([ref_predict, str(src), roll_files["synth"], str(tmp_path / "ref.out")], capture_output=True)
+    a_rc, _, a_stderr = programs[1](str(src), roll_files["synth"], str(tmp_path / "ref.out"))
     b = subprocess.run([tools[0], str(src), roll_files["synth"], str(tmp_path / "mine.out")], capture_output=True)
-    assert a.returncode == b.returncode == 1
-    assert a.stderr == b.stderr == b"Wrong input format at line 13\n"
+    assert a_rc == b.returncode == 1
+    assert a_stderr == b.stderr == b"Wrong input format at line 13\n"
     assert open(tmp_path / "ref.out", "rb").read() == open(tmp_path / "mine.out", "rb").read()
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("svm_mode,rtol", [(0, 1e-5), (1, 1e-13), (2, 1e-5)])
-def test_haf_svm_predict_decision_values_against_libsvm_in_process(roll_files, oracle_lib, svm_mode, rtol):
-    """C ABI: decision values of every row against svm_predict_values of the reference's own svm.cpp (oracle/_ref),
-    labels identical.  Includes rows wider than the model (indices beyond the model's largest) and an all-zero row."""
+def test_haf_svm_predict_decision_values_against_libsvm_in_process(roll_files, oracle_lib, programs, svm_mode, rtol):
+    """C ABI: decision values of every row against svm_predict_values of the reference's own svm.cpp (oracle/_ref; where
+    that is not built, the oracle's restatement of it, whose labels `programs` pinned to the committed outputs of the
+    reference's svm-predict), labels identical.  Includes rows wider than the model (indices beyond the model's largest)
+    and an all-zero row."""
     import haf_grasping_b200 as h
-    _ref_bins(oracle_lib)
-    ref = oracle_lib.Ref(FEATURES, RANGE, roll_files["trained"])
     rows = []
     for ln in open(roll_files["scaled"]).read().split("\n")[:150]:
         t = ln.split()
@@ -251,7 +286,12 @@ def test_haf_svm_predict_decision_values_against_libsvm_in_process(roll_files, o
     rows[5][:] = 0.0
     rows[6][327] = 0.125           # beyond the model's 323 dimensions: contributes x^2 to every distance (svm.cpp:356-364)
     x = np.array(rows)
-    want = [ref.svm_predict(r) for r in x]
+    if oracle_lib.ref_available():
+        ref = oracle_lib.Ref(FEATURES, RANGE, roll_files["trained"])
+        want = [ref.svm_predict(r) for r in x]
+    else:
+        dec, lab = oracle_lib.Oracle(FEATURES, RANGE, roll_files["trained"]).svm_decision(x)
+        want = list(zip(dec.tolist(), lab.tolist()))
     p = h.SvmPredictor(roll_files["trained"], svm_mode=svm_mode, min_dims=330)
     try:
         labels, dec = p.predict(x)
@@ -264,15 +304,14 @@ def test_haf_svm_predict_decision_values_against_libsvm_in_process(roll_files, o
 
 
 @pytest.mark.gpu
-def test_svm_predict_empty_file_and_rows_without_features(tools, roll_files, oracle_lib, tmp_path):
-    _, ref_predict = _ref_bins(oracle_lib)
+def test_svm_predict_empty_file_and_rows_without_features(tools, roll_files, programs, tmp_path):
     for name, text in (("empty.txt", ""), ("bare.txt", "1\n-1 \n+1 3:0.25\n")):
         src = tmp_path / name
         src.write_text(text)
-        a = subprocess.run([ref_predict, str(src), roll_files["synth"], str(tmp_path / "ref.out")], capture_output=True)
+        a_rc, a_stdout, _ = programs[1](str(src), roll_files["synth"], str(tmp_path / "ref.out"))
         b = subprocess.run([tools[0], str(src), roll_files["synth"], str(tmp_path / "mine.out")], capture_output=True)
-        assert a.returncode == b.returncode == 0
-        assert a.stdout == b.stdout
+        assert a_rc == b.returncode == 0
+        assert a_stdout == b.stdout
         assert open(tmp_path / "ref.out", "rb").read() == open(tmp_path / "mine.out", "rb").read()
 
 
