@@ -46,6 +46,18 @@ class haf_best(C.Structure):
         return (self.row, self.col, self.roll, self.tilt, self.topval)
 
 
+class haf_grasp(C.Structure):
+    """GraspOutput (msg/GraspOutput.msg) of one grasp plus the cell and roll it was built from (include/hafgpu.h)."""
+    _fields_ = [("eval", C.c_int), ("roll", C.c_float), ("graspPoint1", C.c_double * 3), ("graspPoint2", C.c_double * 3),
+                ("averagedGraspPoint", C.c_double * 3), ("approachVector", C.c_double * 3), ("row", C.c_int), ("col", C.c_int),
+                ("roll_index", C.c_int), ("reserved", C.c_int)]
+
+    def as_array(self) -> np.ndarray:
+        """the 13 doubles gp1 xyz, gp2 xyz, averaged xyz, approach xyz, roll (rad) -- the oracle's transform_gp_in_wcs order"""
+        return np.array(list(self.graspPoint1) + list(self.graspPoint2) + list(self.averagedGraspPoint) +
+                        list(self.approachVector) + [self.roll], np.float64)
+
+
 class haf_info(C.Structure):
     _fields_ = [("n_features", C.c_int), ("n_dims", C.c_int), ("n_sv", C.c_int), ("n_rolls", C.c_int), ("grid", C.c_int),
                 ("label0", C.c_int), ("label1", C.c_int), ("sm_count", C.c_int), ("gamma", C.c_double),
@@ -63,7 +75,7 @@ class haf_timing(C.Structure):
 
 EXPORTS = ["haf_create", "haf_destroy", "haf_last_error", "haf_get_info", "haf_set_stream", "haf_set_profiling",
            "haf_get_timing", "haf_launch_count", "haf_set_debug", "haf_search", "haf_search_batch", "haf_search_batch_packed",
-           "haf_build_transform", "haf_build_transform_wcs", "haf_best_key", "haf_pack_best_records", "haf_debug_window_count", "haf_debug_windows", "haf_debug_features",
+           "haf_search_grasps", "haf_search_batch_packed_grasps", "haf_build_transform", "haf_build_transform_wcs", "haf_best_key", "haf_pack_best_records", "haf_debug_window_count", "haf_debug_windows", "haf_debug_features",
            "haf_debug_decisions", "haf_debug_tensor_inputs", "haf_debug_integral", "haf_debug_cell_indices", "haf_debug_text_roundtrip", "haf_debug_tc_probe",
            "haf_version", "haf_pcd_decode", "haf_search_pcd", "haf_pointcloud2_to_xyz", "haf_debug_pcd_xyz", "haf_svm_create", "haf_svm_destroy", "haf_svm_predict", "haf_svm_predict_probability", "haf_svm_check_probability_model", "haf_scale_minmax", "haf_scale_apply"]
 
@@ -101,6 +113,10 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.haf_search.argtypes = [vp, vp, cs, cs, C.POINTER(haf_request), ci, C.POINTER(haf_best), C.POINTER(haf_best), vp, vp, vp, vp]
     L.haf_search_batch.argtypes = [vp, C.POINTER(vp), C.POINTER(cs), ci, C.POINTER(haf_request), C.POINTER(haf_best)]
     L.haf_search_batch_packed.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(haf_request), C.POINTER(haf_best)]
+    L.haf_search_grasps.argtypes = [vp, vp, cs, cs, C.POINTER(haf_request), ci, C.POINTER(haf_best), C.POINTER(haf_best), vp, vp, vp, vp,
+                                    C.POINTER(haf_grasp), C.POINTER(haf_grasp), C.POINTER(haf_grasp)]
+    L.haf_search_batch_packed_grasps.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(haf_request), C.POINTER(haf_best),
+                                                 C.POINTER(haf_grasp), C.POINTER(haf_grasp)]
     L.haf_build_transform.argtypes = [C.POINTER(haf_request), ci, ci, C.POINTER(C.c_float)]
     L.haf_build_transform_wcs.argtypes = [C.POINTER(haf_request), ci, ci, C.POINTER(C.c_float)]
     L.haf_best_key.argtypes = [ci, C.c_uint32]
@@ -235,6 +251,38 @@ class GraspSearch:
 
     def search(self, xyz, requests=None, n_points=None, stride_bytes=None, outputs=True):
         """xyz: numpy float32 [n,3] (host), or a torch CUDA tensor [n,3]/[n,4] (device pointer).  Returns a dict."""
+        xyz, reqs, nreq, n, stride, best, per, out = self._search_args(xyz, requests, n_points, stride_bytes, outputs)
+        self._check(self.L.haf_search(self.h, _ptr(xyz), n, stride, reqs, nreq, C.byref(best), per,
+                                      _ptr(out.get("graspseval")), _ptr(out.get("mask")), _ptr(out.get("heights")),
+                                      _ptr(out["per_roll_top"])))
+        out["best"] = best
+        out["best_per_request"] = list(per)
+        return out
+
+    def search_grasps(self, xyz, requests=None, per_roll=False, outputs=False, n_points=None, stride_bytes=None):
+        """``search`` plus the grasp poses computed on the device (haf_search_grasps): the dict also carries ``grasp`` (haf_grasp
+        of ``best``), ``grasp_per_request`` (list) and, with per_roll, ``grasp_per_roll`` ([n_requests][R] lists; only the
+        evaluated rolls are written).  per_roll may also be a ctypes array of n_requests * R haf_grasp records to fill in place."""
+        xyz, reqs, nreq, n, stride, best, per, out = self._search_args(xyz, requests, n_points, stride_bytes, outputs)
+        grasp = haf_grasp()
+        gper = (haf_grasp * nreq)()
+        groll = None
+        if per_roll is not False and per_roll is not None:
+            groll = per_roll if not isinstance(per_roll, bool) else (haf_grasp * (nreq * self.R))()
+            if len(groll) != nreq * self.R:
+                raise ValueError("per_roll needs n_requests * R = %d records" % (nreq * self.R))
+        self._check(self.L.haf_search_grasps(self.h, _ptr(xyz), n, stride, reqs, nreq, C.byref(best), per,
+                                             _ptr(out.get("graspseval")), _ptr(out.get("mask")), _ptr(out.get("heights")),
+                                             _ptr(out["per_roll_top"]), C.byref(grasp), gper, groll))
+        out["best"] = best
+        out["best_per_request"] = list(per)
+        out["grasp"] = grasp
+        out["grasp_per_request"] = list(gper)
+        if groll is not None:
+            out["grasp_per_roll"] = [list(groll[a * self.R:(a + 1) * self.R]) for a in range(nreq)]
+        return out
+
+    def _search_args(self, xyz, requests, n_points, stride_bytes, outputs):
         if requests is None:
             requests = [make_request()]
         if isinstance(requests, haf_request):
@@ -257,12 +305,7 @@ class GraspSearch:
             out["mask"] = np.zeros((nreq, R, G, G), np.uint8)
             out["heights"] = np.zeros((nreq, R, G, G), np.float32)
         out["per_roll_top"] = np.full((nreq, R, 3), -1, np.int32)
-        self._check(self.L.haf_search(self.h, _ptr(xyz), n, stride, reqs, nreq, C.byref(best), per,
-                                      _ptr(out.get("graspseval")), _ptr(out.get("mask")), _ptr(out.get("heights")),
-                                      _ptr(out["per_roll_top"])))
-        out["best"] = best
-        out["best_per_request"] = list(per)
-        return out
+        return xyz, reqs, nreq, n, stride, best, per, out
 
     def search_batch_packed(self, xyz_all, point_offsets, request=None):
         """xyz_all: packed float32 [N,3] host array or CUDA tensor; point_offsets: n_clouds+1 ints."""
@@ -274,6 +317,28 @@ class GraspSearch:
             xyz_all = np.ascontiguousarray(xyz_all, np.float32)
         self._check(self.L.haf_search_batch_packed(self.h, _ptr(xyz_all), off, n_clouds, C.byref(rq), best))
         return best
+
+    def search_batch_packed_grasps(self, xyz_all, point_offsets, request=None, per_roll=False):
+        """``search_batch_packed`` plus one grasp pose per cloud (haf_search_batch_packed_grasps).  Returns a dict: ``best``
+        (haf_best array), ``grasp`` (haf_grasp array, one per cloud) and, with per_roll, ``grasp_per_roll`` (haf_grasp array
+        [n_clouds * R], evaluated rolls only; per_roll may also be such an array to fill in place)."""
+        rq = request or make_request()
+        off = (C.c_size_t * len(point_offsets))(*[int(o) for o in point_offsets])
+        n_clouds = len(point_offsets) - 1
+        best = (haf_best * n_clouds)()
+        grasp = (haf_grasp * n_clouds)()
+        groll = None
+        if per_roll is not False and per_roll is not None:
+            groll = per_roll if not isinstance(per_roll, bool) else (haf_grasp * (n_clouds * self.R))()
+            if len(groll) != n_clouds * self.R:
+                raise ValueError("per_roll needs n_clouds * R = %d records" % (n_clouds * self.R))
+        if isinstance(xyz_all, np.ndarray):
+            xyz_all = np.ascontiguousarray(xyz_all, np.float32)
+        self._check(self.L.haf_search_batch_packed_grasps(self.h, _ptr(xyz_all), off, n_clouds, C.byref(rq), best, grasp, groll))
+        out = {"best": best, "grasp": grasp}
+        if groll is not None:
+            out["grasp_per_roll"] = groll
+        return out
 
     def pack_best_records(self, best, out):
         """haf_best array of a batch -> int32 [n, 8] records (topval, row, col, roll, tilt, approach_idx, n_windows, rolls_done)

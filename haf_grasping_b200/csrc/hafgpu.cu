@@ -211,6 +211,12 @@ struct haf_ctx {
     PinBuf<float> h_out_evals, h_out_heights;   // per-roll outputs asked for in HOST memory go through pinned staging (graph-capturable)
     PinBuf<unsigned char> h_out_mask;
 
+    // grasp poses (haf_search_grasps / haf_search_batch_packed_grasps, kernels.cuh a16): 0 = not asked for (no pose kernel runs),
+    // 1 = one record per job, 2 = the record of every unit comes back to the host as well.  Set for one call by GraspScope.
+    int grasp_mode = 0;
+    DevBuf<GraspRec> d_unit_grasp;       // [U] written chunk by chunk (outlives the per-chunk buffers)
+    PinBuf<GraspRec> h_unit_grasp, h_job_grasp;   // h_job_grasp [n_jobs] is written by grasp_gather_kernel itself (UVA)
+
     // probability estimates (SURVEY 8f-4): the model's sigmoid (svm.cpp:2811-2824); probability calls evaluate EVERY row /
     // window on the FP64 exact-order path (force_exact), whatever svm_mode the context was made with
     bool has_prob = false, force_exact = false;
@@ -996,6 +1002,7 @@ extern "C" void haf_destroy(haf_ctx* ctx) {
     for (size_t i = 0; i < ctx->graphs.size(); i++) cudaGraphExecDestroy(ctx->graphs[i].exec);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
     ctx->h_out_evals.release(); ctx->h_out_heights.release(); ctx->h_out_mask.release(); ctx->h_ring.release();
+    ctx->d_unit_grasp.release(); ctx->h_unit_grasp.release(); ctx->h_job_grasp.release();
     if (ctx->ev_ok) for (int i = 0; i < 10; i++) cudaEventDestroy(ctx->ev[i]);
     for (size_t i = 0; i < ctx->ev_pool.size(); i++) cudaEventDestroy(ctx->ev_pool[i]);
     for (size_t i = 0; i < ctx->copy_ev.size(); i++) cudaEventDestroy(ctx->copy_ev[i]);
@@ -1037,7 +1044,7 @@ extern "C" int haf_build_transform(const haf_request* req, int roll, int roll_st
 }
 extern "C" int haf_build_transform_wcs(const haf_request* req, int roll, int roll_step_deg, float M[16]) {
     if (!req || !M) return HAF_ERR_ARG;
-    hafhost::build_transform(*req, roll, roll_step_deg > 0 ? roll_step_deg : 15, M, true);
+    hafhost::build_transform_wcs(*req, roll, roll_step_deg > 0 ? roll_step_deg : 15, M);
     return HAF_OK;
 }
 // the 32-byte record of the cross-GPU best-grasp exchange (SURVEY 8e), straight from the haf_best structs of a batch
@@ -1273,11 +1280,21 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     const size_t bytes_units = (size_t)U * sizeof(UnitParams), bytes_jobs = (size_t)n_jobs * sizeof(JobParams);
     const size_t bytes_off = (size_t)(n_clouds + 1) * sizeof(long long), bytes_ub = (size_t)(n_clouds + 1) * sizeof(int);
     const size_t o_units = 0, o_jobs = round_up(o_units + bytes_units, 256), o_off = round_up(o_jobs + bytes_jobs, 256), o_ub = round_up(o_off + bytes_off, 256);
-    ENSURE(ctx, ctx->h_stage, o_ub + bytes_ub + 16);
+    // grasp poses: the inverse WCS matrices per (distinct request, roll) and each job's request index, after the block above
+    const bool grasp = ctx->grasp_mode > 0;
+    int n_pose_sets = 0;
+    if (grasp)
+        for (int j = 0; j < n_jobs; j++)
+            if (j == 0 || memcmp(&jobs[j - 1].rq, &jobs[j].rq, sizeof(haf_request)) != 0) n_pose_sets++;
+    const size_t o_jpose = round_up(o_ub + bytes_ub, 256), o_pose = round_up(o_jpose + (grasp ? (size_t)n_jobs * sizeof(int) : 0), 256);
+    const size_t bytes_block = grasp ? o_pose + (size_t)n_pose_sets * R * sizeof(UnitPose) : o_ub + bytes_ub;
+    ENSURE(ctx, ctx->h_stage, bytes_block + 16);
     UnitParams* hu = reinterpret_cast<UnitParams*>(ctx->h_stage.p + o_units);
     JobParams* hj = reinterpret_cast<JobParams*>(ctx->h_stage.p + o_jobs);
     long long* hoff = reinterpret_cast<long long*>(ctx->h_stage.p + o_off);
     int* hub = reinterpret_cast<int*>(ctx->h_stage.p + o_ub);
+    int* hjpose = reinterpret_cast<int*>(ctx->h_stage.p + o_jpose);
+    UnitPose* hpose = reinterpret_cast<UnitPose*>(ctx->h_stage.p + o_pose);
     long long max_points = 0;
     for (int c = 0; c <= n_clouds; c++) hoff[c] = cs.off[c];
     for (int c = 0; c < n_clouds; c++) max_points = std::max(max_points, cs.off[c + 1] - cs.off[c]);
@@ -1301,6 +1318,16 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
         // a batch applies ONE request to every cloud: the transforms and mask constants (host libm, ~1 us per unit) are built
         // once and copied -- at 6144 units per bench step they were ~1 ms of GPU idle time at the head of every call
         const bool same_rq = j > 0 && memcmp(&jobs[j - 1].rq, &jb.rq, sizeof(haf_request)) == 0;
+        if (grasp) {   // transform_gp_in_wcs_and_publish's matrix (:1276-1334), inverted -- once per distinct request as well
+            const int p = same_rq ? hjpose[j - 1] : (j == 0 ? 0 : hjpose[j - 1] + 1);
+            hjpose[j] = p;
+            if (!same_rq)
+                for (int roll = 0; roll < R; roll++) {
+                    float Mw[16];
+                    hafhost::build_transform_wcs(jb.rq, roll, ctx->cfg.roll_step_deg, Mw);
+                    hafhost::invert4(Mw, hpose[(size_t)p * R + roll].Minv);
+                }
+        }
         for (int roll = 0; roll < R; roll++) {
             UnitParams& up = hu[j * R + roll];
             if (same_rq) {
@@ -1365,7 +1392,11 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     if ((out_evals || out_mask || out_heights || keep_debug_state) && chunks.size() != 1)
         return ctx->fail(HAF_ERR_UNSUPPORTED, "per-roll outputs need the whole request in one chunk (windows x dims too large)");
 
-    ENSURE(ctx, ctx->d_params, o_ub + bytes_ub + 16); ENSURE(ctx, ctx->d_results, n_jobs); ENSURE(ctx, ctx->d_per_roll_top, (size_t)U * 3);
+    ENSURE(ctx, ctx->d_params, bytes_block + 16); ENSURE(ctx, ctx->d_results, n_jobs); ENSURE(ctx, ctx->d_per_roll_top, (size_t)U * 3);
+    if (grasp) {
+        ENSURE(ctx, ctx->d_unit_grasp, U); ENSURE(ctx, ctx->h_job_grasp, n_jobs);
+        if (ctx->grasp_mode > 1) ENSURE(ctx, ctx->h_unit_grasp, U);
+    }
     ENSURE(ctx, ctx->d_unit_block, (size_t)2 * U + (U + 1) / 2);
     unsigned long long* const d_unit_top = ctx->d_unit_block.p;
     unsigned long long* const d_unit_run = d_unit_top + U;
@@ -1415,7 +1446,9 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
         long long wsum_all = 0;
         for (int j = 0; j < n_jobs; j++) wsum_all += jobs[j].wbound;
         gkey.wcap = (size_t)wsum_all; gkey.pts_bucket = pts_bucket; gkey.n_jobs = n_jobs; gkey.n_clouds = n_clouds;
-        gkey.flags = (prob ? 1 : 0) | (keep_debug_state ? 2 : 0) | (avg_points_all >= 8 * (long long)GG ? 4 : 0) | (ctx->cfg.emulate_text_roundtrip ? 8 : 0);
+        // (grasp poses: the two pose kernels, the record copies and the size of the parameter block belong to the graph too)
+        gkey.flags = (prob ? 1 : 0) | (keep_debug_state ? 2 : 0) | (avg_points_all >= 8 * (long long)GG ? 4 : 0) | (ctx->cfg.emulate_text_roundtrip ? 8 : 0) |
+                     (ctx->grasp_mode << 4) | (n_pose_sets << 8);
         gkey.tc_passes = ctx->tc_passes; gkey.o_evals = dst_evals; gkey.o_mask = dst_mask; gkey.o_heights = dst_heights; gkey.rolls_hash = hsh; gkey.st = st;
         for (size_t i = 0; i < ctx->graphs.size() && gmode == 0; i++)
             if (ctx->graphs[i].key == gkey) { gmode = 2; graph_slot = (int)i; }
@@ -1443,7 +1476,7 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     // copy-engine memcpy: the H2D engine is a FIFO, and behind a large staging copy of clouds (this call's, or any other
     // stream's) a small memcpy would stall every kernel of the call until that copy has finished.
     {
-        const size_t n16 = (o_ub + bytes_ub + 15) / 16;
+        const size_t n16 = (bytes_block + 15) / 16;
         copy_params_kernel<<<(unsigned)std::min<size_t>((n16 + 255) / 256, 1024), 256, 0, st>>>(reinterpret_cast<const uint4*>(ctx->h_stage.p),
                                                                                               reinterpret_cast<uint4*>(ctx->d_params.p), n16);
         LAUNCHED(ctx);
@@ -1452,6 +1485,8 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     JobParams* const d_jobs = reinterpret_cast<JobParams*>(ctx->d_params.p + o_jobs);
     long long* const d_ptoff = reinterpret_cast<long long*>(ctx->d_params.p + o_off);
     int* const d_cloud_ubegin = reinterpret_cast<int*>(ctx->d_params.p + o_ub);
+    const int* const d_jpose = reinterpret_cast<const int*>(ctx->d_params.p + o_jpose);
+    const UnitPose* const d_pose = reinterpret_cast<const UnitPose*>(ctx->d_params.p + o_pose);
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_unit_block.p, 0, ((size_t)2 * U + (U + 1) / 2) * 8, st));
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_counters.p, 0, 64 * 4, st));
     // host-staged batch in several chunks: chunks alternate between the call's stream and a second one (see haf_ctx::ChunkWs)
@@ -1625,6 +1660,11 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
         }
         tie_rule_kernel<<<dim3((G + 7) / 8, Uc), 256, 0, st>>>(ctx->d_evals.p, G, units_c, d_unit_top + ubase, d_unit_run + ubase);
         LAUNCHED(ctx);
+        if (grasp) {   // a16 per unit while this chunk's heights are still in d_keys (the next chunk of this set overwrites them)
+            grasp_unit_kernel<<<(Uc + 127) / 128, 128, 0, st>>>(ctx->d_keys.p, G, units_c, Uc, d_unit_top + ubase, d_unit_run + ubase, d_pose, d_jpose,
+                                                               R, ctx->cfg.roll_step_deg, ctx->d_unit_grasp.p + ubase);
+            LAUNCHED(ctx);
+        }
         if (prof) CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[ci * 8 + 7], st));
 
         // bookkeeping per chunk: window / guard counts accumulate on the device ([8] windows, [9] guard), no host sync
@@ -1658,6 +1698,14 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     reduce_rolls_kernel<<<(n_jobs + 127) / 128, 128, 0, st>>>(d_unit_top, d_unit_run, d_unit_windows, d_jobs, n_jobs, R, G,
                                                              ctx->d_per_roll_top.p, ctx->d_results.p);
     LAUNCHED(ctx);
+    if (grasp) {   // a16 per job: the winning unit's record (or the roll -1 pose), written straight into pinned host memory (a
+                   // copy node less on a single goal's critical path; the stream synchronise below makes it visible)
+        grasp_gather_kernel<<<(n_jobs + 127) / 128, 128, 0, st>>>(ctx->d_results.p, n_jobs, d_units, d_pose, d_jpose, R, G, ctx->cfg.roll_step_deg,
+                                                                 ctx->d_unit_grasp.p, ctx->h_job_grasp.p);
+        LAUNCHED(ctx);
+        if (ctx->grasp_mode > 1)
+            CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_unit_grasp.p, ctx->d_unit_grasp.p, (size_t)U * sizeof(GraspRec), cudaMemcpyDeviceToHost, st));
+    }
     CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_results.p, ctx->d_results.p, (size_t)n_jobs * sizeof(JobResult), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_per_roll_top.p, ctx->d_per_roll_top.p, (size_t)U * 3 * sizeof(int), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_counters.p, ctx->d_counters.p, 16 * 4, cudaMemcpyDeviceToHost, st));
@@ -1800,18 +1848,47 @@ static int stage_points(haf_ctx* ctx, const void* src, size_t bytes, bool* is_de
     return HAF_OK;
 }
 
+// grasp poses asked for by haf_search_grasps / haf_search_batch_packed_grasps: where the records go (host memory, NULL = not
+// wanted).  best: the overall winner's (single goals only); per_job [n_jobs]; per_roll [n_jobs][R], evaluated rolls only.
+// units: the per-unit records stay readable in ctx->h_unit_grasp after the call (members of a multi-GPU group).
+struct GraspOut {
+    haf_grasp* best = nullptr;
+    haf_grasp* per_job = nullptr;
+    haf_grasp* per_roll = nullptr;
+    bool units = false;
+};
+static_assert(sizeof(haf_grasp) == sizeof(GraspRec) && offsetof(haf_grasp, graspPoint1) == offsetof(GraspRec, gp1) &&
+              offsetof(haf_grasp, approachVector) == offsetof(GraspRec, approach) && offsetof(haf_grasp, row) == offsetof(GraspRec, row) &&
+              offsetof(haf_grasp, reserved) == offsetof(GraspRec, reserved), "haf_grasp and GraspRec must share their layout");
+// grasp_mode of the context for the length of one call
+struct GraspScope {
+    haf_ctx* c;
+    GraspScope(haf_ctx* ctx, const GraspOut* go) : c(ctx) { c->grasp_mode = go ? ((go->per_roll || go->units) ? 2 : 1) : 0; }
+    ~GraspScope() { c->grasp_mode = 0; }
+};
+// per-roll records of the evaluated rolls of each job: h_unit_grasp -> out [n_jobs][R] (the other rolls are left untouched)
+static void copy_roll_grasps(const haf_ctx* ctx, const std::vector<Job>& jobs, haf_grasp* out) {
+    const int R = ctx->R;
+    for (size_t j = 0; j < jobs.size(); j++)
+        if (jobs[j].n_rolls_active > jobs[j].roll_begin)
+            memcpy(out + j * R + jobs[j].roll_begin, ctx->h_unit_grasp.p + j * R + jobs[j].roll_begin,
+                   (size_t)(jobs[j].n_rolls_active - jobs[j].roll_begin) * sizeof(haf_grasp));
+}
+
 static int group_search(haf_ctx* ctx, const float* xyz, size_t n_points, size_t stride_bytes, const haf_request* reqs, int n_requests,
-                        haf_best* best, haf_best* best_per_request, float* graspseval, unsigned char* mask, float* heights, int* per_roll_top);
+                        haf_best* best, haf_best* best_per_request, float* graspseval, unsigned char* mask, float* heights, int* per_roll_top,
+                        const GraspOut* go = nullptr);
 static int group_batch_packed(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* req,
-                              haf_best* best_per_cloud);
+                              haf_best* best_per_cloud, const GraspOut* go = nullptr);
 static void group_timing(haf_ctx* ctx);
 
 // one GPU: the context itself (also what each member of a multi-GPU group runs -- group[0] IS the head context, so the
 // group entry points must never be re-entered from a member thread)
 static int search_single(haf_ctx* ctx, const float* xyz, size_t n_points, size_t stride_bytes, const haf_request* reqs, int n_requests,
-                         haf_best* best, haf_best* best_per_request, float* graspseval, unsigned char* mask, float* heights, int* per_roll_top);
+                         haf_best* best, haf_best* best_per_request, float* graspseval, unsigned char* mask, float* heights, int* per_roll_top,
+                         const GraspOut* go = nullptr);
 static int batch_packed_single(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* req,
-                               haf_best* best_per_cloud);
+                               haf_best* best_per_cloud, const GraspOut* go = nullptr);
 static int batch_single(haf_ctx* ctx, const float* const* clouds, const size_t* n_points, int n_clouds, const haf_request* req,
                         haf_best* best_per_cloud);
 
@@ -1822,8 +1899,20 @@ extern "C" int haf_search(haf_ctx* ctx, const float* xyz, size_t n_points, size_
         return group_search(ctx, xyz, n_points, stride_bytes, reqs, n_requests, best, best_per_request, graspseval, mask, heights, per_roll_top);
     return search_single(ctx, xyz, n_points, stride_bytes, reqs, n_requests, best, best_per_request, graspseval, mask, heights, per_roll_top);
 }
+extern "C" int haf_search_grasps(haf_ctx* ctx, const float* xyz, size_t n_points, size_t stride_bytes, const haf_request* reqs, int n_requests,
+                                 haf_best* best, haf_best* best_per_request, float* graspseval, unsigned char* mask, float* heights,
+                                 int* per_roll_top, haf_grasp* grasp, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll) {
+    if (!ctx) return HAF_ERR_ARG;
+    if (!grasp) return ctx->fail(HAF_ERR_ARG, "haf_search_grasps: grasp is required");
+    GraspOut go;
+    go.best = grasp; go.per_job = grasp_per_request; go.per_roll = grasp_per_roll;
+    if (ctx->group.size() > 1)
+        return group_search(ctx, xyz, n_points, stride_bytes, reqs, n_requests, best, best_per_request, graspseval, mask, heights, per_roll_top, &go);
+    return search_single(ctx, xyz, n_points, stride_bytes, reqs, n_requests, best, best_per_request, graspseval, mask, heights, per_roll_top, &go);
+}
 static int search_single(haf_ctx* ctx, const float* xyz, size_t n_points, size_t stride_bytes, const haf_request* reqs, int n_requests,
-                         haf_best* best, haf_best* best_per_request, float* graspseval, unsigned char* mask, float* heights, int* per_roll_top) {
+                         haf_best* best, haf_best* best_per_request, float* graspseval, unsigned char* mask, float* heights, int* per_roll_top,
+                         const GraspOut* go) {
     if (!reqs || n_requests < 1 || !best) return ctx->fail(HAF_ERR_ARG, "haf_search: reqs, n_requests >= 1 and best are required");
     if (n_points > 0 && !xyz) return ctx->fail(HAF_ERR_ARG, "haf_search: xyz is null");
     if (stride_bytes == 0) stride_bytes = 12;
@@ -1842,7 +1931,11 @@ static int search_single(haf_ctx* ctx, const float* xyz, size_t n_points, size_t
     cs.d_xyz = n_points == 0 ? nullptr : (dev ? reinterpret_cast<const unsigned char*>(xyz) : ctx->d_xyz.p);
     std::vector<Job> jobs(n_requests);
     for (int a = 0; a < n_requests; a++) { jobs[a].cloud = 0; jobs[a].rq = reqs[a]; }
-    int rc = run_jobs(ctx, cs, jobs, graspseval, mask, heights, true);
+    int rc;
+    {
+        GraspScope gs(ctx, go);
+        rc = run_jobs(ctx, cs, jobs, graspseval, mask, heights, true);
+    }
     if (rc) return rc;
     const int R = ctx->R;
     // overall winner over requests: strict >, earliest request wins ties (server.cpp:953 extended over approach vectors)
@@ -1864,6 +1957,11 @@ static int search_single(haf_ctx* ctx, const float* xyz, size_t n_points, size_t
         for (int a = 0; a < n_requests; a++) { nw += ctx->h_results.p[a].n_windows; rd += ctx->h_results.p[a].rolls_done; }
         best->n_windows_scored = (int)nw; best->rolls_done = rd;
     }
+    if (go) {   // no winner at all: request 0's roll -1 pose, like `best`
+        if (go->best) memcpy(go->best, ctx->h_job_grasp.p + (win < 0 ? 0 : win), sizeof(haf_grasp));
+        if (go->per_job) memcpy(go->per_job, ctx->h_job_grasp.p, (size_t)n_requests * sizeof(haf_grasp));
+        if (go->per_roll) copy_roll_grasps(ctx, jobs, go->per_roll);
+    }
     return HAF_OK;
 }
 
@@ -1873,8 +1971,17 @@ extern "C" int haf_search_batch_packed(haf_ctx* ctx, const float* xyz_all, const
     if (ctx->group.size() > 1) return group_batch_packed(ctx, xyz_all, point_offsets, n_clouds, req, best_per_cloud);
     return batch_packed_single(ctx, xyz_all, point_offsets, n_clouds, req, best_per_cloud);
 }
+extern "C" int haf_search_batch_packed_grasps(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* req,
+                                              haf_best* best_per_cloud, haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_roll) {
+    if (!ctx) return HAF_ERR_ARG;
+    if (!grasp_per_cloud) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_packed_grasps: grasp_per_cloud is required");
+    GraspOut go;
+    go.per_job = grasp_per_cloud; go.per_roll = grasp_per_roll;
+    if (ctx->group.size() > 1) return group_batch_packed(ctx, xyz_all, point_offsets, n_clouds, req, best_per_cloud, &go);
+    return batch_packed_single(ctx, xyz_all, point_offsets, n_clouds, req, best_per_cloud, &go);
+}
 static int batch_packed_single(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* req,
-                               haf_best* best_per_cloud) {
+                               haf_best* best_per_cloud, const GraspOut* go) {
     if (!point_offsets || n_clouds < 1 || !req || !best_per_cloud) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_packed: bad arguments");
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     ctx->last_valid = false;
@@ -1942,9 +2049,17 @@ static int batch_packed_single(haf_ctx* ctx, const float* xyz_all, const size_t*
     cs.d_xyz = total == 0 ? nullptr : (dev ? reinterpret_cast<const unsigned char*>(xyz_all) : ctx->d_xyz.p);
     std::vector<Job> jobs(n_clouds);
     for (int c = 0; c < n_clouds; c++) { jobs[c].cloud = c; jobs[c].rq = *req; }
-    int rc = run_jobs(ctx, cs, jobs, nullptr, nullptr, nullptr, ctx->debug_keep_batch);
+    int rc;
+    {
+        GraspScope gs(ctx, go);
+        rc = run_jobs(ctx, cs, jobs, nullptr, nullptr, nullptr, ctx->debug_keep_batch);
+    }
     ctx->copy_pieces = 0;
     if (rc) return rc;
+    if (go) {
+        if (go->per_job) memcpy(go->per_job, ctx->h_job_grasp.p, (size_t)n_clouds * sizeof(haf_grasp));
+        if (go->per_roll) copy_roll_grasps(ctx, jobs, go->per_roll);
+    }
     {   // one request for all clouds: the winning roll's transform is built once per roll, not once per cloud
         std::vector<haf_best> per_roll(ctx->R);
         std::vector<char> have(ctx->R, 0);
@@ -2174,7 +2289,8 @@ static void group_timing(haf_ctx* ctx) {
 // :953-960 (strict >, earliest roll, early exit when return_only_best), so best / rolls_done / n_windows_scored equal the
 // one-GPU result.  The only data that crosses GPUs is R x 3 ints per request.
 static int group_search(haf_ctx* ctx, const float* xyz, size_t n_points, size_t stride_bytes, const haf_request* reqs, int n_requests,
-                        haf_best* best, haf_best* best_per_request, float* graspseval, unsigned char* mask, float* heights, int* per_roll_top) {
+                        haf_best* best, haf_best* best_per_request, float* graspseval, unsigned char* mask, float* heights, int* per_roll_top,
+                        const GraspOut* go) {
     if (!reqs || n_requests < 1 || !best) return ctx->fail(HAF_ERR_ARG, "haf_search: reqs, n_requests >= 1 and best are required");
     const int n = (int)ctx->group.size(), R = ctx->R;
     if (stride_bytes == 0) stride_bytes = 12;
@@ -2187,16 +2303,24 @@ static int group_search(haf_ctx* ctx, const float* xyz, size_t n_points, size_t 
         ubeg[a + 1] = ubeg[a] + (re[a] - rb[a]);
     }
     const long long U = ubeg[n_requests];
+    // grasp poses with no roll to evaluate anywhere: no member would run, so the head builds the roll -1 poses on its own GPU
+    if (go && U == 0)
+        return search_single(ctx, xyz, n_points, stride_bytes, reqs, n_requests, best, best_per_request, graspseval, mask, heights, per_roll_top, go);
     std::vector<int> tops((size_t)n_requests * R * 3);
     std::vector<unsigned> uwin((size_t)n_requests * R, 0u);
     for (size_t u = 0; u < (size_t)n_requests * R; u++) { tops[3 * u] = -1; tops[3 * u + 1] = -1; tops[3 * u + 2] = -1000; }
+    // grasp poses: every member returns the records of its own units (and, for a request with no roll on it, the roll -1 pose)
+    std::vector<GraspRec> ugrasp(go ? (size_t)n_requests * R : 0), nograsp(go ? n_requests : 0);
     std::vector<int> rcs(n, HAF_OK);
     std::vector<long long> guards(n, 0);
     std::vector<std::thread> th;
+    int first_member = -1;
     for (int k = 0; k < n; k++) {
         const long long u0 = U * k / n, u1 = U * (k + 1) / n;   // this GPU's block of the active units
         if (u1 <= u0) { memset(&ctx->group[k]->timing, 0, sizeof(haf_timing)); continue; }
-        th.emplace_back([=, &rcs, &tops, &uwin, &guards, &rb, &re, &ubeg]() {
+        const bool report_nograsp = first_member < 0;   // one member reports the roll -1 poses
+        if (first_member < 0) first_member = k;
+        th.emplace_back([=, &rcs, &tops, &uwin, &guards, &rb, &re, &ubeg, &ugrasp, &nograsp]() {
             haf_ctx* m = ctx->group[k];
             std::vector<haf_request> rq(reqs, reqs + n_requests);
             for (int a = 0; a < n_requests; a++) {
@@ -2210,17 +2334,23 @@ static int group_search(haf_ctx* ctx, const float* xyz, size_t n_points, size_t 
             std::vector<int> local((size_t)n_requests * R * 3);
             haf_best b0;
             std::vector<haf_best> bpr(n_requests);
+            GraspOut mgo;
+            mgo.units = true;
             if (rc == HAF_OK)
-                rc = search_single(m, (const float*)use, n_points, stride_bytes, rq.data(), n_requests, &b0, bpr.data(), graspseval, mask, heights, local.data());
+                rc = search_single(m, (const float*)use, n_points, stride_bytes, rq.data(), n_requests, &b0, bpr.data(), graspseval, mask, heights, local.data(),
+                                   go ? &mgo : nullptr);
             rcs[k] = rc;
             if (rc != HAF_OK) return;
             guards[k] = m->timing.n_guard;
-            for (int a = 0; a < n_requests; a++)
+            for (int a = 0; a < n_requests; a++) {
                 for (int roll = rq[a].roll_begin; roll < (rq[a].roll_limit > 0 ? rq[a].roll_limit : 0); roll++) {
                     const size_t u = (size_t)a * R + roll;
                     tops[3 * u] = local[3 * u]; tops[3 * u + 1] = local[3 * u + 1]; tops[3 * u + 2] = local[3 * u + 2];
                     uwin[u] = m->h_unit_windows.p[u];
+                    if (go) ugrasp[u] = m->h_unit_grasp.p[u];
                 }
+                if (go && report_nograsp && re[a] <= rb[a]) nograsp[a] = m->h_job_grasp.p[a];   // this request has no roll anywhere
+            }
         });
     }
     for (size_t i = 0; i < th.size(); i++) th[i].join();
@@ -2248,6 +2378,18 @@ static int group_search(haf_ctx* ctx, const float* xyz, size_t n_points, size_t 
         if (best_per_request) fill_best(ctx, jobs[a], r, a, n_guard, &best_per_request[a]);
         if (r.topval > wtop) { wtop = r.topval; win = a; }
     }
+    if (go) {   // the winning unit's record from whichever member owns it; eval as the one-GPU gather sets it (:390)
+        std::vector<GraspRec> rec(n_requests);
+        for (int a = 0; a < n_requests; a++) {
+            rec[a] = res[a].roll >= 0 ? ugrasp[(size_t)a * R + res[a].roll] : nograsp[a];
+            rec[a].eval = res[a].topval - 20;
+        }
+        if (go->best) memcpy(go->best, &rec[win < 0 ? 0 : win], sizeof(haf_grasp));
+        if (go->per_job) memcpy(go->per_job, rec.data(), (size_t)n_requests * sizeof(haf_grasp));
+        if (go->per_roll)
+            for (int a = 0; a < n_requests; a++)
+                for (int roll = rb[a]; roll < re[a]; roll++) memcpy(go->per_roll + (size_t)a * R + roll, &ugrasp[(size_t)a * R + roll], sizeof(haf_grasp));
+    }
     if (per_roll_top) memcpy(per_roll_top, tops.data(), tops.size() * sizeof(int));
     if (win < 0) {
         JobResult none; memset(&none, 0, sizeof none);
@@ -2264,7 +2406,7 @@ static int group_search(haf_ctx* ctx, const float* xyz, size_t n_points, size_t 
 
 // Throughput mode: contiguous blocks of clouds per GPU, one host thread each, no cross-GPU data at all.
 static int group_batch_packed(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* req,
-                              haf_best* best_per_cloud) {
+                              haf_best* best_per_cloud, const GraspOut* go) {
     if (!point_offsets || n_clouds < 1 || !req || !best_per_cloud) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_packed: bad arguments");
     const int n = (int)ctx->group.size();
     std::vector<int> rcs(n, HAF_OK);
@@ -2278,8 +2420,10 @@ static int group_batch_packed(haf_ctx* ctx, const float* xyz_all, const size_t* 
             for (int c = c0; c <= c1; c++) off[c - c0] = point_offsets[c] - point_offsets[c0];
             const float* src = xyz_all + point_offsets[c0] * 3;
             const void* use = src;
+            GraspOut mgo;   // this member's clouds' records go straight to their place in the caller's arrays
+            if (go) { mgo.per_job = go->per_job + c0; mgo.per_roll = go->per_roll ? go->per_roll + (size_t)c0 * ctx->R : nullptr; }
             int rc = member_input(m, src, off[c1 - c0] * 12, &use);
-            if (rc == HAF_OK) rc = batch_packed_single(m, (const float*)use, off.data(), c1 - c0, req, best_per_cloud + c0);
+            if (rc == HAF_OK) rc = batch_packed_single(m, (const float*)use, off.data(), c1 - c0, req, best_per_cloud + c0, go ? &mgo : nullptr);
             rcs[k] = rc;
         });
     }

@@ -3,8 +3,8 @@
 // Same member names, same argument meaning, same result fields, so a maintainer can lift the bodies into the ROS
 // node (INTEGRATION.md) and the tests read like the reference's flow:
 //     read_pc_cb (goal -> members, :250-329)  ->  loop_control (:335-402)  ->  transform_gp_in_wcs_and_publish (:1274-1401)
-// Everything numeric on the hot path happens in libhafgpu (CUDA); this file only keeps the reference's bookkeeping
-// and the O(1) host numerics of the final grasp pose.
+// Everything numeric on the hot path happens in libhafgpu (CUDA), the grasp poses included; this file only keeps the
+// reference's bookkeeping.
 #pragma once
 #include <cmath>
 #include <cstring>
@@ -76,6 +76,7 @@ public:
         point_inside_box_grid.assign((size_t)R * G * G, 0);
         graspseval.assign((size_t)R * G * G, 0.0f);
         per_roll_top.assign((size_t)R * 3, -1);
+        grasp_per_roll_.resize(R);
     }
     ~CCalc_Grasppoints_B200() { haf_destroy(ctx_); }
     CCalc_Grasppoints_B200(const CCalc_Grasppoints_B200&) = delete;
@@ -110,7 +111,8 @@ public:
         loop_control(xyz, n_points, stride_bytes);
     }
 
-    // loop_control (:335-402): the five per-roll calls (:376-385) are ONE haf_search call
+    // loop_control (:335-402): the five per-roll calls (:376-385) and the grasp poses of transform_gp_in_wcs_and_publish
+    // (:1274-1401) are ONE haf_search_grasps call; the poses are computed on the device (haf_grasp records)
     void loop_control(const float* xyz, size_t n_points, size_t stride_bytes, int roll_limit = 0) {
         haf_request rq;
         memset(&rq, 0, sizeof rq);
@@ -121,8 +123,9 @@ public:
         rq.return_only_best = return_only_best_gp ? 1 : 0;
         rq.graspval_top = graspval_top;
         rq.roll_limit = roll_limit;
-        int rc = haf_search(ctx_, xyz, n_points, stride_bytes, &rq, 1, &best, NULL, graspseval.data(), point_inside_box_grid.data(),
-                            heightsgridroll.data(), per_roll_top.data());
+        haf_grasp grasp;
+        int rc = haf_search_grasps(ctx_, xyz, n_points, stride_bytes, &rq, 1, &best, NULL, graspseval.data(), point_inside_box_grid.data(),
+                                   heightsgridroll.data(), per_roll_top.data(), &grasp, NULL, grasp_per_roll_.data());
         if (rc != HAF_OK) throw std::runtime_error(std::string("hafgpu: ") + haf_last_error(ctx_));
         published_per_roll.clear();
         // av_trans_mat (:484) = generate_grid's matrix of the roll just evaluated; only its third row is read (:1370-1374), and
@@ -130,95 +133,34 @@ public:
         haf_build_transform(&rq, best.roll >= 0 ? best.roll : 0, step_deg_, av_trans_mat);
         for (int roll = 0; roll < best.rolls_done; roll++) {                      // what show_predicted_gps did per roll
             const int* t = &per_roll_top[roll * 3];
-            if (!return_only_best_gp && t[2] > graspval_th) {                      // :962-972
-                int scaled = t[2] - 20;
-                if (scaled < 10) scaled = 10;
-                published_per_roll.push_back(transform_gp_in_wcs_and_publish(t[0], t[1], roll, 0, scaled));
-            }
+            if (!return_only_best_gp && t[2] > graspval_th)                        // :962-972 (eval = max(top - 20, 10) in the record)
+                published_per_roll.push_back(to_grasp_output(grasp_per_roll_[roll]));
         }
         id_row_top_overall = best.row; id_col_top_overall = best.col; nr_roll_top_overall = best.roll;       // :953-960
         nr_tilt_top_overall = best.tilt; topval_gp_overall = best.topval;
-        gp_result = transform_gp_in_wcs_and_publish(best.row, best.col, best.roll, best.tilt, topval_gp_overall - 20);  // :390
+        gp_result = to_grasp_output(grasp);                                       // :390 (eval = topval_gp_overall - 20)
     }
 
-    // transform_gp_in_wcs_and_publish numerics (:1274-1401); returns the GraspOutput instead of publishing
-    GraspOutput transform_gp_in_wcs_and_publish(int id_row_top_all, int id_col_top_all, int nr_roll_top_all, int /*nr_tilt_top_all*/,
-                                                int scaled_gp_eval) const {
+    // the GraspOutput message transform_gp_in_wcs_and_publish fills (:1384-1401) from the library's record
+    static GraspOutput to_grasp_output(const haf_grasp& g) {
         GraspOutput out;
-        out.eval = scaled_gp_eval;
-        haf_request rq;
-        memset(&rq, 0, sizeof rq);
-        rq.center[0] = graspsearchcenter.x; rq.center[1] = graspsearchcenter.y; rq.center[2] = graspsearchcenter.z;
-        rq.approach[0] = raw_approach_.x; rq.approach[1] = raw_approach_.y; rq.approach[2] = raw_approach_.z;
-        rq.gripper_opening_width = gripper_opening_width;
-        float M[16];
-        // :1276-1334: the same chain as :423-483, but the two angles come from the double approach_vector members (:1293-1303)
-        haf_build_transform_wcs(&rq, nr_roll_top_all < 0 ? 0 : nr_roll_top_all, step_deg_, M);
-        float x_gp_roll = -((float)(G / 2 - id_row_top_all)) / 100;                              // :1339
-        float y_gp_roll = -((float)(G / 2 - id_col_top_all)) / 100;                              // :1340
-        float h_locmax_roll = -10;
-        if (nr_roll_top_all >= 0)
-            for (int row_z = -4; row_z < 5; row_z++)                                              // :1343-1351 (asymmetric column range)
-                for (int col_z = -4; col_z < 4; col_z++) {
-                    const int r = id_row_top_all + row_z, c = id_col_top_all + col_z;
-                    if (r >= 0 && c >= 0 && r < G && c < G) {
-                        const float h = heightsgridroll[((size_t)nr_roll_top_all * G + r) * G + c];
-                        if (h_locmax_roll < h) h_locmax_roll = h;
-                    }
-                }
-        h_locmax_roll = (float)(h_locmax_roll - 0.01);                                            // :1354
-        const float z_gp_roll = h_locmax_roll;
-        const float x_gp_dis = 0.03f;                                                             // :1360
-        const float gp1[4] = {x_gp_roll - x_gp_dis, y_gp_roll, z_gp_roll, 1.0f};
-        const float gp2[4] = {x_gp_roll + x_gp_dis, y_gp_roll, z_gp_roll, 1.0f};
-        float Minv[16], g1[4], g2[4];
-        invert4(M, Minv);                                                                         // Eigen inverse(): not vendored, unpinned
-        mulvec4(Minv, gp1, g1);
-        mulvec4(Minv, gp2, g2);
-        out.graspPoint1.x = g1[0]; out.graspPoint1.y = g1[1]; out.graspPoint1.z = g1[2];          // :1389-1394
-        out.graspPoint2.x = g2[0]; out.graspPoint2.y = g2[1]; out.graspPoint2.z = g2[2];
-        out.averagedGraspPoint.x = (g1[0] + g2[0]) / 2.0;                                          // :1395-1397
-        out.averagedGraspPoint.y = (g1[1] + g2[1]) / 2.0;
-        out.averagedGraspPoint.z = (g1[2] + g2[2]) / 2.0;
-        // :1370-1374: appr_vec = transpose(rotation of av_trans_mat) * (0,0,1) = third ROW of av_trans_mat
-        out.approachVector.x = av_trans_mat[8]; out.approachVector.y = av_trans_mat[9]; out.approachVector.z = av_trans_mat[10];
-        out.roll = (float)((nr_roll_top_all * step_deg_ * 3.141592653) / 180);                     // :1401
+        out.eval = g.eval;
+        out.graspPoint1.x = g.graspPoint1[0]; out.graspPoint1.y = g.graspPoint1[1]; out.graspPoint1.z = g.graspPoint1[2];
+        out.graspPoint2.x = g.graspPoint2[0]; out.graspPoint2.y = g.graspPoint2[1]; out.graspPoint2.z = g.graspPoint2[2];
+        out.averagedGraspPoint.x = g.averagedGraspPoint[0]; out.averagedGraspPoint.y = g.averagedGraspPoint[1];
+        out.averagedGraspPoint.z = g.averagedGraspPoint[2];
+        out.approachVector.x = g.approachVector[0]; out.approachVector.y = g.approachVector[1]; out.approachVector.z = g.approachVector[2];
+        out.roll = g.roll;
         return out;
     }
 
     haf_ctx* ctx() { return ctx_; }
 
-    // general 4x4 float inverse by cofactors (adjugate / determinant)
-    static void invert4(const float* m, float* inv) {
-        float a[16];
-        a[0] = m[5] * m[10] * m[15] - m[5] * m[11] * m[14] - m[9] * m[6] * m[15] + m[9] * m[7] * m[14] + m[13] * m[6] * m[11] - m[13] * m[7] * m[10];
-        a[4] = -m[4] * m[10] * m[15] + m[4] * m[11] * m[14] + m[8] * m[6] * m[15] - m[8] * m[7] * m[14] - m[12] * m[6] * m[11] + m[12] * m[7] * m[10];
-        a[8] = m[4] * m[9] * m[15] - m[4] * m[11] * m[13] - m[8] * m[5] * m[15] + m[8] * m[7] * m[13] + m[12] * m[5] * m[11] - m[12] * m[7] * m[9];
-        a[12] = -m[4] * m[9] * m[14] + m[4] * m[10] * m[13] + m[8] * m[5] * m[14] - m[8] * m[6] * m[13] - m[12] * m[5] * m[10] + m[12] * m[6] * m[9];
-        a[1] = -m[1] * m[10] * m[15] + m[1] * m[11] * m[14] + m[9] * m[2] * m[15] - m[9] * m[3] * m[14] - m[13] * m[2] * m[11] + m[13] * m[3] * m[10];
-        a[5] = m[0] * m[10] * m[15] - m[0] * m[11] * m[14] - m[8] * m[2] * m[15] + m[8] * m[3] * m[14] + m[12] * m[2] * m[11] - m[12] * m[3] * m[10];
-        a[9] = -m[0] * m[9] * m[15] + m[0] * m[11] * m[13] + m[8] * m[1] * m[15] - m[8] * m[3] * m[13] - m[12] * m[1] * m[11] + m[12] * m[3] * m[9];
-        a[13] = m[0] * m[9] * m[14] - m[0] * m[10] * m[13] - m[8] * m[1] * m[14] + m[8] * m[2] * m[13] + m[12] * m[1] * m[10] - m[12] * m[2] * m[9];
-        a[2] = m[1] * m[6] * m[15] - m[1] * m[7] * m[14] - m[5] * m[2] * m[15] + m[5] * m[3] * m[14] + m[13] * m[2] * m[7] - m[13] * m[3] * m[6];
-        a[6] = -m[0] * m[6] * m[15] + m[0] * m[7] * m[14] + m[4] * m[2] * m[15] - m[4] * m[3] * m[14] - m[12] * m[2] * m[7] + m[12] * m[3] * m[6];
-        a[10] = m[0] * m[5] * m[15] - m[0] * m[7] * m[13] - m[4] * m[1] * m[15] + m[4] * m[3] * m[13] + m[12] * m[1] * m[7] - m[12] * m[3] * m[5];
-        a[14] = -m[0] * m[5] * m[14] + m[0] * m[6] * m[13] + m[4] * m[1] * m[14] - m[4] * m[2] * m[13] - m[12] * m[1] * m[6] + m[12] * m[2] * m[5];
-        a[3] = -m[1] * m[6] * m[11] + m[1] * m[7] * m[10] + m[5] * m[2] * m[11] - m[5] * m[3] * m[10] - m[9] * m[2] * m[7] + m[9] * m[3] * m[6];
-        a[7] = m[0] * m[6] * m[11] - m[0] * m[7] * m[10] - m[4] * m[2] * m[11] + m[4] * m[3] * m[10] + m[8] * m[2] * m[7] - m[8] * m[3] * m[6];
-        a[11] = -m[0] * m[5] * m[11] + m[0] * m[7] * m[9] + m[4] * m[1] * m[11] - m[4] * m[3] * m[9] - m[8] * m[1] * m[7] + m[8] * m[3] * m[5];
-        a[15] = m[0] * m[5] * m[10] - m[0] * m[6] * m[9] - m[4] * m[1] * m[10] + m[4] * m[2] * m[9] + m[8] * m[1] * m[6] - m[8] * m[2] * m[5];
-        const float det = m[0] * a[0] + m[1] * a[4] + m[2] * a[8] + m[3] * a[12];
-        const float inv_det = 1.0f / det;
-        for (int i = 0; i < 16; i++) inv[i] = a[i] * inv_det;
-    }
-    static void mulvec4(const float* M, const float* v, float* out) {
-        for (int i = 0; i < 4; i++) out[i] = ((M[i * 4] * v[0] + M[i * 4 + 1] * v[1]) + M[i * 4 + 2] * v[2]) + M[i * 4 + 3] * v[3];
-    }
-
 private:
     haf_ctx* ctx_ = nullptr;
     int step_deg_;
     Point3 raw_approach_{};
+    std::vector<haf_grasp> grasp_per_roll_;   // [R] records of the evaluated rolls (haf_search_grasps)
 };
 
 }  // namespace haf_b200

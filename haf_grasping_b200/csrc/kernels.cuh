@@ -1667,6 +1667,23 @@ struct JobResult {  // per job (cloud x request)
 struct JobParams {
     int return_only_best, graspval_top, n_rolls_active, roll_begin;  // rolls [roll_begin, n_rolls_active) are evaluated
 };
+
+// top cell of a unit after the tie rule (id_row_top_all, id_col_top_all, topval_gp_all of show_predicted_gps, :881-932)
+__device__ __forceinline__ int unit_top_cell(const unsigned long long* __restrict__ unit_top, const unsigned long long* __restrict__ unit_run,
+                                             int u, int G, int* row, int* col) {
+    const int val = (int)(unsigned)(unit_top[u] >> 32) - (1 << 20);
+    const unsigned long long rk = unit_run[u];
+    if (rk) {
+        *row = 0xFFFF - (int)((rk >> 16) & 0xFFFFu);
+        *col = (int)(rk & 0xFFFFu);
+    } else {   // no cell EQUALS topval (probability mode: topval is a truncated float): the first-maximum cell stays (:881-892)
+        const unsigned cell = 0xFFFFFFFFu - (unsigned)(unit_top[u] & 0xFFFFFFFFull);
+        *row = (int)(cell / (unsigned)G);
+        *col = (int)(cell % (unsigned)G);
+    }
+    return val;
+}
+
 // per-unit tops (after the tie rule) + a15 cross-roll reduction with the loop_control rules
 // (server.cpp:362-365 early exit, :953-960 strict >).  One thread per job.
 __global__ void reduce_rolls_kernel(const unsigned long long* __restrict__ unit_top, const unsigned long long* __restrict__ unit_run,
@@ -1680,18 +1697,7 @@ __global__ void reduce_rolls_kernel(const unsigned long long* __restrict__ unit_
     for (int roll = 0; roll < R; roll++) {
         const int u = j * R + roll;
         int row = -1, col = -1, val = -1000;
-        if (roll >= jp.roll_begin && roll < jp.n_rolls_active) {
-            val = (int)(unsigned)(unit_top[u] >> 32) - (1 << 20);
-            const unsigned long long rk = unit_run[u];
-            if (rk) {
-                row = 0xFFFF - (int)((rk >> 16) & 0xFFFFu);
-                col = (int)(rk & 0xFFFFu);
-            } else {   // no cell EQUALS topval (probability mode: topval is a truncated float): the first-maximum cell stays (:881-892)
-                const unsigned cell = 0xFFFFFFFFu - (unsigned)(unit_top[u] & 0xFFFFFFFFull);
-                row = (int)(cell / (unsigned)G);
-                col = (int)(cell % (unsigned)G);
-            }
-        }
+        if (roll >= jp.roll_begin && roll < jp.n_rolls_active) val = unit_top_cell(unit_top, unit_run, u, G, &row, &col);
         per_roll_top[(j * R + roll) * 3 + 0] = row;
         per_roll_top[(j * R + roll) * 3 + 1] = col;
         per_roll_top[(j * R + roll) * 3 + 2] = val;
@@ -1707,6 +1713,90 @@ __global__ void reduce_rolls_kernel(const unsigned long long* __restrict__ unit_
     JobResult r;
     r.row = brow; r.col = bcol; r.roll = broll; r.topval = best; r.rolls_done = done; r.n_windows = nwin; r.pad0 = r.pad1 = 0;
     results[j] = r;
+}
+
+// ---------------------------------------------------------------------------------------------------
+// a16: grasp pose in world coordinates (transform_gp_in_wcs_and_publish, server.cpp:1274-1401).  Launched only by the
+// grasp entry points: grasp_unit_kernel once per chunk while the chunk's heights are resident, grasp_gather_kernel once per
+// call after reduce_rolls_kernel.
+// ---------------------------------------------------------------------------------------------------
+struct GraspRec {      // = haf_grasp (include/hafgpu.h)
+    int eval;
+    float roll;
+    double gp1[3], gp2[3], avg[3], approach[3];
+    int row, col, roll_index, reserved;
+};
+static_assert(sizeof(GraspRec) == 120, "GraspRec layout");
+struct UnitPose {      // one (request, roll): inverse of the transform rebuilt from the double approach vector (:1276-1334), row-major
+    float Minv[16];
+};
+
+// Minv: the roll's UnitPose; Mrow2: third row of generate_grid's matrix of the roll (:1370-1374); heights: the roll's G x G grid,
+// not read when roll < 0 (no roll evaluated: h_locmax stays -10).  Float / double operations in the reference's order, no FMA.
+__device__ void grasp_pose(const float* __restrict__ Minv, const float* __restrict__ Mrow2, const float* __restrict__ heights, int G,
+                           int row, int col, int roll, int roll_step_deg, int eval, GraspRec* __restrict__ out) {
+    const float x_gp = __fdiv_rn(-(float)(G / 2 - row), 100.0f);   // :1339
+    const float y_gp = __fdiv_rn(-(float)(G / 2 - col), 100.0f);   // :1340
+    float h = -10.0f;
+    if (roll >= 0)
+        for (int rz = -4; rz < 5; rz++)           // :1343
+            for (int cz = -4; cz < 4; cz++) {     // :1344 (asymmetric column range)
+                const int r = row + rz, c = col + cz;
+                if (r >= 0 && c >= 0 && r < G && c < G) {
+                    const float v = heights[r * G + c];
+                    if (h < v) h = v;
+                }
+            }
+    const float z_gp = __double2float_rn(__dsub_rn((double)h, 0.01));   // :1354 (float -= double)
+    const float gp1[4] = {__fsub_rn(x_gp, 0.03f), y_gp, z_gp, 1.0f};   // :1360-1367
+    const float gp2[4] = {__fadd_rn(x_gp, 0.03f), y_gp, z_gp, 1.0f};
+    out->eval = eval;
+    out->roll = __double2float_rn(__ddiv_rn(__dmul_rn((double)(roll * roll_step_deg), 3.141592653), 180.0));   // :1401
+#pragma unroll
+    for (int i = 0; i < 3; i++) {
+        const float* m = Minv + 4 * i;
+        const float g1 = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[0], gp1[0]), __fmul_rn(m[1], gp1[1])), __fmul_rn(m[2], gp1[2])), __fmul_rn(m[3], gp1[3]));
+        const float g2 = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[0], gp2[0]), __fmul_rn(m[1], gp2[1])), __fmul_rn(m[2], gp2[2])), __fmul_rn(m[3], gp2[3]));
+        out->gp1[i] = (double)g1;                                   // :1389-1394
+        out->gp2[i] = (double)g2;
+        out->avg[i] = __ddiv_rn((double)__fadd_rn(g1, g2), 2.0);   // :1395-1397 (float sum, double division)
+        out->approach[i] = (double)Mrow2[i];
+    }
+    out->row = row; out->col = col; out->roll_index = roll; out->reserved = 0;
+}
+
+// one thread per unit of the chunk, right after tie_rule_kernel: the unit's top cell (as reduce_rolls_kernel decodes it) and its
+// pose, eval = max(top - 20, 10) (:962-972), into unit_grasp -- an array of the whole call, so it outlives the chunk's buffers.
+// units / unit_top / unit_run / keys_heights / unit_grasp: the chunk's slices; poses [n_requests][R], job_pose [job] -> request.
+__global__ void grasp_unit_kernel(const unsigned* __restrict__ keys_heights, int G, const UnitParams* __restrict__ units, int n_units,
+                                  const unsigned long long* __restrict__ unit_top, const unsigned long long* __restrict__ unit_run,
+                                  const UnitPose* __restrict__ poses, const int* __restrict__ job_pose, int R, int roll_step_deg,
+                                  GraspRec* __restrict__ unit_grasp) {
+    const int u = blockIdx.x * blockDim.x + threadIdx.x;
+    if (u >= n_units) return;
+    const UnitParams* up = units + u;
+    if (up->cloud < 0) return;   // roll not evaluated: its record is left as it is
+    int row, col;
+    const int val = unit_top_cell(unit_top, unit_run, u, G, &row, &col);
+    grasp_pose(poses[job_pose[up->job] * R + up->roll].Minv, up->M + 8, reinterpret_cast<const float*>(keys_heights) + (size_t)u * G * G, G,
+               row, col, up->roll, roll_step_deg, max(val - 20, 10), unit_grasp + u);
+}
+
+// one thread per job, after reduce_rolls_kernel: the winning unit's record with eval = topval - 20 (:390); a job that evaluated
+// no roll gets the reference's pose for roll -1 (roll 0's transforms, no height).  job_grasp: pinned host memory (UVA)
+__global__ void grasp_gather_kernel(const JobResult* __restrict__ results, int n_jobs, const UnitParams* __restrict__ units,
+                                    const UnitPose* __restrict__ poses, const int* __restrict__ job_pose, int R, int G, int roll_step_deg,
+                                    const GraspRec* __restrict__ unit_grasp, GraspRec* __restrict__ job_grasp) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n_jobs) return;
+    const JobResult r = results[j];
+    if (r.roll >= 0) {
+        GraspRec g = unit_grasp[j * R + r.roll];
+        g.eval = r.topval - 20;
+        job_grasp[j] = g;
+    } else {
+        grasp_pose(poses[job_pose[j] * R].Minv, units[j * R].M + 8, nullptr, G, r.row, r.col, -1, roll_step_deg, r.topval - 20, job_grasp + j);
+    }
 }
 
 // parameter block upload: src is pinned HOST memory read over PCIe through its UVA address (see run_jobs)

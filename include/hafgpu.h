@@ -187,6 +187,36 @@ int haf_search_batch(haf_ctx* ctx, const float* const* clouds, const size_t* n_p
 int haf_search_batch_packed(haf_ctx* ctx, const float* xyz_all_hostdev, const size_t* point_offsets, int n_clouds,
                             const haf_request* req, haf_best* best_per_cloud);
 
+/* ---- grasp poses (transform_gp_in_wcs_and_publish, server.cpp:1274-1401) ---------------------------------------------
+ * msg/GraspOutput.msg plus the indices the pose was built from.  The pose is computed on the device from the winning roll's
+ * height grid while that grid is still resident: the maximum over the 9 x 8 neighbourhood of the cell (:1343-1351), minus
+ * 0.01 in double (:1354), the two grasp points (+-0.03 m along the row axis, :1360) mapped through the inverse of the
+ * transform rebuilt from the double approach vector (:1276-1334, inverted on the host by adjugate / determinant), float
+ * sums in the order ((a x + b y) + c z) + d w.  Bit-equal to the reference's arithmetic (oracle/haf_oracle.cpp). */
+typedef struct {
+    int eval;                    /* topval - 20 for a best grasp (:390); max(topval - 20, 10) for a per-roll record (:962-972) */
+    float roll;                  /* radians, (float)((roll * step * 3.141592653) / 180) (:1401) */
+    double graspPoint1[3], graspPoint2[3], averagedGraspPoint[3];   /* world frame (:1339-1397) */
+    double approachVector[3];    /* third row of generate_grid's matrix (:1370-1374) */
+    int row, col, roll_index;    /* the cell and roll the pose was built from (-1 when no roll was evaluated) */
+    int reserved;
+} haf_grasp;
+
+/* haf_search plus the grasp poses, in one call.  grasp: the pose of `best`; grasp_per_request [n_requests] (optional): the
+ * pose of each best_per_request; grasp_per_roll [n_requests][R] (optional): the pose of every evaluated roll's top cell
+ * (per_roll_top), eval = max(top - 20, 10) -- rolls not evaluated (roll_begin / roll_limit) are left untouched.  When no
+ * roll was evaluated the record is the reference's pose for roll -1: roll 0's transforms and no height (h = -10 - 0.01).
+ * Records are written to host memory.  The caller applies graspval_th (70, server.cpp:962) before publishing. */
+int haf_search_grasps(haf_ctx* ctx, const float* xyz_hostdev, size_t n_points, size_t stride_bytes,
+                      const haf_request* reqs, int n_requests, haf_best* best, haf_best* best_per_request,
+                      float* graspseval, unsigned char* mask, float* heights, int* per_roll_top,
+                      haf_grasp* grasp, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll);
+/* haf_search_batch_packed plus one pose per cloud (grasp_per_cloud [n_clouds]) and optionally per evaluated roll of every
+ * cloud (grasp_per_roll [n_clouds][R]); the same staging, chunking and streams as haf_search_batch_packed. */
+int haf_search_batch_packed_grasps(haf_ctx* ctx, const float* xyz_all_hostdev, const size_t* point_offsets, int n_clouds,
+                                   const haf_request* req, haf_best* best_per_cloud,
+                                   haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_roll);
+
 /* ---- PCD / PointCloud2 ingest on the device (SURVEY 8f-2) -----------------------------------------------------------
  * What the reference does on the CPU before the hot path starts: the client's pcl::io::loadPCDFile<pcl::PointXYZ>
  * (src/calc_grasppoints_action_client.cpp:137-157) and the server's pcl::fromROSMsg (src/calc_grasppoints_action_server.cpp
