@@ -75,7 +75,7 @@ class haf_timing(C.Structure):
 
 EXPORTS = ["haf_create", "haf_destroy", "haf_last_error", "haf_get_info", "haf_set_stream", "haf_set_profiling",
            "haf_get_timing", "haf_launch_count", "haf_set_debug", "haf_search", "haf_search_batch", "haf_search_batch_packed",
-           "haf_search_grasps", "haf_search_batch_packed_grasps", "haf_build_transform", "haf_build_transform_wcs", "haf_best_key", "haf_pack_best_records", "haf_debug_window_count", "haf_debug_windows", "haf_debug_features",
+           "haf_search_grasps", "haf_search_batch_packed_grasps", "haf_search_batch_requests", "haf_debug_unit_params", "haf_debug_chunk_copy_waits", "haf_build_transform", "haf_build_transform_wcs", "haf_best_key", "haf_pack_best_records", "haf_debug_window_count", "haf_debug_windows", "haf_debug_features",
            "haf_debug_decisions", "haf_debug_tensor_inputs", "haf_debug_integral", "haf_debug_cell_indices", "haf_debug_text_roundtrip", "haf_debug_tc_probe",
            "haf_version", "haf_pcd_decode", "haf_search_pcd", "haf_pointcloud2_to_xyz", "haf_debug_pcd_xyz", "haf_svm_create", "haf_svm_destroy", "haf_svm_predict", "haf_svm_predict_probability", "haf_svm_check_probability_model", "haf_scale_minmax", "haf_scale_apply"]
 
@@ -117,6 +117,10 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
                                     C.POINTER(haf_grasp), C.POINTER(haf_grasp), C.POINTER(haf_grasp)]
     L.haf_search_batch_packed_grasps.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(haf_request), C.POINTER(haf_best),
                                                  C.POINTER(haf_grasp), C.POINTER(haf_grasp)]
+    L.haf_search_batch_requests.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(haf_request), C.POINTER(ci), C.POINTER(haf_best),
+                                            C.POINTER(haf_best), vp, C.POINTER(haf_grasp), C.POINTER(haf_grasp), C.POINTER(haf_grasp)]
+    L.haf_debug_unit_params.argtypes = [vp, vp, vp, vp, ci]
+    L.haf_debug_chunk_copy_waits.argtypes = [vp, vp, ci]
     L.haf_build_transform.argtypes = [C.POINTER(haf_request), ci, ci, C.POINTER(C.c_float)]
     L.haf_build_transform_wcs.argtypes = [C.POINTER(haf_request), ci, ci, C.POINTER(C.c_float)]
     L.haf_best_key.argtypes = [ci, C.c_uint32]
@@ -162,6 +166,30 @@ def make_request(center=(0.0, 0.0, 0.0), area=(32.0, 44.0), approach=(0.0, 0.0, 
     rq.roll_begin = roll_begin
     rq.svm_with_probability = svm_with_probability
     return rq
+
+
+def make_requests(n=None, centers=(0.0, 0.0, 0.0), approaches=(0.0, 0.0, 1.0), areas=(32.0, 44.0), widths=1, return_only_best=0,
+                  graspval_top=119, roll_limit=0, roll_begin=0, svm_with_probability=0):
+    """Vectorised ``make_request``: a ctypes array of n haf_request.  Every argument is one value (broadcast) or one per request:
+    centers / approaches [n, 3], areas [n, 2], the int fields [n].  n defaults to the longest per-request argument."""
+    vec = dict(centers=np.asarray(centers, np.float64), approaches=np.asarray(approaches, np.float64), areas=np.asarray(areas, np.float32))
+    ints = dict(gripper_opening_width=widths, return_only_best=return_only_best, graspval_top=graspval_top, roll_limit=roll_limit,
+                roll_begin=roll_begin, svm_with_probability=svm_with_probability)
+    ints = {k: np.asarray(v, np.int32) for k, v in ints.items()}
+    if n is None:
+        n = max([len(v) for v in vec.values() if v.ndim == 2] + [len(v) for v in ints.values() if v.ndim == 1] + [1])
+    arr = (haf_request * n)()
+    rec = np.frombuffer(arr, np.dtype({"names": [f[0] for f in haf_request._fields_],
+                                       "formats": [(np.float64, 3), np.float32, np.float32, (np.float64, 3)] + [np.int32] * 6,
+                                       "offsets": [getattr(haf_request, f[0]).offset for f in haf_request._fields_],
+                                       "itemsize": C.sizeof(haf_request)}))
+    rec["center"] = np.broadcast_to(vec["centers"], (n, 3))
+    areas = np.broadcast_to(vec["areas"], (n, 2))
+    rec["area_len_x"], rec["area_len_y"] = areas[:, 0], areas[:, 1]
+    rec["approach"] = np.broadcast_to(vec["approaches"], (n, 3))
+    for k, v in ints.items():
+        rec[k] = np.broadcast_to(v, (n,))
+    return arr
 
 
 def _ptr(a):
@@ -339,6 +367,52 @@ class GraspSearch:
         if groll is not None:
             out["grasp_per_roll"] = groll
         return out
+
+    def search_batch_requests(self, xyz_all, point_offsets, requests, request_offsets=None, grasps=True, per_roll=False,
+                              per_roll_top=False):
+        """Each cloud with its own requests (haf_search_batch_requests): cloud c is searched with
+        requests[request_offsets[c]:request_offsets[c + 1]] (None: one request per cloud).  requests: a haf_request array (see
+        ``make_requests``) or a list.  Returns a dict like ``search_batch_packed_grasps``: ``best`` and, with grasps, ``grasp`` per
+        cloud, plus ``best_per_request``, with grasps ``grasp_per_request``, with per_roll ``grasp_per_roll`` (haf_grasp array
+        [n_requests * R], evaluated rolls only) and with per_roll_top ``per_roll_top`` (int32 [n_requests, R, 3])."""
+        if not isinstance(requests, C.Array):
+            requests = (haf_request * len(requests))(*requests)
+        n_clouds = len(point_offsets) - 1
+        nreq = len(requests)
+        off = (C.c_size_t * len(point_offsets))(*[int(o) for o in point_offsets])
+        roff = None if request_offsets is None else (C.c_int * len(request_offsets))(*[int(o) for o in request_offsets])
+        best, bpr = (haf_best * n_clouds)(), (haf_best * nreq)()
+        grasp = (haf_grasp * n_clouds)() if grasps else None
+        gpr = (haf_grasp * nreq)() if grasps else None
+        groll = (haf_grasp * (nreq * self.R))() if grasps and per_roll else None
+        top = np.full((nreq, self.R, 3), -1, np.int32) if per_roll_top else None
+        if isinstance(xyz_all, np.ndarray):
+            xyz_all = np.ascontiguousarray(xyz_all, np.float32)
+        self._check(self.L.haf_search_batch_requests(self.h, _ptr(xyz_all), off, n_clouds, requests, roff, best, bpr, _ptr(top),
+                                                     grasp, gpr, groll))
+        out = {"best": best, "best_per_request": bpr}
+        if grasps:
+            out["grasp"], out["grasp_per_request"] = grasp, gpr
+        if groll is not None:
+            out["grasp_per_roll"] = groll
+        if top is not None:
+            out["per_roll_top"] = top
+        return out
+
+    def debug_unit_params(self, n_units, poses=True):
+        """unit parameters of the last search (haf_debug_unit_params): (M [U, 16], mask [U, 10], Minv [U, 16] or None)"""
+        M, mask = np.zeros((n_units, 16), np.float32), np.zeros((n_units, 10), np.float32)
+        Minv = np.zeros((n_units, 16), np.float32) if poses else None
+        U = self._check(self.L.haf_debug_unit_params(self.h, _ptr(M), _ptr(mask), _ptr(Minv), n_units))
+        return M[:U], mask[:U], (Minv[:U] if poses else None)
+
+    def debug_chunk_copy_waits(self):
+        """chunks of the last search (haf_debug_chunk_copy_waits): int32 [n, 5] = first cloud, end cloud, stream set, copy piece
+        waited for (-1: device input), end cloud of that piece"""
+        t = self.timing()
+        out = np.zeros((max(int(t.n_chunks), 1), 5), np.int32)
+        n = self._check(self.L.haf_debug_chunk_copy_waits(self.h, _ptr(out), len(out)))
+        return out[:n]
 
     def pack_best_records(self, best, out):
         """haf_best array of a batch -> int32 [n, 8] records (topval, row, col, roll, tilt, approach_idx, n_windows, rolls_done)

@@ -9,6 +9,7 @@
 #include <condition_variable>
 #include <cstring>
 #include <mutex>
+#include <unordered_map>
 #include <string>
 #include <thread>
 #include <vector>
@@ -216,6 +217,32 @@ struct haf_ctx {
     int grasp_mode = 0;
     DevBuf<GraspRec> d_unit_grasp;       // [U] written chunk by chunk (outlives the per-chunk buffers)
     PinBuf<GraspRec> h_unit_grasp, h_job_grasp;   // h_job_grasp [n_jobs] is written by grasp_gather_kernel itself (UVA)
+
+    // unit parameters built on the device (haf_search_batch_requests, kernels.cuh expand_units_kernel); set for one call by
+    // DeviceUnitsScope.  The host part: the libm values per roll (built at haf_create) and per distinct approach vector.
+    bool device_units = false;
+    std::vector<hafhost::RollTrig> roll_trig;            // [R]
+    std::vector<hafhost::ApproachTrig> approach_trig;    // distinct approach vectors of the call, first occurrence order
+    std::vector<int> job_approach;                       // [n_jobs] index into approach_trig
+    struct ApproachKey {
+        uint64_t b[3];
+        bool operator==(const ApproachKey& o) const { return b[0] == o.b[0] && b[1] == o.b[1] && b[2] == o.b[2]; }
+    };
+    struct ApproachHash {
+        size_t operator()(const ApproachKey& k) const { return (size_t)((k.b[0] * 0x9E3779B97F4A7C15ull) ^ (k.b[1] * 0xC2B2AE3D27D4EB4Full) ^ (k.b[2] * 0x165667B19E3779F9ull)); }
+    };
+    std::unordered_map<ApproachKey, int, ApproachHash> approach_index;
+    DevBuf<UnitParams> d_dev_units;      // [U]
+    DevBuf<UnitPose> d_dev_pose;         // [U] one pose per unit
+    PinBuf<float> h_best_M;              // [n_jobs][16] matrix of each job's winning roll (written by reduce_rolls_kernel, UVA)
+    // where the unit parameters of the last call live, whichever path built them (haf_debug_unit_params); units 0 = none
+    const UnitParams* last_up_units = nullptr;
+    const UnitPose* last_up_pose = nullptr;   // NULL: the call built no poses
+    const int* last_up_jpose = nullptr;       // [n_jobs] pose set of each job
+    int last_up_n = 0, last_up_jobs = 0;
+    // per chunk of the last call: first cloud, end cloud, stream set, copy piece its stream waited for (-1: none), that piece's
+    // end cloud (haf_debug_chunk_copy_waits)
+    std::vector<int> last_chunk_waits;
 
     // probability estimates (SURVEY 8f-4): the model's sigmoid (svm.cpp:2811-2824); probability calls evaluate EVERY row /
     // window on the FP64 exact-order path (force_exact), whatever svm_mode the context was made with
@@ -496,6 +523,7 @@ static int create_impl(haf_ctx** out, const haf_config* cfg, bool svm_only, int 
     ctx->device = cfg->device;
     ctx->sm_count = prop.multiProcessorCount;
     ctx->F = F; ctx->D = D; ctx->Dsv = Dsv; ctx->Kpad = Kpad; ctx->S = S; ctx->Spad = Spad; ctx->R = R; ctx->G = G;
+    for (int roll = 0; roll < R; roll++) ctx->roll_trig.push_back(hafhost::roll_trig(roll, step));
     ctx->lower = range.lower; ctx->upper = range.upper; ctx->gamma = model.gamma; ctx->rho = model.rho;
     ctx->label[0] = model.label[0]; ctx->label[1] = model.label[1];
     ctx->gv[0] = hafhost::label_to_gridvalue(model.label[0]);
@@ -1275,19 +1303,46 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     struct ForceExact { haf_ctx* c; bool on; ~ForceExact() { if (on) c->force_exact = false; } } force_exact_scope{ctx, prob};
     if (prob) ctx->force_exact = true;
 
-    // ---- host: unit parameters (transforms and mask constants use the HOST libm, see haf_host.hpp)
+    // ---- host: unit parameters (transforms and mask constants use the HOST libm, see haf_host.hpp).  With device_units the
+    // host writes one JobSpec per job and the libm tables instead, and expand_units_kernel builds the units, JobParams and poses.
+    const bool dev_units = ctx->device_units;
     const int U = n_jobs * R;
-    const size_t bytes_units = (size_t)U * sizeof(UnitParams), bytes_jobs = (size_t)n_jobs * sizeof(JobParams);
+    ctx->last_up_n = 0;
+    ctx->last_chunk_waits.clear();
+    const bool grasp = ctx->grasp_mode > 0;
+    if (dev_units) {   // distinct approach vectors (bitwise), in order of first occurrence
+        ctx->approach_trig.clear(); ctx->approach_index.clear(); ctx->job_approach.resize(n_jobs);
+        for (int j = 0; j < n_jobs; j++) {
+            haf_ctx::ApproachKey k;
+            memcpy(k.b, jobs[j].rq.approach, sizeof k.b);
+            if (j > 0 && memcmp(jobs[j - 1].rq.approach, k.b, sizeof k.b) == 0) { ctx->job_approach[j] = ctx->job_approach[j - 1]; continue; }
+            const auto ins = ctx->approach_index.emplace(k, (int)ctx->approach_trig.size());
+            if (ins.second) {
+                hafhost::ApproachTrig t;
+                hafhost::approach_trig(jobs[j].rq.approach, false, t.grid);
+                if (grasp) hafhost::approach_trig(jobs[j].rq.approach, true, t.wcs);
+                else memset(t.wcs, 0, sizeof t.wcs);
+                ctx->approach_trig.push_back(t);
+            }
+            ctx->job_approach[j] = ins.first->second;
+        }
+    }
+    const int n_approach = dev_units ? (int)ctx->approach_trig.size() : 0;
+    const size_t bytes_units = dev_units ? 0 : (size_t)U * sizeof(UnitParams), bytes_jobs = (size_t)n_jobs * sizeof(JobParams);
     const size_t bytes_off = (size_t)(n_clouds + 1) * sizeof(long long), bytes_ub = (size_t)(n_clouds + 1) * sizeof(int);
     const size_t o_units = 0, o_jobs = round_up(o_units + bytes_units, 256), o_off = round_up(o_jobs + bytes_jobs, 256), o_ub = round_up(o_off + bytes_off, 256);
     // grasp poses: the inverse WCS matrices per (distinct request, roll) and each job's request index, after the block above
-    const bool grasp = ctx->grasp_mode > 0;
+    // (device_units: one pose per unit outside the block, each job its own set)
     int n_pose_sets = 0;
-    if (grasp)
+    if (grasp && !dev_units)
         for (int j = 0; j < n_jobs; j++)
             if (j == 0 || memcmp(&jobs[j - 1].rq, &jobs[j].rq, sizeof(haf_request)) != 0) n_pose_sets++;
     const size_t o_jpose = round_up(o_ub + bytes_ub, 256), o_pose = round_up(o_jpose + (grasp ? (size_t)n_jobs * sizeof(int) : 0), 256);
-    const size_t bytes_block = grasp ? o_pose + (size_t)n_pose_sets * R * sizeof(UnitPose) : o_ub + bytes_ub;
+    const size_t bytes_host_units = grasp ? o_pose + (size_t)n_pose_sets * R * sizeof(UnitPose) : o_ub + bytes_ub;
+    // device_units: the job records and the libm tables
+    const size_t o_spec = round_up(bytes_host_units, 256), o_rtrig = round_up(o_spec + (size_t)n_jobs * sizeof(JobSpec), 256),
+                 o_atrig = round_up(o_rtrig + (size_t)R * sizeof(hafhost::RollTrig), 256);
+    const size_t bytes_block = dev_units ? o_atrig + (size_t)n_approach * sizeof(hafhost::ApproachTrig) : bytes_host_units;
     ENSURE(ctx, ctx->h_stage, bytes_block + 16);
     UnitParams* hu = reinterpret_cast<UnitParams*>(ctx->h_stage.p + o_units);
     JobParams* hj = reinterpret_cast<JobParams*>(ctx->h_stage.p + o_jobs);
@@ -1295,6 +1350,11 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     int* hub = reinterpret_cast<int*>(ctx->h_stage.p + o_ub);
     int* hjpose = reinterpret_cast<int*>(ctx->h_stage.p + o_jpose);
     UnitPose* hpose = reinterpret_cast<UnitPose*>(ctx->h_stage.p + o_pose);
+    JobSpec* hspec = reinterpret_cast<JobSpec*>(ctx->h_stage.p + o_spec);
+    if (dev_units) {
+        memcpy(ctx->h_stage.p + o_rtrig, ctx->roll_trig.data(), (size_t)R * sizeof(hafhost::RollTrig));
+        memcpy(ctx->h_stage.p + o_atrig, ctx->approach_trig.data(), (size_t)n_approach * sizeof(hafhost::ApproachTrig));
+    }
     long long max_points = 0;
     for (int c = 0; c <= n_clouds; c++) hoff[c] = cs.off[c];
     for (int c = 0; c < n_clouds; c++) max_points = std::max(max_points, cs.off[c + 1] - cs.off[c]);
@@ -1313,6 +1373,16 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
         jb.n_rolls_active = (jb.rq.roll_limit > 0) ? std::min(R, jb.rq.roll_limit) : R;
         jb.roll_begin = std::max(0, std::min(jb.rq.roll_begin, jb.n_rolls_active));
         jb.wbound = window_bound(G, jb.rq) * (jb.n_rolls_active - jb.roll_begin);
+        if (dev_units) {
+            JobSpec& sp = hspec[j];
+            memcpy(sp.center, jb.rq.center, sizeof sp.center);
+            sp.cloud = jb.cloud; sp.approach = ctx->job_approach[j];
+            sp.gripper_opening_width = jb.rq.gripper_opening_width; sp.area_x = ax; sp.area_y = ay;
+            sp.roll_begin = jb.roll_begin; sp.n_rolls_active = jb.n_rolls_active;
+            sp.return_only_best = jb.rq.return_only_best; sp.graspval_top = jb.rq.graspval_top; sp.pad = 0;
+            if (grasp) hjpose[j] = j;
+            continue;
+        }
         hj[j].return_only_best = jb.rq.return_only_best; hj[j].graspval_top = jb.rq.graspval_top;
         hj[j].n_rolls_active = jb.n_rolls_active; hj[j].roll_begin = jb.roll_begin;
         // a batch applies ONE request to every cloud: the transforms and mask constants (host libm, ~1 us per unit) are built
@@ -1336,7 +1406,7 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
                 memset(&up, 0, sizeof up);
                 float M[16];
                 hafhost::build_transform(jb.rq, roll, ctx->cfg.roll_step_deg, M);
-                memcpy(up.M, M, 12 * sizeof(float));
+                memcpy(up.M, M, sizeof M);
                 const hafhost::MaskConsts mc = hafhost::mask_consts(G, roll, ctx->cfg.roll_step_deg, ax, ay);
                 up.sa = mc.sa; up.ca = mc.ca; up.cx1 = mc.cx1; up.cy1 = mc.cy1; up.cx2 = mc.cx2; up.cy2 = mc.cy2;
                 up.cx3 = mc.cx3; up.cy3 = mc.cy3; up.cx4 = mc.cx4; up.cy4 = mc.cy4;
@@ -1393,6 +1463,10 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
         return ctx->fail(HAF_ERR_UNSUPPORTED, "per-roll outputs need the whole request in one chunk (windows x dims too large)");
 
     ENSURE(ctx, ctx->d_params, bytes_block + 16); ENSURE(ctx, ctx->d_results, n_jobs); ENSURE(ctx, ctx->d_per_roll_top, (size_t)U * 3);
+    if (dev_units) {
+        ENSURE(ctx, ctx->d_dev_units, U); ENSURE(ctx, ctx->h_best_M, (size_t)n_jobs * 16);
+        if (grasp) ENSURE(ctx, ctx->d_dev_pose, U);
+    }
     if (grasp) {
         ENSURE(ctx, ctx->d_unit_grasp, U); ENSURE(ctx, ctx->h_job_grasp, n_jobs);
         if (ctx->grasp_mode > 1) ENSURE(ctx, ctx->h_unit_grasp, U);
@@ -1448,7 +1522,7 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
         gkey.wcap = (size_t)wsum_all; gkey.pts_bucket = pts_bucket; gkey.n_jobs = n_jobs; gkey.n_clouds = n_clouds;
         // (grasp poses: the two pose kernels, the record copies and the size of the parameter block belong to the graph too)
         gkey.flags = (prob ? 1 : 0) | (keep_debug_state ? 2 : 0) | (avg_points_all >= 8 * (long long)GG ? 4 : 0) | (ctx->cfg.emulate_text_roundtrip ? 8 : 0) |
-                     (ctx->grasp_mode << 4) | (n_pose_sets << 8);
+                     (ctx->grasp_mode << 4) | (dev_units ? 64 : 0) | ((dev_units ? n_approach : n_pose_sets) << 8);
         gkey.tc_passes = ctx->tc_passes; gkey.o_evals = dst_evals; gkey.o_mask = dst_mask; gkey.o_heights = dst_heights; gkey.rolls_hash = hsh; gkey.st = st;
         for (size_t i = 0; i < ctx->graphs.size() && gmode == 0; i++)
             if (ctx->graphs[i].key == gkey) { gmode = 2; graph_slot = (int)i; }
@@ -1459,6 +1533,12 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
             else { seen_slot = (int)(ctx->graph_seen_next++ % haf_ctx::kMaxGraphs); ctx->graph_seen[seen_slot] = gkey; }
         }
     }
+    UnitParams* const d_units = dev_units ? ctx->d_dev_units.p : reinterpret_cast<UnitParams*>(ctx->d_params.p + o_units);
+    JobParams* const d_jobs = reinterpret_cast<JobParams*>(ctx->d_params.p + o_jobs);
+    long long* const d_ptoff = reinterpret_cast<long long*>(ctx->d_params.p + o_off);
+    int* const d_cloud_ubegin = reinterpret_cast<int*>(ctx->d_params.p + o_ub);
+    const int* const d_jpose = reinterpret_cast<const int*>(ctx->d_params.p + o_jpose);
+    const UnitPose* const d_pose = dev_units ? ctx->d_dev_pose.p : reinterpret_cast<const UnitPose*>(ctx->d_params.p + o_pose);
     float ms_stage[7] = {0, 0, 0, 0, 0, 0, 0};
     long long total_windows = 0, total_guard = 0;
     if (gmode == 2) {
@@ -1481,12 +1561,13 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
                                                                                               reinterpret_cast<uint4*>(ctx->d_params.p), n16);
         LAUNCHED(ctx);
     }
-    UnitParams* const d_units = reinterpret_cast<UnitParams*>(ctx->d_params.p + o_units);
-    JobParams* const d_jobs = reinterpret_cast<JobParams*>(ctx->d_params.p + o_jobs);
-    long long* const d_ptoff = reinterpret_cast<long long*>(ctx->d_params.p + o_off);
-    int* const d_cloud_ubegin = reinterpret_cast<int*>(ctx->d_params.p + o_ub);
-    const int* const d_jpose = reinterpret_cast<const int*>(ctx->d_params.p + o_jpose);
-    const UnitPose* const d_pose = reinterpret_cast<const UnitPose*>(ctx->d_params.p + o_pose);
+    if (dev_units) {
+        expand_units_kernel<<<(U + 127) / 128, 128, 0, st>>>(reinterpret_cast<const JobSpec*>(ctx->d_params.p + o_spec),
+                                                            reinterpret_cast<const hafhost::ApproachTrig*>(ctx->d_params.p + o_atrig),
+                                                            reinterpret_cast<const hafhost::RollTrig*>(ctx->d_params.p + o_rtrig), n_jobs, R, G,
+                                                            d_units, d_jobs, grasp ? ctx->d_dev_pose.p : nullptr);
+        LAUNCHED(ctx);
+    }
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_unit_block.p, 0, ((size_t)2 * U + (U + 1) / 2) * 8, st));
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_counters.p, 0, 64 * 4, st));
     // host-staged batch in several chunks: chunks alternate between the call's stream and a second one (see haf_ctx::ChunkWs)
@@ -1512,7 +1593,7 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     const bool smallG = (size_t)G * ld * sizeof(double) <= 200 * 1024;
     const float neg_gamma_log2e = (float)(-ctx->gamma * 1.4426950408889634);
 
-    int next_piece = 0;
+    int last_piece = 0;   // copy piece that holds the last cloud of the current chunk
     for (size_t ci = 0; ci < chunks.size(); ci++) {
         const int j0 = chunks[ci].first, j1 = chunks[ci].second;
         const int Uc = (j1 - j0) * R, ubase = j0 * R;
@@ -1541,15 +1622,22 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
         if (ci >= (size_t)nsets) CUDA_TRY(ctx, cudaMemsetAsync(cnt, 0, 2 * 4, st));  // win_count, guard_count
         const UnitParams* units_c = d_units + ubase;
 
-        // staged host clouds: wait for the copy pieces that cover this chunk's clouds
-        while (next_piece < ctx->copy_pieces && (next_piece == 0 ? 0 : ctx->copy_cloud_end[next_piece - 1]) < c1) {
+        // staged host clouds: this chunk's stream waits for the copy piece that holds the chunk's last cloud.  The pieces are
+        // copied in order on one stream, so that event covers every earlier piece as well.  The wait is made on this chunk's own
+        // stream even when a chunk on another stream has waited for the same piece: a wait orders only the stream it is made on
+        // (chunks split on request boundaries, so several chunks of a call may end inside one piece).
+        if (ctx->copy_pieces > 0) {
+            while (ctx->copy_cloud_end[last_piece] < c1) last_piece++;   // c1 never decreases; the last piece ends at n_clouds
             if (ctx->stager.active) {   // pageable source: the helper thread records the event -- wait until it has (an unrecorded event does not block)
                 std::unique_lock<std::mutex> lk(ctx->stager.mu);
-                ctx->stager.cv.wait(lk, [&] { return ctx->stager.issued > next_piece; });
+                ctx->stager.cv.wait(lk, [&] { return ctx->stager.issued > last_piece; });
                 if (ctx->stager.failed) return ctx->fail(HAF_ERR_CUDA, "staging a pageable host batch failed (pinned ring copy / cudaMemcpyAsync)");
             }
-            CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->copy_ev[next_piece], 0));
-            next_piece++;
+            CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->copy_ev[last_piece], 0));
+        }
+        {
+            const int w[5] = {c0, c1, set, ctx->copy_pieces > 0 ? last_piece : -1, ctx->copy_pieces > 0 ? ctx->copy_cloud_end[last_piece] : -1};
+            ctx->last_chunk_waits.insert(ctx->last_chunk_waits.end(), w, w + 5);
         }
         // 1. binning
         if (prof) CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[ci * 8 + 0], st));
@@ -1562,7 +1650,7 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
             const long long avg_points = (cs.off[c1] - cs.off[c0]) / std::max(1, c1 - c0);
             if (upg >= 1 && avg_points >= 8 * (long long)GG && (c1 - c0) * 8 >= ctx->sm_count && (ctx->cfg.reserved[1] & 15) != 1) {
                 int max_units_per_cloud = 0;
-                for (int c = c0; c < c1; c++) max_units_per_cloud = std::max(max_units_per_cloud, hub[c + 1] - hub[c]);
+                for (int c = c0; c < c1; c++) max_units_per_cloud = std::max(max_units_per_cloud, std::min(hub[c + 1], ubase + Uc) - std::max(hub[c], ubase));
                 const int ug = std::min(upg, std::max(1, max_units_per_cloud));
                 // The kernel is instruction-bound once the REDs are filtered, one 1024-thread CTA per SM.  A CTA costs a fixed part
                 // (150 KB of shared-memory bounds initialised and flushed, launch) plus its slice of the cloud's points; the CTAs
@@ -1585,11 +1673,11 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
                 if (cs.stride == 12 && (ctx->cfg.reserved[1] & 15) != 2)
                     bin_maxz_cloud_kernel<4><<<gridc, 1024, (size_t)ug * GG * 4, st>>>(cs.d_xyz, cs.stride, d_ptoff + c0, d_cloud_ubegin + c0, d_units,
                                                                                      ctx->d_keys.p - (size_t)ubase * GG, G, r, ug,
-                                                                                     reinterpret_cast<unsigned long long*>(cnt + 4));
+                                                                                     reinterpret_cast<unsigned long long*>(cnt + 4), ubase, ubase + Uc);
                 else
                     bin_maxz_cloud_kernel<1><<<gridc, 1024, (size_t)ug * GG * 4, st>>>(cs.d_xyz, cs.stride, d_ptoff + c0, d_cloud_ubegin + c0, d_units,
                                                                                      ctx->d_keys.p - (size_t)ubase * GG, G, r, ug,
-                                                                                     reinterpret_cast<unsigned long long*>(cnt + 4));
+                                                                                     reinterpret_cast<unsigned long long*>(cnt + 4), ubase, ubase + Uc);
                 LAUNCHED(ctx);
             } else {
                 const int PPT = 4;
@@ -1600,7 +1688,7 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
                     // cloud_unit_begin is relative to unit 0 of the call: shift the key base so unit u lands at keys[u - ubase]
                     bin_maxz_kernel<PPT><<<grid, 256, 0, st>>>(cs.d_xyz, cs.stride, d_ptoff + c0, d_cloud_ubegin + c0, d_units,
                                                                ctx->d_keys.p - (size_t)ubase * GG, G, r, nullptr,
-                                                               reinterpret_cast<unsigned long long*>(cnt + 4));
+                                                               reinterpret_cast<unsigned long long*>(cnt + 4), ubase, ubase + Uc);
                     LAUNCHED(ctx);
                 }
             }
@@ -1696,7 +1784,7 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     }
     // 7. cross-roll reduction per job, results to pinned host memory
     reduce_rolls_kernel<<<(n_jobs + 127) / 128, 128, 0, st>>>(d_unit_top, d_unit_run, d_unit_windows, d_jobs, n_jobs, R, G,
-                                                             ctx->d_per_roll_top.p, ctx->d_results.p);
+                                                             ctx->d_per_roll_top.p, ctx->d_results.p, d_units, dev_units ? ctx->h_best_M.p : nullptr);
     LAUNCHED(ctx);
     if (grasp) {   // a16 per job: the winning unit's record (or the roll -1 pose), written straight into pinned host memory (a
                    // copy node less on a single goal's critical path; the stream synchronise below makes it visible)
@@ -1770,6 +1858,8 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     t.escalations = ctx->escalations;
     t.graph_replays = (int)std::min<long long>(ctx->graph_replays, 0x7fffffff);
     if (keep_debug_state) { ctx->last_W = (unsigned)total_windows; ctx->last_valid = true; }
+    ctx->last_up_units = d_units; ctx->last_up_pose = grasp ? d_pose : nullptr; ctx->last_up_jpose = d_jpose;
+    ctx->last_up_n = U; ctx->last_up_jobs = n_jobs;
     return HAF_OK;
 }
 
@@ -1795,12 +1885,17 @@ static int run_jobs(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& jobs, fl
     }
 }
 
-static void fill_best(const haf_ctx* ctx, const Job& jb, const JobResult& r, int approach_idx, long long n_guard, haf_best* b) {
+// M: the winning roll's matrix as the device built it (haf_search_batch_requests); NULL = build it on the host
+static void fill_best(const haf_ctx* ctx, const Job& jb, const JobResult& r, int approach_idx, long long n_guard, haf_best* b,
+                      const float* M = nullptr) {
     memset(b, 0, sizeof *b);
     b->row = r.row; b->col = r.col; b->roll = r.roll; b->tilt = (r.roll >= 0) ? 0 : -1; b->approach_idx = approach_idx;
     b->topval = r.topval; b->eval = r.topval - 20;                                          // server.cpp:390
     b->roll_rad = (float)((r.roll * ctx->cfg.roll_step_deg * hafhost::kPI) / 180);           // :1401
-    if (r.roll >= 0) hafhost::build_transform(jb.rq, r.roll, ctx->cfg.roll_step_deg, b->M);
+    if (r.roll >= 0) {
+        if (M) memcpy(b->M, M, sizeof b->M);
+        else hafhost::build_transform(jb.rq, r.roll, ctx->cfg.roll_step_deg, b->M);
+    }
     b->rolls_done = r.rolls_done; b->n_windows_scored = r.n_windows; b->n_guard = (int)n_guard;
 }
 
@@ -1866,6 +1961,12 @@ struct GraspScope {
     GraspScope(haf_ctx* ctx, const GraspOut* go) : c(ctx) { c->grasp_mode = go ? ((go->per_roll || go->units) ? 2 : 1) : 0; }
     ~GraspScope() { c->grasp_mode = 0; }
 };
+// unit parameters built on the device for the length of one call (haf_search_batch_requests)
+struct DeviceUnitsScope {
+    haf_ctx* c;
+    explicit DeviceUnitsScope(haf_ctx* ctx) : c(ctx) { c->device_units = true; }
+    ~DeviceUnitsScope() { c->device_units = false; }
+};
 // per-roll records of the evaluated rolls of each job: h_unit_grasp -> out [n_jobs][R] (the other rolls are left untouched)
 static void copy_roll_grasps(const haf_ctx* ctx, const std::vector<Job>& jobs, haf_grasp* out) {
     const int R = ctx->R;
@@ -1880,6 +1981,9 @@ static int group_search(haf_ctx* ctx, const float* xyz, size_t n_points, size_t 
                         const GraspOut* go = nullptr);
 static int group_batch_packed(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* req,
                               haf_best* best_per_cloud, const GraspOut* go = nullptr);
+static int group_batch_requests(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
+                                const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
+                                haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll);
 static void group_timing(haf_ctx* ctx);
 
 // one GPU: the context itself (also what each member of a multi-GPU group runs -- group[0] IS the head context, so the
@@ -1889,6 +1993,9 @@ static int search_single(haf_ctx* ctx, const float* xyz, size_t n_points, size_t
                          const GraspOut* go = nullptr);
 static int batch_packed_single(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* req,
                                haf_best* best_per_cloud, const GraspOut* go = nullptr);
+static int batch_requests_single(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
+                                 const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
+                                 haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll);
 static int batch_single(haf_ctx* ctx, const float* const* clouds, const size_t* n_points, int n_clouds, const haf_request* req,
                         haf_best* best_per_cloud);
 
@@ -1980,12 +2087,11 @@ extern "C" int haf_search_batch_packed_grasps(haf_ctx* ctx, const float* xyz_all
     if (ctx->group.size() > 1) return group_batch_packed(ctx, xyz_all, point_offsets, n_clouds, req, best_per_cloud, &go);
     return batch_packed_single(ctx, xyz_all, point_offsets, n_clouds, req, best_per_cloud, &go);
 }
-static int batch_packed_single(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* req,
-                               haf_best* best_per_cloud, const GraspOut* go) {
-    if (!point_offsets || n_clouds < 1 || !req || !best_per_cloud) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_packed: bad arguments");
+// The clouds of a packed batch on the device (cs): device memory is used in place, host memory is staged piece by piece.
+// A pageable batch starts the staging thread; the caller joins it (StagerJoin) once run_jobs has returned.
+static int prepare_batch(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, CloudSet& cs) {
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     ctx->last_valid = false;
-    CloudSet cs;
     cs.stride = 12;
     cs.off.resize(n_clouds + 1);
     for (int c = 0; c <= n_clouds; c++) cs.off[c] = (long long)point_offsets[c];
@@ -2045,8 +2151,20 @@ static int batch_packed_single(haf_ctx* ctx, const float* xyz_all, const size_t*
             }
         }
     }
-    struct StagerJoin { haf_ctx* c; ~StagerJoin() { if (c->stager.active) { c->stager.th.join(); c->stager.active = false; } } } stager_join{ctx};
     cs.d_xyz = total == 0 ? nullptr : (dev ? reinterpret_cast<const unsigned char*>(xyz_all) : ctx->d_xyz.p);
+    return HAF_OK;
+}
+struct StagerJoin {
+    haf_ctx* c;
+    ~StagerJoin() { if (c->stager.active) { c->stager.th.join(); c->stager.active = false; } }
+};
+
+static int batch_packed_single(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* req,
+                               haf_best* best_per_cloud, const GraspOut* go) {
+    if (!point_offsets || n_clouds < 1 || !req || !best_per_cloud) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_packed: bad arguments");
+    CloudSet cs;
+    { const int rc = prepare_batch(ctx, xyz_all, point_offsets, n_clouds, cs); if (rc) return rc; }
+    StagerJoin stager_join{ctx};
     std::vector<Job> jobs(n_clouds);
     for (int c = 0; c < n_clouds; c++) { jobs[c].cloud = c; jobs[c].rq = *req; }
     int rc;
@@ -2073,6 +2191,78 @@ static int batch_packed_single(haf_ctx* ctx, const float* xyz_all, const size_t*
             b.rolls_done = r.rolls_done; b.n_windows_scored = r.n_windows; b.n_guard = 0;
         }
     }
+    return HAF_OK;
+}
+
+extern "C" int haf_search_batch_requests(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
+                                         const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
+                                         haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll) {
+    if (!ctx) return HAF_ERR_ARG;
+    if (!point_offsets || n_clouds < 1 || !reqs || !best_per_cloud) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_requests: bad arguments");
+    if (!grasp_per_cloud && (grasp_per_request || grasp_per_roll))
+        return ctx->fail(HAF_ERR_ARG, "haf_search_batch_requests: grasp_per_request / grasp_per_roll need grasp_per_cloud");
+    std::vector<int> one_each;
+    if (!request_offsets) {
+        one_each.resize(n_clouds + 1);
+        for (int c = 0; c <= n_clouds; c++) one_each[c] = c;
+        request_offsets = one_each.data();
+    }
+    if (request_offsets[0] != 0) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_requests: request_offsets[0] must be 0");
+    for (int c = 0; c < n_clouds; c++)
+        if (request_offsets[c + 1] <= request_offsets[c])
+            return ctx->fail(HAF_ERR_ARG, "haf_search_batch_requests: cloud %d has no request (request_offsets must increase)", c);
+    if ((long long)request_offsets[n_clouds] * ctx->R > 0x7fffffffLL) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_requests: too many requests");
+    if (ctx->group.size() > 1)
+        return group_batch_requests(ctx, xyz_all, point_offsets, n_clouds, reqs, request_offsets, best_per_cloud, best_per_request, per_roll_top,
+                                    grasp_per_cloud, grasp_per_request, grasp_per_roll);
+    return batch_requests_single(ctx, xyz_all, point_offsets, n_clouds, reqs, request_offsets, best_per_cloud, best_per_request, per_roll_top,
+                                 grasp_per_cloud, grasp_per_request, grasp_per_roll);
+}
+// request_offsets: checked, request_offsets[0] = 0
+static int batch_requests_single(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
+                                 const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
+                                 haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll) {
+    CloudSet cs;
+    { const int rc = prepare_batch(ctx, xyz_all, point_offsets, n_clouds, cs); if (rc) return rc; }
+    StagerJoin stager_join{ctx};
+    const int* ro = request_offsets;
+    const int n_reqs = ro[n_clouds], R = ctx->R;
+    std::vector<Job> jobs(n_reqs);
+    for (int c = 0; c < n_clouds; c++)
+        for (int r = ro[c]; r < ro[c + 1]; r++) { jobs[r].cloud = c; jobs[r].rq = reqs[r]; }
+    int rc;
+    {
+        GraspOut go;
+        go.per_roll = grasp_per_roll;
+        GraspScope gs(ctx, grasp_per_cloud ? &go : nullptr);
+        DeviceUnitsScope ds(ctx);
+        rc = run_jobs(ctx, cs, jobs, nullptr, nullptr, nullptr, ctx->debug_keep_batch);
+    }
+    ctx->copy_pieces = 0;
+    if (rc) return rc;
+    // per cloud what haf_search_grasps returns for its request list (n_guard aside, 0 as in the other batch calls)
+    const JobResult* res = ctx->h_results.p;
+    for (int c = 0; c < n_clouds; c++) {
+        int win = -1, wtop = -1000, rd = 0;
+        long long nw = 0;
+        for (int r = ro[c]; r < ro[c + 1]; r++) {
+            if (best_per_request) fill_best(ctx, jobs[r], res[r], r - ro[c], 0, &best_per_request[r], ctx->h_best_M.p + (size_t)r * 16);
+            if (res[r].topval > wtop) { wtop = res[r].topval; win = r; }   // strict >: the earliest request wins ties
+            nw += res[r].n_windows; rd += res[r].rolls_done;
+        }
+        if (win < 0) {
+            JobResult none; memset(&none, 0, sizeof none);
+            none.row = none.col = none.roll = -1; none.topval = -1000;
+            fill_best(ctx, jobs[ro[c]], none, -1, 0, &best_per_cloud[c]);
+        } else {
+            fill_best(ctx, jobs[win], res[win], win - ro[c], 0, &best_per_cloud[c], ctx->h_best_M.p + (size_t)win * 16);
+            best_per_cloud[c].n_windows_scored = (int)nw; best_per_cloud[c].rolls_done = rd;
+        }
+        if (grasp_per_cloud) memcpy(&grasp_per_cloud[c], ctx->h_job_grasp.p + (win < 0 ? ro[c] : win), sizeof(haf_grasp));
+    }
+    if (per_roll_top) memcpy(per_roll_top, ctx->h_per_roll_top.p, (size_t)n_reqs * R * 3 * sizeof(int));
+    if (grasp_per_request) memcpy(grasp_per_request, ctx->h_job_grasp.p, (size_t)n_reqs * sizeof(haf_grasp));
+    if (grasp_per_roll) copy_roll_grasps(ctx, jobs, grasp_per_roll);
     return HAF_OK;
 }
 
@@ -2434,9 +2624,83 @@ static int group_batch_packed(haf_ctx* ctx, const float* xyz_all, const size_t* 
     return HAF_OK;
 }
 
+// haf_search_batch_requests on several GPUs: contiguous blocks of clouds with all their requests, balanced by unit count
+// (requests x R); each member writes its records straight into the caller's arrays.
+static int group_batch_requests(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
+                                const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
+                                haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll) {
+    const int n = (int)ctx->group.size(), R = ctx->R;
+    const int* ro = request_offsets;
+    std::vector<int> cb(n + 1, n_clouds);   // member k: clouds [cb[k], cb[k + 1])
+    cb[0] = 0;
+    for (int k = 1; k < n; k++)
+        cb[k] = (int)(std::lower_bound(ro, ro + n_clouds, (int)((long long)ro[n_clouds] * k / n)) - ro);
+    std::vector<int> rcs(n, HAF_OK);
+    std::vector<std::thread> th;
+    for (int k = 0; k < n; k++) {
+        const int c0 = cb[k], c1 = cb[k + 1];
+        if (c1 <= c0) { memset(&ctx->group[k]->timing, 0, sizeof(haf_timing)); continue; }
+        th.emplace_back([=, &rcs]() {
+            haf_ctx* m = ctx->group[k];
+            std::vector<size_t> off(c1 - c0 + 1);
+            std::vector<int> rof(c1 - c0 + 1);
+            for (int c = c0; c <= c1; c++) { off[c - c0] = point_offsets[c] - point_offsets[c0]; rof[c - c0] = ro[c] - ro[c0]; }
+            const size_t r0 = (size_t)ro[c0];
+            const float* src = xyz_all + point_offsets[c0] * 3;
+            const void* use = src;
+            int rc = member_input(m, src, off[c1 - c0] * 12, &use);
+            if (rc == HAF_OK)
+                rc = batch_requests_single(m, (const float*)use, off.data(), c1 - c0, reqs + r0, rof.data(), best_per_cloud + c0,
+                                           best_per_request ? best_per_request + r0 : nullptr, per_roll_top ? per_roll_top + r0 * R * 3 : nullptr,
+                                           grasp_per_cloud ? grasp_per_cloud + c0 : nullptr, grasp_per_request ? grasp_per_request + r0 : nullptr,
+                                           grasp_per_roll ? grasp_per_roll + r0 * R : nullptr);
+            rcs[k] = rc;
+        });
+    }
+    for (size_t i = 0; i < th.size(); i++) th[i].join();
+    for (int k = 0; k < n; k++)
+        if (rcs[k] != HAF_OK) { const std::string msg = ctx->group[k]->err; return ctx->fail(rcs[k], "GPU %d: %s", ctx->group[k]->device, msg.c_str()); }
+    group_timing(ctx);
+    return HAF_OK;
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // parity / inspection entry points
 // ------------------------------------------------------------------------------------------------------------
+extern "C" int haf_debug_unit_params(haf_ctx* ctx, float* M, float* mask, float* Minv, int cap_units) {
+    if (!ctx || cap_units < 0) return HAF_ERR_ARG;
+    if (ctx->last_up_n <= 0) return ctx->fail(HAF_ERR_ARG, "haf_debug_unit_params: the context has no search to report");
+    if (Minv && !ctx->last_up_pose) return ctx->fail(HAF_ERR_ARG, "haf_debug_unit_params: the last call built no grasp poses");
+    const int U = std::min(cap_units, ctx->last_up_n), R = ctx->R;
+    if (U == 0) return 0;
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    std::vector<UnitParams> up(U);
+    CUDA_TRY(ctx, cudaMemcpy(up.data(), ctx->last_up_units, (size_t)U * sizeof(UnitParams), cudaMemcpyDeviceToHost));
+    std::vector<int> jpose;
+    std::vector<UnitPose> pose;
+    if (Minv) {
+        jpose.resize(ctx->last_up_jobs);
+        CUDA_TRY(ctx, cudaMemcpy(jpose.data(), ctx->last_up_jpose, jpose.size() * sizeof(int), cudaMemcpyDeviceToHost));
+        const int n_sets = *std::max_element(jpose.begin(), jpose.end()) + 1;
+        pose.resize((size_t)n_sets * R);
+        CUDA_TRY(ctx, cudaMemcpy(pose.data(), ctx->last_up_pose, pose.size() * sizeof(UnitPose), cudaMemcpyDeviceToHost));
+    }
+    static_assert(offsetof(UnitParams, cy4) - offsetof(UnitParams, sa) == 9 * sizeof(float), "mask constants are contiguous");
+    for (int u = 0; u < U; u++) {
+        if (M) memcpy(M + (size_t)u * 16, up[u].M, 16 * sizeof(float));
+        if (mask) memcpy(mask + (size_t)u * 10, &up[u].sa, 10 * sizeof(float));
+        if (Minv) memcpy(Minv + (size_t)u * 16, pose[(size_t)jpose[up[u].job] * R + up[u].roll].Minv, 16 * sizeof(float));
+    }
+    return U;
+}
+
+extern "C" int haf_debug_chunk_copy_waits(const haf_ctx* ctx, int* out, int cap_chunks) {
+    if (!ctx || !out || cap_chunks < 0) return HAF_ERR_ARG;
+    const int n = std::min(cap_chunks, (int)(ctx->last_chunk_waits.size() / 5));
+    memcpy(out, ctx->last_chunk_waits.data(), (size_t)n * 5 * sizeof(int));
+    return n;
+}
+
 extern "C" int haf_debug_window_count(const haf_ctx* ctx) { return (ctx && ctx->last_valid) ? (int)ctx->last_W : -1; }
 
 extern "C" int haf_debug_windows(haf_ctx* ctx, int* win_unit_cell, int cap) {
@@ -2537,7 +2801,7 @@ extern "C" int haf_debug_cell_indices(haf_ctx* ctx, const float* xyz, size_t n_p
     const float r = (float)((0.5 * (float)G) / 100.0);
     bin_maxz_kernel<4><<<dim3((unsigned)((n_points + 1023) / 1024), 1), 256, 0, ctx->stream>>>(dx, stride_bytes, ctx->d_ptoff.p, ctx->d_cloud_ubegin.p, ctx->d_units.p,
                                                                                             ctx->d_keys.p, G, r, d_cells,
-                                                                                            reinterpret_cast<unsigned long long*>(ctx->d_counters.p + 4));
+                                                                                            reinterpret_cast<unsigned long long*>(ctx->d_counters.p + 4), 0, 1);
     LAUNCHED(ctx);
     CUDA_TRY(ctx, cudaMemcpyAsync(cell_idx_host, d_cells, n_points * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));

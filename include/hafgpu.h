@@ -216,6 +216,22 @@ int haf_search_grasps(haf_ctx* ctx, const float* xyz_hostdev, size_t n_points, s
 int haf_search_batch_packed_grasps(haf_ctx* ctx, const float* xyz_all_hostdev, const size_t* point_offsets, int n_clouds,
                                    const haf_request* req, haf_best* best_per_cloud,
                                    haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_roll);
+/* Batched goals with their own requests: cloud c is searched with reqs[request_offsets[c] .. request_offsets[c+1]) (at least one
+ * request per cloud; request_offsets [n_clouds+1] starts at 0; NULL = one request per cloud), each request with its own centre,
+ * area, approach vector, gripper width, roll range and return_only_best.  For every cloud, every output equals what
+ * haf_search_grasps returns for that cloud with that request list, field for field (n_guard aside: 0, as in the other batch
+ * calls): best_per_cloud [n_clouds] is the winner over the cloud's requests (strict >, earliest request wins ties, approach_idx =
+ * index within the cloud's list, n_windows_scored / rolls_done summed over them); best_per_request [n_reqs], per_roll_top
+ * [n_reqs][R][3], grasp_per_request [n_reqs] and grasp_per_roll [n_reqs][R] (evaluated rolls only) are optional, n_reqs =
+ * request_offsets[n_clouds].  grasp_per_cloud NULL: no pose kernel runs (and the other two grasp outputs must be NULL too).
+ * Every request of a call must agree on svm_with_probability.  The same staging, chunking (on request boundaries: a cloud's
+ * requests may span two chunks), streams, CUDA graphs and multi-GPU sharding (blocks of clouds with all their requests) as
+ * haf_search_batch_packed.  The unit parameters (transforms, mask constants, inverse WCS matrices) are built on the device by one
+ * kernel per call; the host evaluates only the libm calls, once per distinct approach vector (bitwise) and per roll, so its
+ * work per call grows with the requests, not with the units.  Bit-equal to the host build of haf_search. */
+int haf_search_batch_requests(haf_ctx* ctx, const float* xyz_all_hostdev, const size_t* point_offsets, int n_clouds,
+                              const haf_request* reqs, const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request,
+                              int* per_roll_top, haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll);
 
 /* ---- PCD / PointCloud2 ingest on the device (SURVEY 8f-2) -----------------------------------------------------------
  * What the reference does on the CPU before the hot path starts: the client's pcl::io::loadPCDFile<pcl::PointXYZ>
@@ -298,6 +314,17 @@ int haf_debug_tensor_inputs(haf_ctx* ctx, float* x, int cap_windows);
 int haf_debug_decisions(haf_ctx* ctx, double* dec, int* labels, unsigned char* guard, int cap_windows);
 /* integral images [n_units][G+1][G+1] float of the last search */
 int haf_debug_integral(haf_ctx* ctx, float* integral, size_t cap_floats);
+/* unit parameters of the last search, whichever path built them (host: haf_search* / haf_search_batch_packed*; device:
+ * haf_search_batch_requests), unit u = job * R + roll: M [U][16] mat_transform (row-major), mask [U][10] pnt_in_box constants
+ * (sinf / cosf(alpha), then cx1 cy1 cx2 cy2 cx3 cy3 cx4 cy4), Minv [U][16] the inverse WCS matrix of the unit's pose (only after a
+ * call that built poses: the *_grasps entry points, or haf_search_batch_requests with grasp_per_cloud).  Any of the three may be
+ * NULL.  Returns the number of units written (<= cap_units).  On a multi-GPU context: the share of the first GPU. */
+int haf_debug_unit_params(haf_ctx* ctx, float* M, float* mask, float* Minv, int cap_units);
+/* chunks of the last search, out [n][5] = {first cloud, end cloud, stream set (0 = the call's stream), copy piece of a host-staged
+ * batch the chunk's stream waited for (-1: input in device memory), end cloud of that piece}.  Pieces are copied in order on one
+ * stream, so a chunk's clouds are all on the device once its piece is: end cloud of the piece >= end cloud of the chunk.
+ * Returns the number of chunks written (<= cap_chunks). */
+int haf_debug_chunk_copy_waits(const haf_ctx* ctx, int* out, int cap_chunks);
 /* cell index (idx_x*G+idx_y, or -1 outside the box) of every point for one request / roll */
 int haf_debug_cell_indices(haf_ctx* ctx, const float* xyz_hostdev, size_t n_points, size_t stride_bytes,
                            const haf_request* req, int roll, int* cell_idx_host);
