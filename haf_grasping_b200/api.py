@@ -77,7 +77,7 @@ EXPORTS = ["haf_create", "haf_destroy", "haf_last_error", "haf_get_info", "haf_s
            "haf_get_timing", "haf_launch_count", "haf_set_debug", "haf_search", "haf_search_batch", "haf_search_batch_packed",
            "haf_search_grasps", "haf_search_batch_packed_grasps", "haf_search_batch_requests", "haf_debug_unit_params", "haf_debug_chunk_copy_waits", "haf_build_transform", "haf_build_transform_wcs", "haf_best_key", "haf_pack_best_records", "haf_debug_window_count", "haf_debug_windows", "haf_debug_features",
            "haf_debug_decisions", "haf_debug_tensor_inputs", "haf_debug_integral", "haf_debug_cell_indices", "haf_debug_text_roundtrip", "haf_debug_tc_probe",
-           "haf_version", "haf_pcd_decode", "haf_search_pcd", "haf_pointcloud2_to_xyz", "haf_debug_pcd_xyz", "haf_svm_create", "haf_svm_destroy", "haf_svm_predict", "haf_svm_predict_probability", "haf_svm_check_probability_model", "haf_scale_minmax", "haf_scale_apply"]
+           "haf_version", "haf_pcd_decode", "haf_search_pcd", "haf_pointcloud2_to_xyz", "haf_debug_pcd_xyz", "haf_svm_create", "haf_svm_create_config", "haf_svm_destroy", "haf_svm_predict", "haf_svm_predict_probability", "haf_svm_check_probability_model", "haf_scale_minmax", "haf_scale_apply"]
 
 _lib = None
 
@@ -141,6 +141,7 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.haf_pointcloud2_to_xyz.argtypes = [vp, vp, cs, cs, ci, ci, ci, C.POINTER(vp)]
     L.haf_debug_pcd_xyz.argtypes = [vp, vp, cs]
     L.haf_svm_create.argtypes = [C.POINTER(vp), C.c_char_p, ci, ci, ci, C.c_float]
+    L.haf_svm_create_config.argtypes = [C.POINTER(vp), C.POINTER(haf_config), ci]
     L.haf_svm_destroy.argtypes = [vp]
     L.haf_svm_destroy.restype = None
     L.haf_svm_predict.argtypes = [vp, vp, vp, vp, ci, vp, vp]
@@ -203,6 +204,20 @@ def _ptr(a):
     return C.c_void_p(int(a))
 
 
+def _set_svm_knobs(cfg, svm_mode, guard_rel, tc_variant, tc_passes, audit_every, guard_tier2, guard_kernel, sv_table_global):
+    """the decision-value switches of a haf_config, shared by GraspSearch and SvmPredictor"""
+    cfg.svm_mode = svm_mode
+    cfg.guard_rel = guard_rel
+    # tc_variant: 0 auto (X-resident CTA pair where eligible), 1 single CTA, 2 streaming CTA pair; tc_passes: 0 = calibrated
+    # per model, 1-3 forced; audit_every: None = library default (every 4096th window), 0 = no sample, n = every n-th window
+    cfg.reserved[0] = tc_variant | (tc_passes << 4)
+    if audit_every is not None:
+        cfg.reserved[0] |= 0x100 if audit_every == 0 else (int(audit_every) << 16)
+    # guard_tier2: 0 on, 1 off, 2 on + escalate everything (tests); guard_kernel: 0 auto, 1 FP64 tensor cores (DMMA), 2 DFMA
+    cfg.reserved[2] = guard_tier2 | (guard_kernel << 2)
+    cfg.reserved[3] = sv_table_global   # 1: SV table read from global memory (the > 4096-SV path)
+
+
 class GraspSearch:
     """One context = one GPU.  Mirrors the reference's per-goal flow: construct once with the three files the
     action server is configured with (server.cpp:218-225), then ``search`` per goal."""
@@ -219,18 +234,9 @@ class GraspSearch:
         cfg.grid, cfg.roll_step_deg, cfg.roll_max_deg = grid, roll_step_deg, roll_max_deg
         cfg.device = device
         cfg.emulate_text_roundtrip = 1 if emulate_text_roundtrip else -1   # 0 would also mean "on" (zeroed config = reference-exact)
-        cfg.svm_mode = svm_mode
-        cfg.guard_rel = guard_rel
-        # tc_variant: 0 auto (X-resident CTA pair where eligible), 1 single CTA, 2 streaming CTA pair; tc_passes: 0 = calibrated
-        # per model, 1-3 forced; audit_every: None = library default (every 4096th window), 0 = no sample, n = every n-th window
-        cfg.reserved[0] = tc_variant | (tc_passes << 4)
-        if audit_every is not None:
-            cfg.reserved[0] |= 0x100 if audit_every == 0 else (int(audit_every) << 16)
+        _set_svm_knobs(cfg, svm_mode, guard_rel, tc_variant, tc_passes, audit_every, guard_tier2, guard_kernel, sv_table_global)
         # bin_variant: 0 auto, 1 point-parallel binning only, 2 whole-cloud kernel with scalar loads; bit 4: CUDA graph capture / replay
         cfg.reserved[1] = bin_variant | (16 if use_graph else 0)
-        # guard_tier2: 0 on, 1 off, 2 on + escalate everything (tests); guard_kernel: 0 auto, 1 FP64 tensor cores (DMMA), 2 DFMA
-        cfg.reserved[2] = guard_tier2 | (guard_kernel << 2)
-        cfg.reserved[3] = sv_table_global   # 1: SV table read from global memory (the > 4096-SV path)
         if devices is not None and len(devices) > 1:   # one context driving several GPUs (haf_config.n_devices / devices)
             self._devs = (C.c_int * len(devices))(*devices)
             cfg.n_devices, cfg.devices = len(devices), self._devs
@@ -543,16 +549,25 @@ def _csr(rows_or_dense):
 class SvmPredictor:
     """svm_predict on the GPU for a libsvm text model (C-SVC, RBF, two classes): what svm-predict-b200 binds."""
 
-    def __init__(self, model_path, device=0, svm_mode=HAF_SVM_TENSOR_GUARD, min_dims=0, guard_rel=0.0):
+    def __init__(self, model_path, device=0, svm_mode=HAF_SVM_TENSOR_GUARD, min_dims=0, guard_rel=0.0, tc_variant=0, tc_passes=0,
+                 sv_table_global=0, guard_tier2=0, guard_kernel=0, audit_every=None):
+        """the keyword arguments after min_dims mean what they mean for GraspSearch"""
         self.L = load_library()
         self.h = C.c_void_p()
-        rc = self.L.haf_svm_create(C.byref(self.h), model_path.encode(), device, svm_mode, min_dims, guard_rel)
+        cfg = haf_config()
+        self._model = model_path.encode()
+        cfg.model_path = self._model
+        cfg.device = device
+        _set_svm_knobs(cfg, svm_mode, guard_rel, tc_variant, tc_passes, audit_every, guard_tier2, guard_kernel, sv_table_global)
+        rc = self.L.haf_svm_create_config(C.byref(self.h), C.byref(cfg), min_dims)
         if rc != 0:
             raise HafError(rc, (self.L.haf_last_error(None) or b"").decode())
         self.info = haf_info()
         self.L.haf_get_info(self.h, C.byref(self.info))
 
     def predict(self, rows, want_dec=True):
+        """(labels [n], decision values [n] or None); afterwards info.reserved[2] / [3] name the contraction kernel that ran
+        and its support-vector split"""
         rp, idx, val = _csr(rows)
         n = len(rp) - 1
         labels = np.zeros(max(n, 1), np.float64)
@@ -560,6 +575,7 @@ class SvmPredictor:
         rc = self.L.haf_svm_predict(self.h, _ptr(rp), _ptr(idx), _ptr(val), n, _ptr(labels), _ptr(dec))
         if rc != 0:
             raise HafError(rc, (self.L.haf_last_error(self.h) or b"").decode())
+        self.L.haf_get_info(self.h, C.byref(self.info))
         return labels[:n], (dec[:n] if want_dec else None)
 
     def check_probability_model(self):
@@ -574,6 +590,7 @@ class SvmPredictor:
         rc = self.L.haf_svm_predict_probability(self.h, _ptr(rp), _ptr(idx), _ptr(val), n, _ptr(labels), _ptr(probs))
         if rc != 0:
             raise HafError(rc, (self.L.haf_last_error(self.h) or b"").decode())
+        self.L.haf_get_info(self.h, C.byref(self.info))
         return labels[:n], probs[:n]
 
     def timing(self):

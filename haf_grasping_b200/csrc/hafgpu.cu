@@ -121,6 +121,9 @@ struct haf_ctx {
     int tc_variant = 0;         // 0: auto (X-resident CTA-pair kernel where eligible, else streaming CTA pair), 2: streaming CTA pair always
     int tc_passes = 3;          // tensor-core products per k-slice: 3, 2 or 1 (calibrate_tensor_passes)
     double tc_operand_err = 0;  // calibrated operand error of the chosen scheme, as a fraction of the guard scale E
+    int last_svm_kernel = 0;    // contraction kernel of the last stage-5 launch (haf_info.reserved[2]): 0 none / FP64 exact, 1 tc3, 2 tc2, 3 SIMT
+    int last_nsplit2 = 0;       // its SV-tile split (haf_info.reserved[3]; 0 outside the tensor kernels)
+    int smem_optin = 0;         // the device's opt-in shared memory per block
 
     // per-call state
     DevBuf<unsigned char> d_xyz;       // staging for host clouds
@@ -522,6 +525,7 @@ static int create_impl(haf_ctx** out, const haf_config* cfg, bool svm_only, int 
     ctx->cfg.grid = G; ctx->cfg.roll_step_deg = step; ctx->cfg.roll_max_deg = rmax; ctx->cfg.nr_features_without_shaf = nshaf;
     ctx->device = cfg->device;
     ctx->sm_count = prop.multiProcessorCount;
+    ctx->smem_optin = (int)prop.sharedMemPerBlockOptin;
     ctx->F = F; ctx->D = D; ctx->Dsv = Dsv; ctx->Kpad = Kpad; ctx->S = S; ctx->Spad = Spad; ctx->R = R; ctx->G = G;
     for (int roll = 0; roll < R; roll++) ctx->roll_trig.push_back(hafhost::roll_trig(roll, step));
     ctx->lower = range.lower; ctx->upper = range.upper; ctx->gamma = model.gamma; ctx->rho = model.rho;
@@ -621,7 +625,15 @@ static int create_impl(haf_ctx** out, const haf_config* cfg, bool svm_only, int 
     CREATE_TRY(cudaFuncSetAttribute(guard_fma_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
     CREATE_TRY(cudaFuncSetAttribute(svm_rbf_simt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SVM_STAGES * SVM_BK * (SVM_BM + SVM_BN) * 4));
     CREATE_TRY(cudaFuncSetAttribute(integral_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    CREATE_TRY(cudaFuncSetAttribute(svm_exact_terms_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
+    {   // the exact-order kernel stages the inputs of HAF_EXACT_WB windows (Dsv doubles each) in shared memory; a model too wide
+        // for the device's opt-in maximum reads them from global memory instead (launch_exact).  The limit is only ever raised:
+        // it is per function, and a context made earlier may need more than this one.
+        const size_t need = (size_t)HAF_EXACT_WB * Dsv * sizeof(double);
+        cudaFuncAttributes fa;
+        CREATE_TRY(cudaFuncGetAttributes(&fa, svm_exact_terms_kernel));
+        const int want = (int)std::max<size_t>(100 * 1024, need <= (size_t)ctx->smem_optin ? need : 0);
+        if (want > fa.maxDynamicSharedSizeBytes) CREATE_TRY(cudaFuncSetAttribute(svm_exact_terms_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, want));
+    }
     CREATE_TRY(cudaFuncSetAttribute(bin_maxz_cloud_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     CREATE_TRY(cudaFuncSetAttribute(bin_maxz_cloud_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     if (cfg->svm_mode == HAF_SVM_TENSOR_GUARD) {
@@ -784,6 +796,15 @@ extern "C" int haf_create(haf_ctx** out, const haf_config* cfg) {
 
 // ---- libsvm front ends (SURVEY 8f-3) -------------------------------------------------------------------------
 static int svm_stage(haf_ctx* ctx, unsigned* cnt, size_t Wcap, size_t ldx, int G, int ubase, cudaStream_t st, cudaEvent_t ev_guard);
+extern "C" int haf_svm_create_config(haf_svm** out, const haf_config* cfg, int min_dims) {
+    if (!out || !cfg) return create_fail(HAF_ERR_ARG, "haf_svm_create_config: null argument");
+    haf_config one = *cfg;
+    one.features_path = one.range_path = nullptr;
+    one.n_devices = 0; one.devices = nullptr;
+    const int rc = create_impl(out, &one, true, min_dims);
+    if (rc == HAF_OK) (*out)->svm_only = true;
+    return rc;
+}
 extern "C" int haf_svm_create(haf_svm** out, const char* model_path, int device, int svm_mode, int min_dims, float guard_rel) {
     haf_config cfg;
     memset(&cfg, 0, sizeof cfg);
@@ -791,9 +812,7 @@ extern "C" int haf_svm_create(haf_svm** out, const char* model_path, int device,
     cfg.device = device;
     cfg.svm_mode = svm_mode;
     cfg.guard_rel = guard_rel;
-    const int rc = create_impl(out, &cfg, true, min_dims);
-    if (rc == HAF_OK) (*out)->svm_only = true;
-    return rc;
+    return haf_svm_create_config(out, &cfg, min_dims);
 }
 extern "C" void haf_svm_destroy(haf_svm* s) { haf_destroy(s); }
 
@@ -1047,6 +1066,8 @@ extern "C" int haf_get_info(const haf_ctx* ctx, haf_info* info) {
     info->gamma = ctx->gamma; info->rho = ctx->rho;
     info->reserved[0] = ctx->cfg.svm_mode == HAF_SVM_TENSOR_GUARD ? ctx->tc_passes : 0;   // tensor-core products per k-slice
     info->reserved[1] = (int)lrint(ctx->guard_rel * 1e9);                                  // guard_rel in units of 1e-9
+    info->reserved[2] = ctx->last_svm_kernel;                                              // what the last stage-5 launch ran
+    info->reserved[3] = ctx->last_nsplit2;
     return HAF_OK;
 }
 extern "C" int haf_set_stream(haf_ctx* ctx, void* s) { if (!ctx) return HAF_ERR_ARG; ctx->stream = (cudaStream_t)s; return HAF_OK; }
@@ -1123,15 +1144,19 @@ bool is_device_ptr(const void* p) {
 }  // namespace
 
 static size_t ft_smem_bytes(const haf_ctx* ctx) { return ft_smem_layout(ctx->G, ctx->tc_passes >= 3 ? 2 : 1); }
-static size_t exact_smem_bytes(const haf_ctx* ctx) { return (size_t)HAF_EXACT_WB * ctx->Dsv * sizeof(double); }
 // launches the two phases of the FP64 exact-order path on stream st
 static int launch_exact(haf_ctx* ctx, ExactArgs a, cudaStream_t st, size_t max_windows) {
     const int slices = (ctx->S + HAF_EXACT_SLICE - 1) / HAF_EXACT_SLICE;
+    // inputs of HAF_EXACT_WB windows in shared memory where they fit (create_impl raised the kernel's limit), else from global memory
+    const size_t smem = (size_t)HAF_EXACT_WB * ctx->Dsv * sizeof(double);
+    a.x_global = smem > (size_t)ctx->smem_optin ? 1 : 0;
     // all-windows mode (list == NULL) walks the windows in passes of max_entries; guard mode is a single pass
     const size_t passes = a.list ? 1 : (max_windows + a.max_entries - 1) / (size_t)a.max_entries;
     for (size_t p = 0; p < passes; p++) {
         a.entry_begin = (int)(p * (size_t)a.max_entries);
-        svm_exact_terms_kernel<<<dim3((unsigned)(ctx->sm_count * 2), (unsigned)slices), 256, exact_smem_bytes(ctx), st>>>(a);
+        const dim3 grid((unsigned)(ctx->sm_count * 2), (unsigned)slices);
+        if (a.x_global) svm_exact_terms_xglobal_kernel<<<grid, 256, 0, st>>>(a);
+        else svm_exact_terms_kernel<<<grid, 256, smem, st>>>(a);
         LAUNCHED(ctx);
         svm_exact_sum_kernel<<<ctx->sm_count * 4, 128, 0, st>>>(a);
         LAUNCHED(ctx);
@@ -1193,6 +1218,7 @@ static ExactArgs make_exact_args(haf_ctx* ctx, const int* list, const unsigned* 
     a.entry_begin = 0;
     a.overflow_flag = list ? (int*)(cnt + 10) : nullptr;   // guard mode: one launch must cover the whole list
     a.xdense = ctx->cur_xdense;
+    a.x_global = 0;   // launch_exact decides
     return a;
 }
 
@@ -1207,6 +1233,8 @@ static int tc_debug_flags() {
 static int svm_stage(haf_ctx* ctx, unsigned* cnt, size_t Wcap, size_t ldx, int G, int ubase, cudaStream_t st, cudaEvent_t ev_guard) {
     const bool tc = ctx->cfg.svm_mode == HAF_SVM_TENSOR_GUARD && !ctx->force_exact;
     const float neg_gamma_log2e = (float)(-ctx->gamma * 1.4426950408889634);
+    ctx->last_svm_kernel = 0;
+    ctx->last_nsplit2 = 0;
     if (ctx->cfg.svm_mode == HAF_SVM_FP64_EXACT || ctx->force_exact) {
         CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_guardflag.p, 0, ldx, st));
         { int rce = launch_exact(ctx, make_exact_args(ctx, nullptr, nullptr, cnt, G, ubase), st, Wcap); if (rce) return rce; }
@@ -1246,6 +1274,8 @@ static int svm_stage(haf_ctx* ctx, unsigned* cnt, size_t Wcap, size_t ldx, int G
             int stages3 = 0;
             if (ctx->tc_variant == 0 && ctx->tc_passes == 1 && kblocks <= haftc::XK_MAX)
                 stages3 = std::min(8, (haftc::TC3_SMEM_LIMIT - haftc::tc3_smem_bytes(kblocks, 0, (int)(tab_bytes / 4))) / (haftc::KBS * haftc::B2_TILE_BYTES));
+            ctx->last_svm_kernel = stages3 >= 2 ? 1 : 2;
+            ctx->last_nsplit2 = nsplit2;
             if (stages3 >= 2 && (tc_debug_flags() & 64))   // experiment: four epilogue warps per TMEM lane quarter
                 haftc::svm_rbf_tc3_kernel<4><<<grid2, 64 + 128 * 4, haftc::tc3_smem_bytes(kblocks, stages3, (int)(tab_bytes / 4)), st>>>(
                     tmXh, ctx->tmSh2, ctx->d_xn.p, ctx->d_svcoef.p, ctx->c_log2, cnt + 0, n_ntiles, nsplit2, kblocks, last_slices, stages3, ctx->d_dec.p,
@@ -1271,6 +1301,7 @@ static int svm_stage(haf_ctx* ctx, unsigned* cnt, size_t Wcap, size_t ldx, int G
         if (ev_guard) CUDA_TRY(ctx, cudaEventRecord(ev_guard, st));
         { int rce = launch_guard(ctx, cnt, G, ubase, st, Wcap, ldx); if (rce) return rce; }
     } else {
+        ctx->last_svm_kernel = 3;
         svm_rbf_simt_kernel<<<(unsigned)(ldx / SVM_BM), 256, SVM_STAGES * SVM_BK * (SVM_BM + SVM_BN) * 4, st>>>(
             ctx->d_X.p, ldx, ctx->d_svT.p, ctx->Spad, ctx->Kpad, ctx->d_xn.p, ctx->d_svn.p, ctx->d_coef.p, neg_gamma_log2e, ctx->rho,
             ctx->guard_rel, ctx->e_floor, cnt + 0, ctx->d_dec.p, ctx->d_guardflag.p, ctx->d_guardlist.p, cnt + 1);

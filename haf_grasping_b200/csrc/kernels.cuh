@@ -1109,6 +1109,7 @@ struct ExactArgs {
     int entry_begin;      // this launch covers list entries [entry_begin, entry_begin + max_entries)
     int max_entries;      // capacity of `terms` in windows
     const double* xdense; // haf_svm_predict: the SVM inputs are GIVEN ([window][Dsv] doubles) instead of derived from a cloud
+    int x_global;         // 1: the inputs of HAF_EXACT_WB windows do not fit in shared memory (svm_exact_terms_xglobal_kernel)
 };
 // SVM input d of window w, re-derived in double from the integral image with the bit-exact emulation of both text round
 // trips (a7-a9: calc_featurevalue, "%.4g", svm-scale.c:339-352 with "%g"): exactly what svm-predict parses.
@@ -1139,22 +1140,26 @@ __device__ __forceinline__ double exact_scaled_input(const ExactArgs& A, int w, 
 // grid = (window blocks, SV slices).  x is re-derived in double from the integral image with the bit-exact emulation of
 // both text round trips; K_i = exp(-gamma * sum_d (x_d - sv_i,d)^2) with the d loop sequential and un-fused
 // (Kernel::k_function, svm.cpp:326-365: absent entries are zeros, adding 0.0 is exact).  WB = 8 windows share every SV
-// element (throughput); WB = 1 spreads a short list over many CTAs (latency of a single goal).
-template <int WB>
+// element (throughput); WB = 1 spreads a short list over many CTAs (latency of a single goal).  XG (models too wide for
+// the shared-memory copy, WB = 1 only): every thread reads x_d in place -- one broadcast load per d.
+template <int WB, bool XG = false>
 __device__ __forceinline__ void svm_exact_terms_body(const ExactArgs& A, double* xs, unsigned n) {
     const int Dsv = A.Dsv, Spad = A.Spad;
     const int i0 = blockIdx.y * HAF_EXACT_SLICE;
     if (i0 >= A.S) return;
     for (unsigned e0 = A.entry_begin + blockIdx.x * WB; e0 < n; e0 += gridDim.x * WB) {
         const int nb = min((unsigned)WB, n - e0);
-        __syncthreads();
-        for (int t = threadIdx.x; t < WB * Dsv; t += blockDim.x) {
-            const int b = t / Dsv, d = t - b * Dsv;
-            double x = 0.0;
-            if (b < nb && d < A.D) x = exact_scaled_input(A, A.list ? A.list[e0 + b] : (int)(e0 + b), d);
-            xs[t] = x;
+        const int w0 = XG ? (A.list ? A.list[e0] : (int)e0) : 0;   // XG: the one window of this step
+        if (!XG) {
+            __syncthreads();
+            for (int t = threadIdx.x; t < WB * Dsv; t += blockDim.x) {
+                const int b = t / Dsv, d = t - b * Dsv;
+                double x = 0.0;
+                if (b < nb && d < A.D) x = exact_scaled_input(A, A.list ? A.list[e0 + b] : (int)(e0 + b), d);
+                xs[t] = x;
+            }
+            __syncthreads();
         }
-        __syncthreads();
         double sum[WB][HAF_EXACT_SVT];
 #pragma unroll
         for (int b = 0; b < WB; b++)
@@ -1167,7 +1172,7 @@ __device__ __forceinline__ void svm_exact_terms_body(const ExactArgs& A, double*
             for (int k = 0; k < HAF_EXACT_SVT; k++) sv[k] = A.sv64T[(size_t)d * Spad + ia + 256 * k];
 #pragma unroll
             for (int b = 0; b < WB; b++) {
-                const double xb = xs[b * Dsv + d];
+                const double xb = XG ? (d < A.D ? exact_scaled_input(A, w0, d) : 0.0) : xs[b * Dsv + d];
 #pragma unroll
                 for (int k = 0; k < HAF_EXACT_SVT; k++) {
                     const double diff = __dsub_rn(xb, sv[k]);
@@ -1194,6 +1199,14 @@ __global__ void __launch_bounds__(256) svm_exact_terms_kernel(const ExactArgs A)
     if (n <= (unsigned)A.entry_begin) return;
     if (n - A.entry_begin >= (unsigned)gridDim.x * 2u) svm_exact_terms_body<HAF_EXACT_WB>(A, xs, n);
     else svm_exact_terms_body<1>(A, xs, n);
+}
+// the same for models whose inputs of HAF_EXACT_WB windows do not fit in shared memory (ExactArgs.x_global): one window per
+// CTA step, x read in place (a kernel of its own, so that the register allocation of the one above stays as it is)
+__global__ void __launch_bounds__(256) svm_exact_terms_xglobal_kernel(const ExactArgs A) {
+    unsigned n = A.list ? *A.list_count : *A.win_count;
+    n = min(n, (unsigned)(A.entry_begin + A.max_entries));
+    if (n <= (unsigned)A.entry_begin) return;
+    svm_exact_terms_body<1, true>(A, nullptr, n);
 }
 // Phase 2: dec = (sum of the terms in FILE ORDER, one sequential chain) - rho   (svm.cpp:2500-2514).  One warp per
 // entry: 32 terms are fetched with one coalesced load and broadcast lane by lane, every lane runs the same chain.

@@ -125,7 +125,11 @@ typedef struct {
     int label0, label1; /* model label order (svm.cpp:2516-2531)                                              */
     int sm_count;
     double gamma, rho;
-    int reserved[4];  /* [0]: tensor-core products per k-slice in use (1-3; 0 outside tensor mode); [1]: guard_rel * 1e9 */
+    int reserved[4];  /* [0]: tensor-core products per k-slice in use (1-3; 0 outside tensor mode); [1]: guard_rel * 1e9;
+                         [2]: contraction kernel of the context's last decision-value launch (haf_search* / haf_svm_predict*):
+                              0 none / FP64 exact order, 1 svm_rbf_tc3_kernel (X-resident pair), 2 svm_rbf_tc2_kernel (streaming
+                              pair), 3 FP32 SIMT -- tc3 falls back to tc2 where the X tile, ring and table do not fit;
+                         [3]: that launch's split of the support-vector tiles per work item (tensor kernels; 0 otherwise) */
 } haf_info;
 
 typedef struct {
@@ -263,6 +267,10 @@ typedef struct haf_ctx haf_svm;
 /* model only (C-SVC, RBF, 2 classes: what svm_load_model reads for this path, svm.cpp:2714-2927).  min_dims: largest
  * feature index the data will carry (the distance loop covers max(model, data) dimensions, svm.cpp:328-364). */
 int haf_svm_create(haf_svm** out, const char* model_path, int device, int svm_mode, int min_dims, float guard_rel);
+/* the same, with every knob of the config: model_path, device, svm_mode, guard_rel and the reserved[] switches: tensor kernel,
+ * products per k-slice, audit, guard tier 2 and its kernel, global coef table.  features_path, range_path, n_devices and
+ * devices are ignored.  haf_svm_create(...) is haf_svm_create_config with a zeroed config carrying its four arguments. */
+int haf_svm_create_config(haf_svm** out, const haf_config* cfg, int min_dims);
 void haf_svm_destroy(haf_svm* s);
 /* svm_predict for every row (svm.cpp:2535-2548): labels [n_rows] (as doubles, what svm-predict prints with %g) and,
  * optionally, the decision values [n_rows] (svm_predict_values, svm.cpp:2459-2533).  Labels equal libsvm's; decision
