@@ -15,6 +15,7 @@ from . import build as _build
 HAF_SVM_TENSOR_GUARD = 0
 HAF_SVM_FP64_EXACT = 1
 HAF_SVM_FP32_GUARD = 2
+CHUNK_RECORD = 10   # ints per chunk of haf_debug_chunk_copy_waits (HAF_CHUNK_RECORD)
 
 
 class HafError(RuntimeError):
@@ -70,12 +71,12 @@ class haf_timing(C.Structure):
                 ("n_points", C.c_longlong), ("n_units", C.c_longlong), ("n_windows", C.c_longlong),
                 ("n_guard", C.c_longlong), ("launches", C.c_longlong), ("n_chunks", C.c_longlong),
                 ("n_exact", C.c_longlong), ("n_audit", C.c_longlong), ("audit_max_rel", C.c_float), ("tc_passes", C.c_int),
-                ("escalations", C.c_int), ("graph_replays", C.c_int)]
+                ("escalations", C.c_int), ("graph_replays", C.c_int), ("n_clamped", C.c_longlong)]
 
 
 EXPORTS = ["haf_create", "haf_destroy", "haf_last_error", "haf_get_info", "haf_set_stream", "haf_set_profiling",
            "haf_get_timing", "haf_launch_count", "haf_set_debug", "haf_search", "haf_search_batch", "haf_search_batch_packed",
-           "haf_search_grasps", "haf_search_batch_packed_grasps", "haf_search_batch_requests", "haf_debug_unit_params", "haf_debug_chunk_copy_waits", "haf_build_transform", "haf_build_transform_wcs", "haf_best_key", "haf_pack_best_records", "haf_debug_window_count", "haf_debug_windows", "haf_debug_features",
+           "haf_search_grasps", "haf_search_batch_packed_grasps", "haf_search_batch_requests", "haf_debug_unit_params", "haf_debug_chunk_copy_waits", "haf_debug_heights", "haf_build_transform", "haf_build_transform_wcs", "haf_best_key", "haf_pack_best_records", "haf_debug_window_count", "haf_debug_windows", "haf_debug_features",
            "haf_debug_decisions", "haf_debug_tensor_inputs", "haf_debug_integral", "haf_debug_cell_indices", "haf_debug_text_roundtrip", "haf_debug_tc_probe",
            "haf_version", "haf_pcd_decode", "haf_search_pcd", "haf_pointcloud2_to_xyz", "haf_debug_pcd_xyz", "haf_svm_create", "haf_svm_create_config", "haf_svm_destroy", "haf_svm_predict", "haf_svm_predict_probability", "haf_svm_check_probability_model", "haf_scale_minmax", "haf_scale_apply"]
 
@@ -121,6 +122,7 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
                                             C.POINTER(haf_best), vp, C.POINTER(haf_grasp), C.POINTER(haf_grasp), C.POINTER(haf_grasp)]
     L.haf_debug_unit_params.argtypes = [vp, vp, vp, vp, ci]
     L.haf_debug_chunk_copy_waits.argtypes = [vp, vp, ci]
+    L.haf_debug_heights.argtypes = [vp, vp, cs]
     L.haf_build_transform.argtypes = [C.POINTER(haf_request), ci, ci, C.POINTER(C.c_float)]
     L.haf_build_transform_wcs.argtypes = [C.POINTER(haf_request), ci, ci, C.POINTER(C.c_float)]
     L.haf_best_key.argtypes = [ci, C.c_uint32]
@@ -413,10 +415,12 @@ class GraspSearch:
         return M[:U], mask[:U], (Minv[:U] if poses else None)
 
     def debug_chunk_copy_waits(self):
-        """chunks of the last search (haf_debug_chunk_copy_waits): int32 [n, 5] = first cloud, end cloud, stream set, copy piece
-        waited for (-1: device input), end cloud of that piece"""
+        """chunks of the last search (haf_debug_chunk_copy_waits): int32 [n, 10] = first cloud, end cloud, stream set, copy piece
+        waited for (-1: device input), end cloud of that piece, binning kernel (0 point-parallel, 1 whole-cloud with 16-byte loads,
+        2 whole-cloud with scalar loads), unit groups, units per group, slices (whole-cloud kernel; 0 otherwise), integral image
+        (0 one kernel, 1 row + column passes)"""
         t = self.timing()
-        out = np.zeros((max(int(t.n_chunks), 1), 5), np.int32)
+        out = np.zeros((max(int(t.n_chunks), 1), CHUNK_RECORD), np.int32)
         n = self._check(self.L.haf_debug_chunk_copy_waits(self.h, _ptr(out), len(out)))
         return out[:n]
 
@@ -500,6 +504,12 @@ class GraspSearch:
         g = np.zeros(max(W, 1), np.uint8)
         self._check(self.L.haf_debug_decisions(self.h, _ptr(d), _ptr(lab), _ptr(g), W))
         return d[:W], lab[:W], g[:W]
+
+    def debug_heights(self, n_units):
+        """decoded height grids [n_units, G, G] of the last search (haf_debug_heights); only active units are defined"""
+        a = np.zeros((n_units, self.G, self.G), np.float32)
+        self._check(self.L.haf_debug_heights(self.h, _ptr(a), a.size))
+        return a
 
     def debug_integral(self, n_units):
         a = np.zeros((n_units, self.G + 1, self.G + 1), np.float32)

@@ -244,7 +244,7 @@ struct haf_ctx {
     const int* last_up_jpose = nullptr;       // [n_jobs] pose set of each job
     int last_up_n = 0, last_up_jobs = 0;
     // per chunk of the last call: first cloud, end cloud, stream set, copy piece its stream waited for (-1: none), that piece's
-    // end cloud (haf_debug_chunk_copy_waits)
+    // end cloud, then binning kernel, unit groups, units per group, slices and integral variant (haf_debug_chunk_copy_waits)
     std::vector<int> last_chunk_waits;
 
     // probability estimates (SURVEY 8f-4): the model's sigmoid (svm.cpp:2811-2824); probability calls evaluate EVERY row /
@@ -1666,10 +1666,9 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
             }
             CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->copy_ev[last_piece], 0));
         }
-        {
-            const int w[5] = {c0, c1, set, ctx->copy_pieces > 0 ? last_piece : -1, ctx->copy_pieces > 0 ? ctx->copy_cloud_end[last_piece] : -1};
-            ctx->last_chunk_waits.insert(ctx->last_chunk_waits.end(), w, w + 5);
-        }
+        // the chunk's record (haf_debug_chunk_copy_waits): its clouds and copy wait, then the binning and integral launches it made
+        int rec[HAF_CHUNK_RECORD] = {c0, c1, set, ctx->copy_pieces > 0 ? last_piece : -1, ctx->copy_pieces > 0 ? ctx->copy_cloud_end[last_piece] : -1,
+                                     0, 0, 0, 0, smallG ? 0 : 1};
         // 1. binning
         if (prof) CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[ci * 8 + 0], st));
         {
@@ -1701,7 +1700,9 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
                     }
                 }
                 dim3 gridc((unsigned)(c1 - c0), (unsigned)((max_units_per_cloud + ug - 1) / ug), (unsigned)slices);
-                if (cs.stride == 12 && (ctx->cfg.reserved[1] & 15) != 2)
+                const bool vec4 = cs.stride == 12 && (ctx->cfg.reserved[1] & 15) != 2;
+                rec[5] = vec4 ? 1 : 2; rec[6] = (int)gridc.y; rec[7] = ug; rec[8] = slices;
+                if (vec4)
                     bin_maxz_cloud_kernel<4><<<gridc, 1024, (size_t)ug * GG * 4, st>>>(cs.d_xyz, cs.stride, d_ptoff + c0, d_cloud_ubegin + c0, d_units,
                                                                                      ctx->d_keys.p - (size_t)ubase * GG, G, r, ug,
                                                                                      reinterpret_cast<unsigned long long*>(cnt + 4), ubase, ubase + Uc);
@@ -1724,6 +1725,7 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
                 }
             }
         }
+        ctx->last_chunk_waits.insert(ctx->last_chunk_waits.end(), rec, rec + HAF_CHUNK_RECORD);
         // 2. integral image
         if (prof) CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[ci * 8 + 1], st));
         if (smallG) {
@@ -1888,6 +1890,11 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     t.tc_passes = ctx->cfg.svm_mode == HAF_SVM_TENSOR_GUARD ? ctx->tc_passes : 0;
     t.escalations = ctx->escalations;
     t.graph_replays = (int)std::min<long long>(ctx->graph_replays, 0x7fffffff);
+    {   // d_counters[4..5]: points clamped into row / column G - 1 (both binning kernels; zeroed above, merged across streams)
+        unsigned long long clamped;
+        memcpy(&clamped, &ctx->h_counters.p[4], sizeof clamped);
+        t.n_clamped = (long long)clamped;
+    }
     if (keep_debug_state) { ctx->last_W = (unsigned)total_windows; ctx->last_valid = true; }
     ctx->last_up_units = d_units; ctx->last_up_pose = grasp ? d_pose : nullptr; ctx->last_up_jpose = d_jpose;
     ctx->last_up_n = U; ctx->last_up_jobs = n_jobs;
@@ -2498,7 +2505,7 @@ static void group_timing(haf_ctx* ctx) {
         t.ms_features = std::max(t.ms_features, c.ms_features); t.ms_svm = std::max(t.ms_svm, c.ms_svm); t.ms_guard = std::max(t.ms_guard, c.ms_guard);
         t.ms_score = std::max(t.ms_score, c.ms_score);
         t.n_points += c.n_points; t.n_units += c.n_units; t.n_windows += c.n_windows; t.n_guard += c.n_guard; t.launches += c.launches;
-        t.n_chunks += c.n_chunks; t.n_exact += c.n_exact; t.n_audit += c.n_audit;
+        t.n_chunks += c.n_chunks; t.n_exact += c.n_exact; t.n_audit += c.n_audit; t.n_clamped += c.n_clamped;
         t.audit_max_rel = std::max(t.audit_max_rel, c.audit_max_rel); t.tc_passes = std::max(t.tc_passes, c.tc_passes); t.escalations += c.escalations;
     }
     ctx->timing = t;
@@ -2727,9 +2734,19 @@ extern "C" int haf_debug_unit_params(haf_ctx* ctx, float* M, float* mask, float*
 
 extern "C" int haf_debug_chunk_copy_waits(const haf_ctx* ctx, int* out, int cap_chunks) {
     if (!ctx || !out || cap_chunks < 0) return HAF_ERR_ARG;
-    const int n = std::min(cap_chunks, (int)(ctx->last_chunk_waits.size() / 5));
-    memcpy(out, ctx->last_chunk_waits.data(), (size_t)n * 5 * sizeof(int));
+    const int n = std::min(cap_chunks, (int)(ctx->last_chunk_waits.size() / HAF_CHUNK_RECORD));
+    memcpy(out, ctx->last_chunk_waits.data(), (size_t)n * HAF_CHUNK_RECORD * sizeof(int));
     return n;
+}
+
+// the heights are decoded in place in d_keys by the integral kernels, so they stay there until the next search
+extern "C" int haf_debug_heights(haf_ctx* ctx, float* heights, size_t cap_floats) {
+    if (!ctx || !ctx->last_valid || !heights) return HAF_ERR_ARG;
+    const size_t n = (size_t)ctx->last_units * ctx->G * ctx->G;
+    if (cap_floats < n) return ctx->fail(HAF_ERR_ARG, "haf_debug_heights: buffer too small");
+    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+    CUDA_TRY(ctx, cudaMemcpy(heights, ctx->d_keys.p, n * sizeof(float), cudaMemcpyDeviceToHost));
+    return ctx->last_units;
 }
 
 extern "C" int haf_debug_window_count(const haf_ctx* ctx) { return (ctx && ctx->last_valid) ? (int)ctx->last_W : -1; }

@@ -176,11 +176,13 @@ __device__ __forceinline__ void bin_points_into_units(const float (&x)[VEC], con
             const float tx = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m0.x, x[k]), __fmul_rn(m0.y, y[k])), __fmul_rn(m0.z, z[k])), m0.w);
             const float ty = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m1.x, x[k]), __fmul_rn(m1.y, y[k])), __fmul_rn(m1.z, z[k])), m1.w);
             // -r < t < r  <=>  |t| < r, exactly (both false for NaN): strict (server.cpp:510-511)
-            const bool in = fabsf(tx) < r && fabsf(ty) < r && keyz[k] != 0u;
+            const bool inbox = fabsf(tx) < r && fabsf(ty) < r;
+            const bool in = inbox && keyz[k] != 0u;
             int ix = __float2int_rd(__fmul_rn(100.0f, __fadd_rn(tx, r)));  // :513  (int)floorf(.)
             int iy = __float2int_rd(__fmul_rn(100.0f, __fadd_rn(ty, r)));  // :514
-            // t > -r makes t + r >= 0, so an index of a point inside cannot be negative; rounding can push one to G (t just below r)
-            if (in && max(ix, iy) > Gm1) atomicAdd(clamp_count, 1ull);
+            // t > -r makes t + r >= 0, so an index of a point inside cannot be negative; rounding can push one to G (t just below r).
+            // Counted whatever its z, as the reference and bin_maxz_kernel count it: the clamp precedes the height test (:513-518)
+            if (inbox && max(ix, iy) > Gm1) atomicAdd(clamp_count, 1ull);
             ix = min(max(ix, 0), Gm1);
             iy = min(max(iy, 0), Gm1);
             const int cell = ix * G + iy;

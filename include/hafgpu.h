@@ -143,6 +143,9 @@ typedef struct {
     int tc_passes;      /* tensor-core products per k-slice the call ended with (0 outside tensor mode)           */
     int escalations;    /* times this context repeated a call with more products because the audit left < 4x     */
     int graph_replays;  /* calls of this context served by replaying its captured CUDA graph (reserved[1] bit 4)      */
+    long long n_clamped; /* points of the call inside the box whose cell index floor(100 (t + r)) reached G and was clamped
+                            to G - 1 (summed over units; the reference clamps and counts them the same way).  0 at G = 56;
+                            a point a few ulps inside +r reaches it at many other grid sides */
 } haf_timing;
 
 /* ---- lifetime --------------------------------------------------------------------------------------------- */
@@ -328,11 +331,19 @@ int haf_debug_integral(haf_ctx* ctx, float* integral, size_t cap_floats);
  * call that built poses: the *_grasps entry points, or haf_search_batch_requests with grasp_per_cloud).  Any of the three may be
  * NULL.  Returns the number of units written (<= cap_units).  On a multi-GPU context: the share of the first GPU. */
 int haf_debug_unit_params(haf_ctx* ctx, float* M, float* mask, float* Minv, int cap_units);
-/* chunks of the last search, out [n][5] = {first cloud, end cloud, stream set (0 = the call's stream), copy piece of a host-staged
- * batch the chunk's stream waited for (-1: input in device memory), end cloud of that piece}.  Pieces are copied in order on one
- * stream, so a chunk's clouds are all on the device once its piece is: end cloud of the piece >= end cloud of the chunk.
+/* chunks of the last search, out [n][HAF_CHUNK_RECORD = 10] = {first cloud, end cloud, stream set (0 = the call's stream), copy
+ * piece of a host-staged batch the chunk's stream waited for (-1: input in device memory), end cloud of that piece, binning kernel
+ * (0 point-parallel, 1 whole-cloud with 16-byte loads, 2 whole-cloud with scalar loads), unit groups per cloud, units per group,
+ * slices per cloud (the last three: the whole-cloud kernel's grid; 0 for the point-parallel kernel), integral image (0 one kernel
+ * per unit with the tile in shared memory, 1 row pass + column pass)}.  Pieces are copied in order on one stream, so a chunk's
+ * clouds are all on the device once its piece is: end cloud of the piece >= end cloud of the chunk.
  * Returns the number of chunks written (<= cap_chunks). */
+#define HAF_CHUNK_RECORD 10
 int haf_debug_chunk_copy_waits(const haf_ctx* ctx, int* out, int cap_chunks);
+/* decoded height grids [n_units][G][G] float of the last search (unit u = job * R + roll; batches under haf_set_debug(1)).  Only
+ * the units of active rolls are defined: inactive ones (outside [roll_begin, roll_limit)) are never decoded and hold bin keys.
+ * Returns the number of units written. */
+int haf_debug_heights(haf_ctx* ctx, float* heights, size_t cap_floats);
 /* cell index (idx_x*G+idx_y, or -1 outside the box) of every point for one request / roll */
 int haf_debug_cell_indices(haf_ctx* ctx, const float* xyz_hostdev, size_t n_points, size_t stride_bytes,
                            const haf_request* req, int roll, int* cell_idx_host);
