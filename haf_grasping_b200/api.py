@@ -78,7 +78,8 @@ EXPORTS = ["haf_create", "haf_destroy", "haf_last_error", "haf_get_info", "haf_s
            "haf_get_timing", "haf_launch_count", "haf_set_debug", "haf_search", "haf_search_batch", "haf_search_batch_packed",
            "haf_search_grasps", "haf_search_batch_packed_grasps", "haf_search_batch_requests", "haf_debug_unit_params", "haf_debug_chunk_copy_waits", "haf_debug_heights", "haf_build_transform", "haf_build_transform_wcs", "haf_best_key", "haf_pack_best_records", "haf_debug_window_count", "haf_debug_windows", "haf_debug_features",
            "haf_debug_decisions", "haf_debug_tensor_inputs", "haf_debug_integral", "haf_debug_cell_indices", "haf_debug_text_roundtrip", "haf_debug_tc_probe",
-           "haf_version", "haf_pcd_decode", "haf_search_pcd", "haf_pointcloud2_to_xyz", "haf_debug_pcd_xyz", "haf_svm_create", "haf_svm_create_config", "haf_svm_destroy", "haf_svm_predict", "haf_svm_predict_probability", "haf_svm_check_probability_model", "haf_scale_minmax", "haf_scale_apply"]
+           "haf_version", "haf_pcd_decode", "haf_search_pcd", "haf_pointcloud2_to_xyz", "haf_debug_pcd_xyz",
+           "haf_pcd_decode_batch", "haf_search_batch_pcd", "haf_pointcloud2_batch_to_xyz", "haf_svm_create", "haf_svm_create_config", "haf_svm_destroy", "haf_svm_predict", "haf_svm_predict_probability", "haf_svm_check_probability_model", "haf_scale_minmax", "haf_scale_apply"]
 
 _lib = None
 
@@ -142,6 +143,10 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.haf_search_pcd.argtypes = [vp, vp, cs, C.POINTER(haf_request), ci, C.POINTER(haf_best), C.POINTER(haf_best), vp, vp, vp, vp]
     L.haf_pointcloud2_to_xyz.argtypes = [vp, vp, cs, cs, ci, ci, ci, C.POINTER(vp)]
     L.haf_debug_pcd_xyz.argtypes = [vp, vp, cs]
+    L.haf_pcd_decode_batch.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(vp), C.POINTER(cs)]
+    L.haf_search_batch_pcd.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(haf_request), C.POINTER(ci), C.POINTER(haf_best),
+                                       C.POINTER(haf_best), vp, C.POINTER(haf_grasp), C.POINTER(haf_grasp), C.POINTER(haf_grasp)]
+    L.haf_pointcloud2_batch_to_xyz.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(ci), C.POINTER(vp), C.POINTER(cs)]
     L.haf_svm_create.argtypes = [C.POINTER(vp), C.c_char_p, ci, ci, ci, C.c_float]
     L.haf_svm_create_config.argtypes = [C.POINTER(vp), C.POINTER(haf_config), ci]
     L.haf_svm_destroy.argtypes = [vp]
@@ -477,6 +482,85 @@ class GraspSearch:
         top = np.zeros((len(reqs), self.R, 3), np.int32)
         self._check(self.L.haf_search_pcd(self.h, _ptr(buf), len(buf), arr, len(reqs), C.byref(best), per, None, None, None, _ptr(top)))
         return {"best": best, "best_per_request": list(per), "per_roll_top": top}
+
+    # ---- batches of PCD files / PointCloud2 buffers: one decode for all clouds ----
+    @staticmethod
+    def _pcd_batch(files):
+        """files: a list of bytes-like objects (concatenated here once), or (data, file_offsets) with data a contiguous uint8
+        numpy array or host torch tensor (pinned or not) that already holds the files back to back"""
+        if isinstance(files, tuple):
+            data, offs = files
+            offs = [int(o) for o in offs]
+            if isinstance(data, np.ndarray):
+                data = np.ascontiguousarray(data, np.uint8)
+        else:
+            lens = [len(memoryview(f).cast("B")) for f in files]
+            offs = [0] + list(np.cumsum(lens, dtype=np.int64).tolist())
+            data = np.frombuffer(b"".join(files), np.uint8) if files else np.zeros(0, np.uint8)
+        return data, (C.c_size_t * len(offs))(*offs), len(offs) - 1
+
+    def pcd_decode_batch(self, files):
+        """PCD files -> (device pointer of the packed xyz of every cloud, point_offsets int64 [n_files + 1]) (haf_pcd_decode_batch);
+        the buffer belongs to the context.  files: see _pcd_batch."""
+        data, off, n = self._pcd_batch(files)
+        d = C.c_void_p()
+        po = (C.c_size_t * (n + 1))()
+        self._check(self.L.haf_pcd_decode_batch(self.h, _ptr(data), off, n, C.byref(d), po))
+        return (d.value or 0), np.array(po[:], np.int64)
+
+    def pcd_decode_batch_to_host(self, files):
+        """decode a batch on the device, then copy it back: a list of float32 [n_i, 3] arrays"""
+        _, po = self.pcd_decode_batch(files)
+        xyz = self.debug_pcd_xyz(int(po[-1]))
+        return [xyz[po[f]:po[f + 1]] for f in range(len(po) - 1)]
+
+    def search_batch_pcd(self, files, requests=None, request_offsets=None, grasps=True, per_roll=False, per_roll_top=False):
+        """haf_search_batch_pcd: decode every file on the device, then ``search_batch_requests`` on the clouds.  requests=None:
+        ``make_request()`` for every file.  Returns the dict of ``search_batch_requests`` plus ``point_offsets``."""
+        data, off, n = self._pcd_batch(files)
+        if requests is None:
+            requests = make_requests(n)
+        elif not isinstance(requests, C.Array):
+            requests = (haf_request * len(requests))(*requests)
+        nreq = len(requests)
+        roff = None if request_offsets is None else (C.c_int * len(request_offsets))(*[int(o) for o in request_offsets])
+        best, bpr = (haf_best * n)(), (haf_best * nreq)()
+        grasp = (haf_grasp * n)() if grasps else None
+        gpr = (haf_grasp * nreq)() if grasps else None
+        groll = (haf_grasp * (nreq * self.R))() if grasps and per_roll else None
+        top = np.full((nreq, self.R, 3), -1, np.int32) if per_roll_top else None
+        self._check(self.L.haf_search_batch_pcd(self.h, _ptr(data), off, n, requests, roff, best, bpr, _ptr(top), grasp, gpr, groll))
+        out = {"best": best, "best_per_request": bpr}
+        if grasps:
+            out["grasp"], out["grasp_per_request"] = grasp, gpr
+        if groll is not None:
+            out["grasp_per_roll"] = groll
+        if top is not None:
+            out["per_roll_top"] = top
+        out["point_offsets"] = self._pcd_point_offsets(data, off, n)
+        return out
+
+    @staticmethod
+    def _pcd_point_offsets(data, off, n):
+        """cumulative POINTS of the headers (what the decode reports as point_offsets)"""
+        from . import pcd
+        raw = data.numpy() if hasattr(data, "numpy") else data
+        po = [0]
+        for f in range(n):
+            po.append(po[-1] + pcd.header_points(raw[off[f]:off[f + 1]]))
+        return np.array(po, np.int64)
+
+    def pointcloud2_batch_to_xyz(self, data, byte_offsets, layouts):
+        """haf_pointcloud2_batch_to_xyz: data (host array or CUDA tensor) holds the clouds' records back to back, cloud c =
+        bytes [byte_offsets[c], byte_offsets[c + 1]); layouts [n_clouds][4] = (point_step, off_x, off_y, off_z).  Returns
+        (device pointer of the packed xyz, point_offsets int64 [n_clouds + 1])."""
+        n = len(byte_offsets) - 1
+        off = (C.c_size_t * (n + 1))(*[int(o) for o in byte_offsets])
+        lay = np.ascontiguousarray(np.asarray(layouts, np.int32).reshape(n, 4))
+        d = C.c_void_p()
+        po = (C.c_size_t * (n + 1))()
+        self._check(self.L.haf_pointcloud2_batch_to_xyz(self.h, _ptr(data), off, n, lay.ctypes.data_as(C.POINTER(C.c_int)), C.byref(d), po))
+        return (d.value or 0), np.array(po[:], np.int64)
 
     def debug_windows(self):
         W = self._check(self.L.haf_debug_window_count(self.h))

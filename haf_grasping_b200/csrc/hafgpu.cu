@@ -259,7 +259,11 @@ struct haf_ctx {
     DevBuf<unsigned char> d_pcd_raw, d_pcd_blob;
     DevBuf<float> d_pcd_xyz;
     DevBuf<unsigned> d_pcd_tiles;
-    DevBuf<unsigned long long> d_pcd_words;   // [0] record count, [1] LZF stream descriptor (4 words), [8] status / flags (ints)
+    DevBuf<unsigned long long> d_pcd_status;  // per call: [0] ASCII record total, then record counts, flags and LZF status per file
+    DevBuf<unsigned char> d_pcd_params;       // per call: the file / segment tables (pcd_ingest.cuh), sent from h_pcd_params
+    PinBuf<unsigned char> h_pcd_params;
+    PinBuf<unsigned long long> h_pcd_status;
+    cudaEvent_t pcd_params_ev = nullptr;      // the last H2D copy of h_pcd_params (the next call refills it after that copy)
 
     // libsvm front end (haf_svm_*): inputs given by the caller
     bool svm_only = false;
@@ -1033,7 +1037,7 @@ extern "C" void haf_destroy(haf_ctx* ctx) {
     ctx->d_integral.release(); ctx->d_rowscan.release(); ctx->d_mask.release(); ctx->d_labelgrid.release(); ctx->d_evals.release();
     ctx->d_unit_block.release(); ctx->d_win.release(); ctx->d_X.release();
     ctx->d_xn.release(); ctx->d_dec.release(); ctx->d_guardflag.release(); ctx->d_guardlist.release(); ctx->d_kscratch.release();
-    ctx->d_xdense.release(); ctx->d_labels.release(); ctx->d_probs.release(); ctx->d_probgrid.release(); ctx->d_pcd_raw.release(); ctx->d_pcd_blob.release(); ctx->d_pcd_xyz.release(); ctx->d_pcd_tiles.release(); ctx->d_pcd_words.release(); ctx->d_csr_ptr.release(); ctx->d_csr_idx.release(); ctx->d_csr_val.release();
+    ctx->d_xdense.release(); ctx->d_labels.release(); ctx->d_probs.release(); ctx->d_probgrid.release(); ctx->d_pcd_raw.release(); ctx->d_pcd_blob.release(); ctx->d_pcd_xyz.release(); ctx->d_pcd_tiles.release(); ctx->d_pcd_status.release(); ctx->d_pcd_params.release(); ctx->h_pcd_params.release(); ctx->h_pcd_status.release(); ctx->d_csr_ptr.release(); ctx->d_csr_idx.release(); ctx->d_csr_val.release();
     ctx->d_svn64.release(); ctx->d_Xg.release(); ctx->d_xn64.release(); ctx->d_g2accum.release(); ctx->d_g2tickets.release(); ctx->d_guardlist2.release();
     ctx->d_SVh.release(); ctx->d_SVl.release(); ctx->d_Xh.release(); ctx->d_Xl.release(); ctx->d_svcoef.release(); ctx->d_dec_tc.release(); ctx->d_asum.release(); ctx->d_dimfeat.release(); ctx->d_round4.release();
     ctx->d_params.release(); ctx->d_counters.release(); ctx->h_stage.release(); ctx->h_results.release(); ctx->h_per_roll_top.release(); ctx->h_counters.release(); ctx->h_unit_windows.release();
@@ -1054,6 +1058,7 @@ extern "C" void haf_destroy(haf_ctx* ctx) {
     for (size_t i = 0; i < ctx->ev_pool.size(); i++) cudaEventDestroy(ctx->ev_pool[i]);
     for (size_t i = 0; i < ctx->copy_ev.size(); i++) cudaEventDestroy(ctx->copy_ev[i]);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
+    if (ctx->pcd_params_ev) cudaEventDestroy(ctx->pcd_params_ev);
     cudaGetLastError();
     delete ctx;
 }
@@ -1938,8 +1943,8 @@ static void fill_best(const haf_ctx* ctx, const Job& jb, const JobResult& r, int
 }
 
 // helper thread of a pageable host batch (haf_ctx::Stager): piece by piece, src -> pinned ring slot (stage_threads host threads),
-// then the slot -> device copy and the piece's event on copy_stream.  A slot is reused once the copy that read it has finished.
-static void stager_main(haf_ctx* ctx, const unsigned char* src, std::vector<std::pair<size_t, size_t> > pieces, size_t slot_bytes) {
+// then the slot -> dst (device) copy and the piece's event on copy_stream.  A slot is reused once the copy that read it has finished.
+static void stager_main(haf_ctx* ctx, unsigned char* dst, const unsigned char* src, std::vector<std::pair<size_t, size_t> > pieces, size_t slot_bytes) {
     bool ok = cudaSetDevice(ctx->device) == cudaSuccess;
     const int T = std::max(1, std::min(16, ctx->stage_threads));
     for (size_t k = 0; k < pieces.size(); k++) {
@@ -1960,7 +1965,7 @@ static void stager_main(haf_ctx* ctx, const unsigned char* src, std::vector<std:
             memcpy(slot, src + b0, std::min(per, n));
             if (covered < n) memcpy(slot + covered, src + b0 + covered, n - covered);
             for (size_t t = 0; t < helpers.size(); t++) helpers[t].join();
-            ok = cudaMemcpyAsync(ctx->d_xyz.p + b0, slot, n, cudaMemcpyHostToDevice, ctx->copy_stream) == cudaSuccess;
+            ok = cudaMemcpyAsync(dst + b0, slot, n, cudaMemcpyHostToDevice, ctx->copy_stream) == cudaSuccess;
         }
         if (cudaEventRecord(ctx->copy_ev[k], ctx->copy_stream) != cudaSuccess) ok = false;
         {
@@ -2125,6 +2130,22 @@ extern "C" int haf_search_batch_packed_grasps(haf_ctx* ctx, const float* xyz_all
     if (ctx->group.size() > 1) return group_batch_packed(ctx, xyz_all, point_offsets, n_clouds, req, best_per_cloud, &go);
     return batch_packed_single(ctx, xyz_all, point_offsets, n_clouds, req, best_per_cloud, &go);
 }
+// starts the staging thread (stager_main) for pieces [b0, b1) of src, copied to dst + b0 on copy_stream; copy_ev holds an event
+// per piece, copy_stream already follows the work queued before on the stream
+static int start_stager(haf_ctx* ctx, unsigned char* dst, const unsigned char* src, const std::vector<std::pair<size_t, size_t> >& piece_bytes) {
+    size_t slot = 0;
+    for (size_t i = 0; i < piece_bytes.size(); i++) slot = std::max(slot, piece_bytes[i].second - piece_bytes[i].first);
+    slot = round_up(slot, 4096);
+    ENSURE(ctx, ctx->h_ring, slot * haf_ctx::kRingSlots);
+    ctx->stager.issued = 0; ctx->stager.failed = false;
+    try {
+        ctx->stager.th = std::thread(stager_main, ctx, dst, src, piece_bytes, slot);
+        ctx->stager.active = true;
+    } catch (...) {
+        return ctx->fail(HAF_ERR_NOMEM, "could not start the staging thread for a pageable host batch (set HAF_STAGE_THREADS=0 to use the driver's copy path)");
+    }
+    return HAF_OK;
+}
 // The clouds of a packed batch on the device (cs): device memory is used in place, host memory is staged piece by piece.
 // A pageable batch starts the staging thread; the caller joins it (StagerJoin) once run_jobs has returned.
 static int prepare_batch(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, CloudSet& cs) {
@@ -2175,18 +2196,8 @@ static int prepare_batch(haf_ctx* ctx, const float* xyz_all, const size_t* point
         }
         ctx->copy_pieces = k;
         if (own_staging) {
-            size_t slot = 0;
-            for (size_t i = 0; i < piece_bytes.size(); i++) slot = std::max(slot, piece_bytes[i].second - piece_bytes[i].first);
-            slot = round_up(slot, 4096);
-            ENSURE(ctx, ctx->h_ring, slot * haf_ctx::kRingSlots);
-            ctx->stager.issued = 0; ctx->stager.failed = false;
-            try {
-                ctx->stager.th = std::thread(stager_main, ctx, reinterpret_cast<const unsigned char*>(xyz_all), piece_bytes, slot);
-                ctx->stager.active = true;
-            } catch (...) {
-                ctx->copy_pieces = 0;
-                return ctx->fail(HAF_ERR_NOMEM, "could not start the staging thread for a pageable host batch (set HAF_STAGE_THREADS=0 to use the driver's copy path)");
-            }
+            const int rc = start_stager(ctx, ctx->d_xyz.p, reinterpret_cast<const unsigned char*>(xyz_all), piece_bytes);
+            if (rc) { ctx->copy_pieces = 0; return rc; }
         }
     }
     cs.d_xyz = total == 0 ? nullptr : (dev ? reinterpret_cast<const unsigned char*>(xyz_all) : ctx->d_xyz.p);
@@ -2342,118 +2353,339 @@ static int batch_single(haf_ctx* ctx, const float* const* clouds, const size_t* 
 // ------------------------------------------------------------------------------------------------------------
 // PCD / PointCloud2 ingest on the device (SURVEY 8f-2; kernels and the PCL semantics they restate: pcd_ingest.cuh)
 // ------------------------------------------------------------------------------------------------------------
+// Host bytes -> dst (device).  Pinned memory, and pageable buffers under 4 MB, take one cudaMemcpyAsync on the stream; larger
+// pageable buffers go through the staging thread (stager_main) in pieces that end on `cuts` (ascending offsets into src, the
+// last one = bytes), and the call returns once the last piece has arrived (the pinned ring is free for the next call).
+static int upload_host_bytes(haf_ctx* ctx, unsigned char* dst, const unsigned char* src, size_t bytes, const std::vector<size_t>& cuts) {
+    if (bytes == 0) return HAF_OK;
+    if (ctx->stage_threads <= 0 || bytes < ((size_t)4 << 20) || is_pinned_host_ptr(src)) {
+        CUDA_TRY(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
+        return HAF_OK;
+    }
+    std::vector<std::pair<size_t, size_t> > pieces;   // pieces of at least 16 MB (the last one aside)
+    size_t b0 = 0;
+    for (size_t i = 0; i < cuts.size(); i++)
+        if (cuts[i] > b0 && (cuts[i] - b0 >= ((size_t)16 << 20) || cuts[i] == bytes)) { pieces.push_back(std::make_pair(b0, cuts[i])); b0 = cuts[i]; }
+    if (!ctx->copy_stream) CUDA_TRY(ctx, cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+    cudaEvent_t start_ev;
+    CUDA_TRY(ctx, cudaEventCreateWithFlags(&start_ev, cudaEventDisableTiming));
+    CUDA_TRY(ctx, cudaEventRecord(start_ev, ctx->stream));            // dst may still be read by work queued before
+    CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->copy_stream, start_ev, 0));
+    cudaEventDestroy(start_ev);
+    while (ctx->copy_ev.size() < pieces.size()) {
+        cudaEvent_t e;
+        CUDA_TRY(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        ctx->copy_ev.push_back(e);
+    }
+    { const int rc = start_stager(ctx, dst, src, pieces); if (rc) return rc; }
+    ctx->stager.th.join();
+    ctx->stager.active = false;
+    if (ctx->stager.failed) return ctx->fail(HAF_ERR_CUDA, "staging a pageable host buffer failed");
+    CUDA_TRY(ctx, cudaEventSynchronize(ctx->copy_ev[pieces.size() - 1]));
+    return HAF_OK;
+}
+
+// The tables of one ingest call in one pinned block, sent with one H2D copy: add() places an array (16-byte aligned), open()
+// sizes both copies once the previous call's copy has read the pinned one, send() queues the copy.
+struct IngestParams {
+    haf_ctx* c;
+    size_t bytes = 0;
+    explicit IngestParams(haf_ctx* ctx) : c(ctx) {}
+    size_t add(size_t n) { const size_t o = bytes; bytes = round_up(bytes + n, 16); return o; }
+    int open() {
+        if (c->pcd_params_ev) CUDA_TRY(c, cudaEventSynchronize(c->pcd_params_ev));
+        else CUDA_TRY(c, cudaEventCreateWithFlags(&c->pcd_params_ev, cudaEventDisableTiming));
+        ENSURE(c, c->h_pcd_params, bytes + 16);
+        ENSURE(c, c->d_pcd_params, bytes + 16);
+        return HAF_OK;
+    }
+    template <typename T> T* h(size_t o) { return reinterpret_cast<T*>(c->h_pcd_params.p + o); }
+    template <typename T> T* d(size_t o) { return reinterpret_cast<T*>(c->d_pcd_params.p + o); }
+    int send() {
+        CUDA_TRY(c, cudaMemcpyAsync(c->d_pcd_params.p, c->h_pcd_params.p, bytes, cudaMemcpyHostToDevice, c->stream));
+        CUDA_TRY(c, cudaEventRecord(c->pcd_params_ev, c->stream));
+        return HAF_OK;
+    }
+};
+
+// one gather over the segments of a call (hafpcdk::gather_segments_kernel), tables already in the parameter block
+static int launch_gather(haf_ctx* ctx, IngestParams& P, size_t o_segs, size_t o_begin, int n_segs, unsigned long long n_points) {
+    if (n_segs == 0) return HAF_OK;
+    hafpcdk::gather_segments_kernel<<<(unsigned)std::min<unsigned long long>((n_points + 255) / 256, 148 * 16), 256, 0, ctx->stream>>>(
+        P.d<hafpcdk::GatherSeg>(o_segs), P.d<unsigned long long>(o_begin), n_segs, ctx->d_pcd_xyz.p);
+    LAUNCHED(ctx);
+    return HAF_OK;
+}
+
+// PCD files [file_offsets[f], file_offsets[f + 1]) of `files` (host memory) -> packed xyz of every cloud in ctx->d_pcd_xyz.
+// Every header is parsed and checked on the host first (the lowest failing file is named before any device work); then each
+// data kind present runs its fixed launch sequence over all its files, and one stream sync ends the call.  batch: messages
+// name the file ("PCD file <i>: ..."); haf_pcd_decode (the batch of one) keeps the bare single-file texts.
+static int pcd_decode_files(haf_ctx* ctx, const unsigned char* files, const size_t* file_offsets, int n_files, bool batch,
+                            const float** d_xyz, size_t* point_offsets) {
+    char buf[512];
+    auto fail_file = [&](int f, int code, const char* fmt, ...) {
+        va_list ap;
+        va_start(ap, fmt);
+        vsnprintf(buf, sizeof buf, fmt, ap);
+        va_end(ap);
+        return batch ? ctx->fail(code, "PCD file %d: %s", f, buf) : ctx->fail(code, "%s", buf);
+    };
+    for (int f = 0; f < n_files; f++)
+        if (file_offsets[f + 1] < file_offsets[f]) return ctx->fail(HAF_ERR_ARG, "haf_pcd_decode_batch: file_offsets must be non-decreasing");
+    const size_t base = file_offsets[0], bytes = file_offsets[n_files] - base;
+    if (bytes > 0 && !files) return ctx->fail(HAF_ERR_ARG, "haf_pcd_decode_batch: files is null");
+    // ---- host: headers, checks and the tables (source addresses as offsets: raw copy or blob, fixed up below)
+    std::vector<size_t> pts(n_files + 1, 0);
+    std::vector<hafpcdk::AsciiFile> asc;
+    std::vector<int> asc_file, tile_file, lzf_file;
+    std::vector<hafpcdk::GatherSeg> segs;
+    std::vector<unsigned long long> seg_begin(1, 0);
+    std::vector<char> seg_in_blob;
+    std::vector<hafpcdk::LzfStream> lzf;
+    std::vector<size_t> cuts;
+    size_t blob_bytes = 0;
+    unsigned long long ascii_records_max = 0;
+    const size_t tile_bytes = (size_t)HAF_PCD_TILE_THREADS * HAF_PCD_BYTES_PER_THREAD;
+    for (int f = 0; f < n_files; f++) {
+        const size_t fb = file_offsets[f] - base, nb = file_offsets[f + 1] - file_offsets[f];
+        cuts.push_back(fb + nb);
+        const unsigned char* raw = files + file_offsets[f];
+        hafpcd::PcdHeader hd;
+        std::string herr;
+        if (!hafpcd::parse_pcd_header(raw, nb, hd, &herr)) return fail_file(f, HAF_ERR_IO, "%s", herr.c_str());
+        for (int a = 0; a < 3; a++)
+            if (hd.types[hd.idx[a]] != "F" || hd.sizes[hd.idx[a]] != 4) return fail_file(f, HAF_ERR_UNSUPPORTED, "PCD: x / y / z must be float32 fields");
+        const size_t npts = (size_t)hd.npts;
+        pts[f + 1] = pts[f] + npts;
+        if (npts == 0) continue;
+        const size_t data = fb + hd.data_begin, dn = nb - hd.data_begin;
+        hafpcdk::GatherSeg sg;
+        memset(&sg, 0, sizeof sg);
+        sg.out_begin = pts[f];
+        if (hd.data_kind == "ascii") {
+            if (dn == 0) return fail_file(f, HAF_ERR_IO, "fewer records than POINTS in the PCD data");
+            std::vector<int> tokoff(hd.fields.size() + 1, 0);
+            for (size_t k = 0; k < hd.fields.size(); k++) tokoff[k + 1] = tokoff[k] + hd.counts[k];
+            hafpcdk::AsciiFile af;
+            memset(&af, 0, sizeof af);
+            af.begin = data; af.len = dn; af.n_points = npts; af.out_begin = pts[f];
+            const size_t n_tiles = (dn + tile_bytes - 1) / tile_bytes;
+            if (tile_file.size() + n_tiles > 0x7fffffffu) return fail_file(f, HAF_ERR_UNSUPPORTED, "ASCII PCD too large");
+            af.tile_begin = (int)tile_file.size(); af.tile_end = (int)(tile_file.size() + n_tiles);
+            for (int a = 0; a < 3; a++) af.tok[a] = tokoff[hd.idx[a]];
+            ascii_records_max += (dn + 1) / 2;     // a record is a token and a line end at least
+            if (ascii_records_max > 0xFFFFFFFFull) return fail_file(f, HAF_ERR_UNSUPPORTED, "ASCII PCD too large");
+            tile_file.insert(tile_file.end(), n_tiles, (int)asc.size());
+            asc.push_back(af);
+            asc_file.push_back(f);
+        } else if (hd.data_kind == "binary") {
+            size_t rec_bytes = 0;
+            std::vector<size_t> foff(hd.fields.size());
+            for (size_t k = 0; k < hd.fields.size(); k++) { foff[k] = rec_bytes; rec_bytes += (size_t)hd.sizes[k] * hd.counts[k]; }
+            if (rec_bytes * npts > dn) return fail_file(f, HAF_ERR_IO, "binary PCD truncated");
+            sg.src = reinterpret_cast<const unsigned char*>(data);
+            for (int a = 0; a < 3; a++) { sg.off[a] = foff[hd.idx[a]]; sg.stride[a] = rec_bytes; }
+            segs.push_back(sg); seg_in_blob.push_back(0); seg_begin.push_back(seg_begin.back() + npts);
+        } else if (hd.data_kind == "binary_compressed") {
+            if (dn < 8) return fail_file(f, HAF_ERR_IO, "compressed PCD truncated");
+            uint32_t comp, uncomp;
+            memcpy(&comp, raw + hd.data_begin, 4);
+            memcpy(&uncomp, raw + hd.data_begin + 4, 4);
+            if ((size_t)comp + 8 > dn) return fail_file(f, HAF_ERR_IO, "compressed PCD truncated");
+            std::vector<size_t> foff(hd.fields.size());
+            size_t off = 0;
+            for (size_t k = 0; k < hd.fields.size(); k++) { foff[k] = off; off += npts * (size_t)hd.sizes[k] * hd.counts[k]; }
+            for (int a = 0; a < 3; a++)
+                if (foff[hd.idx[a]] + (npts - 1) * 4 * (size_t)hd.counts[hd.idx[a]] + 4 > uncomp)
+                    return fail_file(f, HAF_ERR_IO, "compressed PCD: the stream is shorter than the header's fields");
+            hafpcdk::LzfStream ls;
+            ls.in = reinterpret_cast<const unsigned char*>(data + 8); ls.in_len = comp;
+            ls.out = reinterpret_cast<unsigned char*>(blob_bytes); ls.out_len = uncomp;
+            lzf.push_back(ls);
+            lzf_file.push_back(f);
+            sg.src = reinterpret_cast<const unsigned char*>(blob_bytes);
+            for (int a = 0; a < 3; a++) { sg.off[a] = foff[hd.idx[a]]; sg.stride[a] = 4 * (size_t)hd.counts[hd.idx[a]]; }
+            segs.push_back(sg); seg_in_blob.push_back(1); seg_begin.push_back(seg_begin.back() + npts);
+            blob_bytes = round_up(blob_bytes + uncomp, 16);
+        } else {
+            return fail_file(f, HAF_ERR_UNSUPPORTED, "unsupported PCD DATA kind '%s'", hd.data_kind.c_str());
+        }
+    }
+    const size_t total = pts[n_files];
+    if (total > 0) {
+        CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+        cudaStream_t st = ctx->stream;
+        const int n_asc = (int)asc.size(), n_lzf = (int)lzf.size();
+        const unsigned n_tiles = (unsigned)tile_file.size();
+        ENSURE(ctx, ctx->d_pcd_xyz, total * 3);
+        ENSURE(ctx, ctx->d_pcd_raw, bytes + 16);
+        ENSURE(ctx, ctx->d_pcd_blob, blob_bytes + 16);
+        ENSURE(ctx, ctx->d_pcd_tiles, (size_t)n_tiles + 1);
+        // status: [0] ASCII record total, then u32 count [n_asc], int flags [2 n_asc], int LZF status [n_lzf]
+        const size_t status_words = 1 + ((size_t)n_asc * 12 + (size_t)n_lzf * 4 + 7) / 8;
+        ENSURE(ctx, ctx->d_pcd_status, status_words);
+        ENSURE(ctx, ctx->h_pcd_status, status_words);
+        unsigned* d_count = reinterpret_cast<unsigned*>(ctx->d_pcd_status.p + 1);
+        int* d_flags = reinterpret_cast<int*>(d_count + n_asc);
+        int* d_lzf_status = d_flags + 2 * n_asc;
+        for (size_t s = 0; s < segs.size(); s++)
+            segs[s].src = (seg_in_blob[s] ? ctx->d_pcd_blob.p : ctx->d_pcd_raw.p) + reinterpret_cast<size_t>(segs[s].src);
+        for (int l = 0; l < n_lzf; l++) {
+            lzf[l].in = ctx->d_pcd_raw.p + reinterpret_cast<size_t>(lzf[l].in);
+            lzf[l].out = ctx->d_pcd_blob.p + reinterpret_cast<size_t>(lzf[l].out);
+        }
+        IngestParams P(ctx);
+        const size_t o_asc = P.add(asc.size() * sizeof(hafpcdk::AsciiFile)), o_tiles = P.add(tile_file.size() * sizeof(int));
+        const size_t o_segs = P.add(segs.size() * sizeof(hafpcdk::GatherSeg)), o_begin = P.add(seg_begin.size() * 8);
+        const size_t o_lzf = P.add(lzf.size() * sizeof(hafpcdk::LzfStream));
+        { const int rc = P.open(); if (rc) return rc; }
+        if (n_asc) memcpy(P.h<hafpcdk::AsciiFile>(o_asc), asc.data(), asc.size() * sizeof(hafpcdk::AsciiFile));
+        if (n_tiles) memcpy(P.h<int>(o_tiles), tile_file.data(), tile_file.size() * sizeof(int));
+        if (!segs.empty()) memcpy(P.h<hafpcdk::GatherSeg>(o_segs), segs.data(), segs.size() * sizeof(hafpcdk::GatherSeg));
+        memcpy(P.h<unsigned long long>(o_begin), seg_begin.data(), seg_begin.size() * 8);
+        if (n_lzf) memcpy(P.h<hafpcdk::LzfStream>(o_lzf), lzf.data(), lzf.size() * sizeof(hafpcdk::LzfStream));
+        { const int rc = upload_host_bytes(ctx, ctx->d_pcd_raw.p, files + base, bytes, cuts); if (rc) return rc; }
+        { const int rc = P.send(); if (rc) return rc; }
+        CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_pcd_status.p, 0, status_words * 8, st));
+        if (n_asc) {
+            hafpcdk::ascii_count_kernel<<<n_tiles, HAF_PCD_TILE_THREADS, 0, st>>>(ctx->d_pcd_raw.p, P.d<hafpcdk::AsciiFile>(o_asc), P.d<int>(o_tiles),
+                                                                                  ctx->d_pcd_tiles.p);
+            LAUNCHED(ctx);
+            hafpcdk::ascii_scan_kernel<<<1, 1024, 0, st>>>(ctx->d_pcd_tiles.p, n_tiles, ctx->d_pcd_status.p);
+            LAUNCHED(ctx);
+            hafpcdk::ascii_parse_kernel<<<n_tiles, HAF_PCD_TILE_THREADS, 0, st>>>(ctx->d_pcd_raw.p, P.d<hafpcdk::AsciiFile>(o_asc), P.d<int>(o_tiles),
+                                                                                  ctx->d_pcd_tiles.p, n_tiles, ctx->d_pcd_status.p, ctx->d_pcd_xyz.p,
+                                                                                  d_count, d_flags);
+            LAUNCHED(ctx);
+        }
+        if (n_lzf) {
+            hafpcdk::lzf_decompress_kernel<<<n_lzf, 32, 0, st>>>(P.d<hafpcdk::LzfStream>(o_lzf), d_lzf_status);
+            LAUNCHED(ctx);
+        }
+        { const int rc = launch_gather(ctx, P, o_segs, o_begin, (int)segs.size(), seg_begin.back()); if (rc) return rc; }
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_pcd_status.p, ctx->d_pcd_status.p, status_words * 8, cudaMemcpyDeviceToHost, st));
+        CUDA_TRY(ctx, cudaStreamSynchronize(st));
+        // the lowest failing file, with the single-file checks in their order
+        const unsigned* h_count = reinterpret_cast<const unsigned*>(ctx->h_pcd_status.p + 1);
+        const int* h_flags = reinterpret_cast<const int*>(h_count + n_asc);
+        const int* h_lzf_status = h_flags + 2 * n_asc;
+        int la = 0, ll = 0;
+        while (la < n_asc || ll < n_lzf) {
+            const bool take_asc = ll >= n_lzf || (la < n_asc && asc_file[la] < lzf_file[ll]);
+            if (take_asc) {
+                const int f = asc_file[la], a = la++;
+                if (h_count[a] < asc[a].n_points)
+                    return fail_file(f, HAF_ERR_IO, "fewer records than POINTS in the PCD data (%llu of %zu)", (unsigned long long)h_count[a], (size_t)asc[a].n_points);
+                if (h_flags[2 * a]) return fail_file(f, HAF_ERR_IO, "short ASCII record in the PCD data");
+                if (h_flags[2 * a + 1])
+                    return fail_file(f, HAF_ERR_UNSUPPORTED, "an ASCII token has more than 19 significant digits and lies next to a float rounding boundary");
+            } else {
+                const int f = lzf_file[ll], l = ll++;
+                if (h_lzf_status[l]) return fail_file(f, HAF_ERR_IO, "corrupt LZF stream in the PCD data");
+            }
+        }
+    }
+    for (int f = 0; f <= n_files; f++) point_offsets[f] = pts[f];
+    *d_xyz = total ? ctx->d_pcd_xyz.p : nullptr;
+    return HAF_OK;
+}
+
+// PointCloud2 data: cloud c = bytes [byte_offsets[c], byte_offsets[c + 1]) of data (host or device), records of layouts[4c]
+// bytes with x / y / z float32 at layouts[4c + 1 .. 4c + 3] -> packed xyz in ctx->d_pcd_xyz (one gather, no sync).  Clouds of
+// no bytes are empty and not checked.  batch: messages name the cloud (haf_pointcloud2_to_xyz is the batch of one).
+static int pointcloud2_clouds(haf_ctx* ctx, const void* data, const size_t* byte_offsets, int n_clouds, const int* layouts, bool batch,
+                              const float** d_xyz, size_t* point_offsets) {
+    const char* who = batch ? "haf_pointcloud2_batch_to_xyz" : "haf_pointcloud2_to_xyz";
+    std::vector<size_t> pts(n_clouds + 1, 0);
+    for (int c = 0; c < n_clouds; c++) {
+        if (byte_offsets[c + 1] < byte_offsets[c]) return ctx->fail(HAF_ERR_ARG, "%s: byte_offsets must be non-decreasing", who);
+        const size_t span = byte_offsets[c + 1] - byte_offsets[c];
+        pts[c + 1] = pts[c];
+        if (span == 0) continue;
+        const int* L = layouts + 4 * c;
+        if (L[0] < 4 || L[1] < 0 || L[2] < 0 || L[3] < 0 || std::max(L[1], std::max(L[2], L[3])) + 4 > L[0]) {
+            if (batch) return ctx->fail(HAF_ERR_ARG, "%s: cloud %d: x / y / z offsets must lie inside point_step", who, c);
+            return ctx->fail(HAF_ERR_ARG, "%s: x / y / z offsets must lie inside point_step", who);
+        }
+        if (span % (size_t)L[0]) return ctx->fail(HAF_ERR_ARG, "%s: cloud %d: %zu bytes are not a whole number of %d-byte records", who, c, span, L[0]);
+        pts[c + 1] += span / (size_t)L[0];
+    }
+    const size_t base = byte_offsets[0], bytes = byte_offsets[n_clouds] - base, total = pts[n_clouds];
+    if (bytes > 0 && !data) return ctx->fail(HAF_ERR_ARG, "%s: data is null", who);
+    if (total > 0) {
+        CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+        const unsigned char* src = reinterpret_cast<const unsigned char*>(data) + base;
+        if (!is_device_ptr(data)) {
+            ENSURE(ctx, ctx->d_pcd_raw, bytes + 16);
+            std::vector<size_t> cuts;
+            for (int c = 1; c <= n_clouds; c++) cuts.push_back(byte_offsets[c] - base);
+            const int rc = upload_host_bytes(ctx, ctx->d_pcd_raw.p, src, bytes, cuts);
+            if (rc) return rc;
+            src = ctx->d_pcd_raw.p;
+        }
+        ENSURE(ctx, ctx->d_pcd_xyz, total * 3);
+        std::vector<hafpcdk::GatherSeg> segs;
+        std::vector<unsigned long long> seg_begin(1, 0);
+        for (int c = 0; c < n_clouds; c++) {
+            if (pts[c + 1] == pts[c]) continue;
+            hafpcdk::GatherSeg sg;
+            sg.src = src + (byte_offsets[c] - base);
+            sg.out_begin = pts[c];
+            for (int a = 0; a < 3; a++) { sg.off[a] = (unsigned long long)layouts[4 * c + 1 + a]; sg.stride[a] = (unsigned long long)layouts[4 * c]; }
+            segs.push_back(sg);
+            seg_begin.push_back(pts[c + 1]);
+        }
+        IngestParams P(ctx);
+        const size_t o_segs = P.add(segs.size() * sizeof(hafpcdk::GatherSeg)), o_begin = P.add(seg_begin.size() * 8);
+        { const int rc = P.open(); if (rc) return rc; }
+        memcpy(P.h<hafpcdk::GatherSeg>(o_segs), segs.data(), segs.size() * sizeof(hafpcdk::GatherSeg));
+        memcpy(P.h<unsigned long long>(o_begin), seg_begin.data(), seg_begin.size() * 8);
+        { const int rc = P.send(); if (rc) return rc; }
+        { const int rc = launch_gather(ctx, P, o_segs, o_begin, (int)segs.size(), seg_begin.back()); if (rc) return rc; }
+    }
+    if (point_offsets) for (int c = 0; c <= n_clouds; c++) point_offsets[c] = pts[c];
+    *d_xyz = total ? ctx->d_pcd_xyz.p : nullptr;
+    return HAF_OK;
+}
+
 extern "C" int haf_pointcloud2_to_xyz(haf_ctx* ctx, const void* data, size_t n_points, size_t point_step, int off_x, int off_y, int off_z,
                                       const float** d_xyz) {
     if (!ctx || !d_xyz) return HAF_ERR_ARG;
     *d_xyz = nullptr;
     if (n_points == 0) return HAF_OK;
-    if (!data || point_step < 4 || off_x < 0 || off_y < 0 || off_z < 0 || (size_t)std::max(off_x, std::max(off_y, off_z)) + 4 > point_step)
+    if (!data || point_step < 4 || point_step > 0x7fffffff)
         return ctx->fail(HAF_ERR_ARG, "haf_pointcloud2_to_xyz: x / y / z offsets must lie inside point_step");
-    haf_ctx* c0 = ctx;
-    CUDA_TRY(c0, cudaSetDevice(c0->device));
-    const unsigned char* src = reinterpret_cast<const unsigned char*>(data);
-    if (!is_device_ptr(data)) {
-        ENSURE(c0, c0->d_pcd_raw, n_points * point_step + 16);
-        CUDA_TRY(c0, cudaMemcpyAsync(c0->d_pcd_raw.p, data, n_points * point_step, cudaMemcpyHostToDevice, c0->stream));
-        src = c0->d_pcd_raw.p;
-    }
-    ENSURE(c0, c0->d_pcd_xyz, n_points * 3);
-    hafpcdk::gather_records_kernel<<<(unsigned)std::min<size_t>((n_points + 255) / 256, 148 * 16), 256, 0, c0->stream>>>(src, n_points, point_step, off_x, off_y, off_z,
-                                                                                                                 c0->d_pcd_xyz.p);
-    LAUNCHED(c0);
-    *d_xyz = c0->d_pcd_xyz.p;
-    return HAF_OK;
+    const size_t byte_offsets[2] = {0, n_points * point_step};
+    const int layout[4] = {(int)point_step, off_x, off_y, off_z};
+    return pointcloud2_clouds(ctx, data, byte_offsets, 1, layout, false, d_xyz, nullptr);
+}
+
+extern "C" int haf_pointcloud2_batch_to_xyz(haf_ctx* ctx, const void* data, const size_t* byte_offsets, int n_clouds, const int* layouts,
+                                            const float** d_xyz, size_t* point_offsets) {
+    if (!ctx || !d_xyz) return HAF_ERR_ARG;
+    *d_xyz = nullptr;
+    if (!byte_offsets || n_clouds < 1 || !layouts || !point_offsets) return ctx->fail(HAF_ERR_ARG, "haf_pointcloud2_batch_to_xyz: bad arguments");
+    return pointcloud2_clouds(ctx, data, byte_offsets, n_clouds, layouts, true, d_xyz, point_offsets);
 }
 
 extern "C" int haf_pcd_decode(haf_ctx* ctx, const void* file_bytes, size_t n_bytes, const float** d_xyz, size_t* n_points) {
     if (!ctx || !d_xyz || !n_points) return HAF_ERR_ARG;
     *d_xyz = nullptr; *n_points = 0;
     if (!file_bytes || n_bytes == 0) return ctx->fail(HAF_ERR_ARG, "haf_pcd_decode: empty buffer");
-    const unsigned char* raw = reinterpret_cast<const unsigned char*>(file_bytes);
-    hafpcd::PcdHeader hd;
-    std::string herr;
-    if (!hafpcd::parse_pcd_header(raw, n_bytes, hd, &herr)) return ctx->fail(HAF_ERR_IO, "%s", herr.c_str());
-    for (int a = 0; a < 3; a++)
-        if (hd.types[hd.idx[a]] != "F" || hd.sizes[hd.idx[a]] != 4) return ctx->fail(HAF_ERR_UNSUPPORTED, "PCD: x / y / z must be float32 fields");
-    const size_t npts = (size_t)hd.npts;
-    if (npts == 0) return HAF_OK;
-    CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
-    const unsigned char* data = raw + hd.data_begin;
-    const size_t dn = n_bytes - hd.data_begin;
-    ENSURE(ctx, ctx->d_pcd_xyz, npts * 3);
-    ENSURE(ctx, ctx->d_pcd_words, 16);
-    ENSURE(ctx, ctx->h_stage, 256);
-    const unsigned grid_pts = (unsigned)std::min<size_t>((npts + 255) / 256, 148 * 16);
-    CUDA_TRY(ctx, cudaMemsetAsync(ctx->d_pcd_words.p, 0, 16 * 8, st));
-    int* d_flags = reinterpret_cast<int*>(ctx->d_pcd_words.p + 8);
-    unsigned long long* h_words = reinterpret_cast<unsigned long long*>(ctx->h_stage.p);
-    if (hd.data_kind == "ascii") {
-        if (dn == 0) return ctx->fail(HAF_ERR_IO, "fewer records than POINTS in the PCD data");
-        std::vector<int> tokoff(hd.fields.size() + 1, 0);
-        for (size_t k = 0; k < hd.fields.size(); k++) tokoff[k + 1] = tokoff[k] + hd.counts[k];
-        ENSURE(ctx, ctx->d_pcd_raw, dn + 16);
-        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_pcd_raw.p, data, dn, cudaMemcpyHostToDevice, st));
-        const size_t tile_bytes = (size_t)HAF_PCD_TILE_THREADS * HAF_PCD_BYTES_PER_THREAD;
-        const size_t n_tiles = (dn + tile_bytes - 1) / tile_bytes;
-        if (n_tiles > 0x7fffffffu) return ctx->fail(HAF_ERR_UNSUPPORTED, "ASCII PCD too large");
-        ENSURE(ctx, ctx->d_pcd_tiles, n_tiles);
-        hafpcdk::ascii_count_kernel<<<(unsigned)n_tiles, HAF_PCD_TILE_THREADS, 0, st>>>(ctx->d_pcd_raw.p, dn, ctx->d_pcd_tiles.p);
-        LAUNCHED(ctx);
-        hafpcdk::ascii_scan_kernel<<<1, 1024, 0, st>>>(ctx->d_pcd_tiles.p, (unsigned)n_tiles, ctx->d_pcd_words.p);
-        LAUNCHED(ctx);
-        hafpcdk::ascii_parse_kernel<<<(unsigned)n_tiles, HAF_PCD_TILE_THREADS, 0, st>>>(ctx->d_pcd_raw.p, dn, ctx->d_pcd_tiles.p, (unsigned long long)npts,
-                                                                                       tokoff[hd.idx[0]], tokoff[hd.idx[1]], tokoff[hd.idx[2]], ctx->d_pcd_xyz.p, d_flags);
-        LAUNCHED(ctx);
-        CUDA_TRY(ctx, cudaMemcpyAsync(h_words, ctx->d_pcd_words.p, 16 * 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(ctx, cudaStreamSynchronize(st));
-        const int* hf = reinterpret_cast<const int*>(h_words + 8);
-        if (h_words[0] < npts) return ctx->fail(HAF_ERR_IO, "fewer records than POINTS in the PCD data (%llu of %zu)", h_words[0], npts);
-        if (hf[0]) return ctx->fail(HAF_ERR_IO, "short ASCII record in the PCD data");
-        if (hf[1]) return ctx->fail(HAF_ERR_UNSUPPORTED, "an ASCII token has more than 19 significant digits and lies next to a float rounding boundary");
-    } else if (hd.data_kind == "binary") {
-        size_t rec_bytes = 0;
-        std::vector<size_t> foff(hd.fields.size());
-        for (size_t k = 0; k < hd.fields.size(); k++) { foff[k] = rec_bytes; rec_bytes += (size_t)hd.sizes[k] * hd.counts[k]; }
-        if (rec_bytes * npts > dn) return ctx->fail(HAF_ERR_IO, "binary PCD truncated");
-        ENSURE(ctx, ctx->d_pcd_raw, rec_bytes * npts + 16);
-        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_pcd_raw.p, data, rec_bytes * npts, cudaMemcpyHostToDevice, st));
-        hafpcdk::gather_records_kernel<<<grid_pts, 256, 0, st>>>(ctx->d_pcd_raw.p, npts, rec_bytes, (int)foff[hd.idx[0]], (int)foff[hd.idx[1]], (int)foff[hd.idx[2]],
-                                                                 ctx->d_pcd_xyz.p);
-        LAUNCHED(ctx);
-    } else if (hd.data_kind == "binary_compressed") {
-        if (dn < 8) return ctx->fail(HAF_ERR_IO, "compressed PCD truncated");
-        uint32_t comp, uncomp;
-        memcpy(&comp, data, 4);
-        memcpy(&uncomp, data + 4, 4);
-        if ((size_t)comp + 8 > dn) return ctx->fail(HAF_ERR_IO, "compressed PCD truncated");
-        std::vector<size_t> foff(hd.fields.size());
-        size_t off = 0;
-        for (size_t k = 0; k < hd.fields.size(); k++) { foff[k] = off; off += npts * (size_t)hd.sizes[k] * hd.counts[k]; }
-        for (int a = 0; a < 3; a++)
-            if (foff[hd.idx[a]] + (npts - 1) * 4 * (size_t)hd.counts[hd.idx[a]] + 4 > uncomp) return ctx->fail(HAF_ERR_IO, "compressed PCD: the stream is shorter than the header's fields");
-        ENSURE(ctx, ctx->d_pcd_raw, (size_t)comp + 16);
-        ENSURE(ctx, ctx->d_pcd_blob, (size_t)uncomp + 16);
-        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_pcd_raw.p, data + 8, comp, cudaMemcpyHostToDevice, st));
-        hafpcdk::LzfStream ls;
-        ls.in = ctx->d_pcd_raw.p; ls.in_len = comp; ls.out = ctx->d_pcd_blob.p; ls.out_len = uncomp;
-        CUDA_TRY(ctx, cudaStreamSynchronize(st));   // h_stage may still feed an earlier call's copy
-        memcpy(ctx->h_stage.p + 128, &ls, sizeof ls);
-        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_pcd_words.p + 1, ctx->h_stage.p + 128, sizeof ls, cudaMemcpyHostToDevice, st));
-        hafpcdk::lzf_decompress_kernel<<<1, 32, 0, st>>>(reinterpret_cast<const hafpcdk::LzfStream*>(ctx->d_pcd_words.p + 1), d_flags);
-        LAUNCHED(ctx);
-        hafpcdk::gather_soa_kernel<<<grid_pts, 256, 0, st>>>(ctx->d_pcd_blob.p, npts, foff[hd.idx[0]], foff[hd.idx[1]], foff[hd.idx[2]], 4 * hd.counts[hd.idx[0]],
-                                                             4 * hd.counts[hd.idx[1]], 4 * hd.counts[hd.idx[2]], ctx->d_pcd_xyz.p);
-        LAUNCHED(ctx);
-        CUDA_TRY(ctx, cudaMemcpyAsync(h_words, ctx->d_pcd_words.p, 16 * 8, cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(ctx, cudaStreamSynchronize(st));
-        if (reinterpret_cast<const int*>(h_words + 8)[0]) return ctx->fail(HAF_ERR_IO, "corrupt LZF stream in the PCD data");
-    } else {
-        return ctx->fail(HAF_ERR_UNSUPPORTED, "unsupported PCD DATA kind '%s'", hd.data_kind.c_str());
-    }
-    *d_xyz = ctx->d_pcd_xyz.p;
-    *n_points = npts;
-    return HAF_OK;
+    const size_t file_offsets[2] = {0, n_bytes};
+    size_t point_offsets[2];
+    const int rc = pcd_decode_files(ctx, reinterpret_cast<const unsigned char*>(file_bytes), file_offsets, 1, false, d_xyz, point_offsets);
+    if (rc == HAF_OK) *n_points = point_offsets[1];
+    return rc;
+}
+
+extern "C" int haf_pcd_decode_batch(haf_ctx* ctx, const void* files, const size_t* file_offsets, int n_files, const float** d_xyz,
+                                    size_t* point_offsets) {
+    if (!ctx || !d_xyz) return HAF_ERR_ARG;
+    *d_xyz = nullptr;
+    if (!file_offsets || n_files < 1 || !point_offsets) return ctx->fail(HAF_ERR_ARG, "haf_pcd_decode_batch: bad arguments");
+    return pcd_decode_files(ctx, reinterpret_cast<const unsigned char*>(files), file_offsets, n_files, true, d_xyz, point_offsets);
 }
 
 extern "C" int haf_debug_pcd_xyz(haf_ctx* ctx, float* xyz_host, size_t n_points) {
@@ -2472,6 +2704,19 @@ extern "C" int haf_search_pcd(haf_ctx* ctx, const void* file_bytes, size_t n_byt
     const int rc = haf_pcd_decode(ctx, file_bytes, n_bytes, &d_xyz, &n);
     if (rc != HAF_OK) return rc;
     return haf_search(ctx, d_xyz, n, 12, reqs, n_requests, best, best_per_request, graspseval, mask, heights, per_roll_top);
+}
+
+extern "C" int haf_search_batch_pcd(haf_ctx* ctx, const void* files, const size_t* file_offsets, int n_files, const haf_request* reqs,
+                                    const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
+                                    haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll) {
+    if (!ctx) return HAF_ERR_ARG;
+    if (!file_offsets || n_files < 1) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_pcd: bad arguments");
+    std::vector<size_t> point_offsets(n_files + 1);
+    const float* d_xyz = nullptr;
+    const int rc = haf_pcd_decode_batch(ctx, files, file_offsets, n_files, &d_xyz, point_offsets.data());
+    if (rc != HAF_OK) return rc;
+    return haf_search_batch_requests(ctx, d_xyz, point_offsets.data(), n_files, reqs, request_offsets, best_per_cloud, best_per_request,
+                                     per_roll_top, grasp_per_cloud, grasp_per_request, grasp_per_roll);
 }
 
 // ------------------------------------------------------------------------------------------------------------

@@ -13,6 +13,7 @@
 #include <vector>
 
 #include "../../../include/hafgpu.h"
+#include "pcd_io.hpp"
 
 namespace haf_b200 {
 
@@ -95,6 +96,30 @@ public:
 
     // read_pc_cb (:250-329): goal -> members (the tf transform of the cloud is the caller's business), then loop_control
     void read_pc_cb(const GraspInput& goal, const float* xyz, size_t n_points, size_t stride_bytes) {
+        set_goal(goal);
+        loop_control(xyz, n_points, stride_bytes);
+    }
+
+    // One goal on every cloud of a batch: what loop_control leaves behind for each cloud when it runs on that cloud alone
+    struct CloudResult {
+        size_t n_points;
+        haf_best best;                          // row, col, roll, tilt, topval, rolls_done, n_windows_scored as loop_control reads them
+        GraspOutput gp_result;
+        std::vector<int> per_roll_top;          // [R][3]
+        std::vector<GraspOutput> published_per_roll;
+    };
+    // PCD files back to back in host memory (file f = bytes [file_offsets[f], file_offsets[f+1])), decoded on the device in one
+    // call (haf_search_batch_pcd)
+    std::vector<CloudResult> open_pcds_and_trig_get_grasps_cb(const GraspInput& goal, const void* files, const size_t* file_offsets, int n_files) {
+        return batch_control(goal, files, file_offsets, NULL, NULL, n_files);
+    }
+    // clouds already decoded on the host: packed xyz, cloud c = points [point_offsets[c], point_offsets[c+1]) (haf_search_batch_requests)
+    std::vector<CloudResult> read_pcs_cb(const GraspInput& goal, const float* xyz_all, const size_t* point_offsets, int n_clouds) {
+        return batch_control(goal, NULL, NULL, xyz_all, point_offsets, n_clouds);
+    }
+
+    // goal -> members (:258-326)
+    void set_goal(const GraspInput& goal) {
         graspsearchcenter = goal.grasp_area_center;                              // :258-260
         grasp_search_area_size_x_dir = (int)goal.grasp_area_length_x;             // :266-267
         grasp_search_area_size_y_dir = (int)goal.grasp_area_length_y;
@@ -108,34 +133,20 @@ public:
         return_only_best_gp = goal.show_only_best_grasp;                          // :284
         id_row_top_overall = id_col_top_overall = nr_roll_top_overall = nr_tilt_top_overall = -1;  // :322-326
         topval_gp_overall = -1000;
-        loop_control(xyz, n_points, stride_bytes);
     }
 
     // loop_control (:335-402): the five per-roll calls (:376-385) and the grasp poses of transform_gp_in_wcs_and_publish
     // (:1274-1401) are ONE haf_search_grasps call; the poses are computed on the device (haf_grasp records)
     void loop_control(const float* xyz, size_t n_points, size_t stride_bytes, int roll_limit = 0) {
-        haf_request rq;
-        memset(&rq, 0, sizeof rq);
-        rq.center[0] = graspsearchcenter.x; rq.center[1] = graspsearchcenter.y; rq.center[2] = graspsearchcenter.z;
-        rq.area_len_x = (float)grasp_search_area_size_x_dir; rq.area_len_y = (float)grasp_search_area_size_y_dir;
-        rq.approach[0] = raw_approach_.x; rq.approach[1] = raw_approach_.y; rq.approach[2] = raw_approach_.z;
-        rq.gripper_opening_width = gripper_opening_width;
-        rq.return_only_best = return_only_best_gp ? 1 : 0;
-        rq.graspval_top = graspval_top;
-        rq.roll_limit = roll_limit;
+        haf_request rq = request(roll_limit);
         haf_grasp grasp;
         int rc = haf_search_grasps(ctx_, xyz, n_points, stride_bytes, &rq, 1, &best, NULL, graspseval.data(), point_inside_box_grid.data(),
                                    heightsgridroll.data(), per_roll_top.data(), &grasp, NULL, grasp_per_roll_.data());
         if (rc != HAF_OK) throw std::runtime_error(std::string("hafgpu: ") + haf_last_error(ctx_));
-        published_per_roll.clear();
+        published_per_roll = published(per_roll_top.data(), grasp_per_roll_.data(), best.rolls_done);
         // av_trans_mat (:484) = generate_grid's matrix of the roll just evaluated; only its third row is read (:1370-1374), and
         // that row is the same for every roll (S * Rroll leaves it untouched)
         haf_build_transform(&rq, best.roll >= 0 ? best.roll : 0, step_deg_, av_trans_mat);
-        for (int roll = 0; roll < best.rolls_done; roll++) {                      // what show_predicted_gps did per roll
-            const int* t = &per_roll_top[roll * 3];
-            if (!return_only_best_gp && t[2] > graspval_th)                        // :962-972 (eval = max(top - 20, 10) in the record)
-                published_per_roll.push_back(to_grasp_output(grasp_per_roll_[roll]));
-        }
         id_row_top_overall = best.row; id_col_top_overall = best.col; nr_roll_top_overall = best.roll;       // :953-960
         nr_tilt_top_overall = best.tilt; topval_gp_overall = best.topval;
         gp_result = to_grasp_output(grasp);                                       // :390 (eval = topval_gp_overall - 20)
@@ -155,6 +166,64 @@ public:
     }
 
     haf_ctx* ctx() { return ctx_; }
+
+private:
+    // the request loop_control sends for the current members
+    haf_request request(int roll_limit) const {
+        haf_request rq;
+        memset(&rq, 0, sizeof rq);
+        rq.center[0] = graspsearchcenter.x; rq.center[1] = graspsearchcenter.y; rq.center[2] = graspsearchcenter.z;
+        rq.area_len_x = (float)grasp_search_area_size_x_dir; rq.area_len_y = (float)grasp_search_area_size_y_dir;
+        rq.approach[0] = raw_approach_.x; rq.approach[1] = raw_approach_.y; rq.approach[2] = raw_approach_.z;
+        rq.gripper_opening_width = gripper_opening_width;
+        rq.return_only_best = return_only_best_gp ? 1 : 0;
+        rq.graspval_top = graspval_top;
+        rq.roll_limit = roll_limit;
+        return rq;
+    }
+    // what show_predicted_gps published per evaluated roll (:962-972; eval = max(top - 20, 10) in the record)
+    std::vector<GraspOutput> published(const int* top, const haf_grasp* grasp_per_roll, int rolls_done) const {
+        std::vector<GraspOutput> out;
+        for (int roll = 0; roll < rolls_done; roll++)
+            if (!return_only_best_gp && top[roll * 3 + 2] > graspval_th) out.push_back(to_grasp_output(grasp_per_roll[roll]));
+        return out;
+    }
+    // one haf_search_batch_pcd (files) or haf_search_batch_requests (xyz_all) call with the goal's request for every cloud
+    std::vector<CloudResult> batch_control(const GraspInput& goal, const void* files, const size_t* file_offsets, const float* xyz_all,
+                                           const size_t* point_offsets, int n) {
+        set_goal(goal);
+        const std::vector<haf_request> reqs(n, request(0));
+        std::vector<haf_best> best_c(n);
+        std::vector<int> top((size_t)n * R * 3, -1);
+        std::vector<haf_grasp> grasp_c(n), grasp_r((size_t)n * R);
+        const int rc = files ? haf_search_batch_pcd(ctx_, files, file_offsets, n, reqs.data(), NULL, best_c.data(), NULL, top.data(), grasp_c.data(),
+                                                    NULL, grasp_r.data())
+                             : haf_search_batch_requests(ctx_, xyz_all, point_offsets, n, reqs.data(), NULL, best_c.data(), NULL, top.data(),
+                                                         grasp_c.data(), NULL, grasp_r.data());
+        if (rc != HAF_OK) throw std::runtime_error(std::string("hafgpu: ") + haf_last_error(ctx_));
+        std::vector<size_t> pts(n + 1, 0);
+        if (files) {   // the clouds' sizes: the headers' POINTS (the call above has parsed every header)
+            for (int c = 0; c < n; c++) {
+                hafpcd::PcdHeader hd;
+                hafpcd::parse_pcd_header(static_cast<const unsigned char*>(files) + file_offsets[c], file_offsets[c + 1] - file_offsets[c], hd, NULL);
+                pts[c + 1] = pts[c] + (size_t)hd.npts;
+            }
+        } else {
+            pts.assign(point_offsets, point_offsets + n + 1);
+        }
+        std::vector<CloudResult> out(n);
+        for (int c = 0; c < n; c++) {
+            CloudResult& r = out[c];
+            r.n_points = pts[c + 1] - pts[c];
+            r.best = best_c[c];
+            r.gp_result = to_grasp_output(grasp_c[c]);
+            r.per_roll_top.assign(top.begin() + (size_t)c * R * 3, top.begin() + (size_t)(c + 1) * R * 3);
+            r.published_per_roll = published(r.per_roll_top.data(), grasp_r.data() + (size_t)c * R, best_c[c].rolls_done);
+        }
+        return out;
+    }
+
+public:
 
 private:
     haf_ctx* ctx_ = nullptr;

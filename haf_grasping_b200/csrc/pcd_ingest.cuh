@@ -12,6 +12,8 @@
 //   * binary_compressed -- u32 compressed size, u32 uncompressed size, one LZF stream (liblzf, as embedded in PCL), fields
 //                          stored struct-of-arrays;
 //   * fromROSMsg        -- x / y / z FLOAT32 at their declared byte offsets inside records of point_step bytes.
+// A call takes a batch of files / buffers (haf_pcd_decode and haf_pointcloud2_to_xyz are batches of one): every cloud keeps
+// the semantics above, and each data kind present runs one fixed sequence of launches over all its clouds.
 // The text header stays on the host (csrc/host/pcd_io.hpp, parse_pcd_header).  Parity: byte-equal xyz with the host reader
 // (csrc/host/pcd_io.hpp, haf_grasping_b200/pcd.py) on every bundled PCD and on generated files (tests/test_pcd_device.py).
 #pragma once
@@ -27,23 +29,35 @@ __device__ __forceinline__ float load_f32_any(const unsigned char* p) {   // rec
     const uint32_t u = (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
     return __uint_as_float(u);
 }
-// binary PCD records / PointCloud2 data: x, y, z at byte offsets ox, oy, oz of records of rec_bytes bytes
-__global__ void gather_records_kernel(const unsigned char* __restrict__ rec, size_t n, size_t rec_bytes, int ox, int oy, int oz,
-                                      float* __restrict__ xyz) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-        const unsigned char* r = rec + i * rec_bytes;
-        xyz[3 * i] = load_f32_any(r + ox);
-        xyz[3 * i + 1] = load_f32_any(r + oy);
-        xyz[3 * i + 2] = load_f32_any(r + oz);
-    }
-}
-// binary_compressed after the LZF stage: field arrays one after the other (all x, all y, all z ...); stride = 4 * COUNT
-__global__ void gather_soa_kernel(const unsigned char* __restrict__ blob, size_t n, size_t fx, size_t fy, size_t fz, int sx, int sy, int sz,
-                                  float* __restrict__ xyz) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-        xyz[3 * i] = load_f32_any(blob + fx + i * sx);
-        xyz[3 * i + 1] = load_f32_any(blob + fy + i * sy);
-        xyz[3 * i + 2] = load_f32_any(blob + fz + i * sz);
+
+// ---------------------------------------------------------------------------------------------------------------------
+// A call decodes a BATCH of files or PointCloud2 buffers (a single one is the batch of one): each data kind present runs one
+// fixed sequence of launches over all its clouds, described by tables the host sends in one parameter block.
+// ---------------------------------------------------------------------------------------------------------------------
+// Gather: point i of segment s has x / y / z at src + off[a] + i * stride[a]; it becomes point out_begin + i of the packed
+// output.  Binary PCD records (stride = record bytes for all three), the struct-of-arrays blob of binary_compressed files
+// after the LZF stage (stride = 4 * COUNT), PointCloud2 records (stride = point_step).
+struct GatherSeg {
+    const unsigned char* src;
+    unsigned long long out_begin;
+    unsigned long long off[3], stride[3];
+};
+// seg_begin [n_segs + 1]: exclusive prefix of the segments' point counts (no empty segment); a point finds its segment by
+// binary search
+__global__ void gather_segments_kernel(const GatherSeg* __restrict__ segs, const unsigned long long* __restrict__ seg_begin, int n_segs,
+                                       float* __restrict__ xyz) {
+    const unsigned long long n = seg_begin[n_segs];
+    for (unsigned long long p = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; p < n; p += (unsigned long long)gridDim.x * blockDim.x) {
+        int lo = 0, hi = n_segs - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (seg_begin[mid] <= p) lo = mid; else hi = mid - 1;
+        }
+        const GatherSeg& S = segs[lo];
+        const unsigned long long i = p - seg_begin[lo], o = 3 * (S.out_begin + i);
+        xyz[o] = load_f32_any(S.src + S.off[0] + i * S.stride[0]);
+        xyz[o + 1] = load_f32_any(S.src + S.off[1] + i * S.stride[1]);
+        xyz[o + 2] = load_f32_any(S.src + S.off[2] + i * S.stride[2]);
     }
 }
 
@@ -53,7 +67,7 @@ __global__ void gather_soa_kernel(const unsigned char* __restrict__ blob, size_t
 // WARP per stream -- all lanes read the control bytes from a shared-memory ring of the input, the lanes copy a token's bytes
 // together (an overlapping reference repeats its `distance` bytes: source index (k mod distance)), back references read a
 // 16 KB shared-memory ring of the output, so no global load sits on the token chain.  status: 0 ok, 1 corrupt stream.
-// grid = streams (a batch of clouds decodes one stream per CTA), block = 32.
+// grid = streams (a batch of files decodes one stream per CTA, each into its own range of one blob buffer), block = 32.
 // ---------------------------------------------------------------------------------------------------------------------
 #define HAF_LZF_IN_RING 8192
 #define HAF_LZF_OUT_RING 16384
@@ -113,13 +127,23 @@ __global__ void __launch_bounds__(32) lzf_decompress_kernel(const LzfStream* __r
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// ASCII.  A byte is a RECORD START when it begins a line that holds at least one token.  Three passes over the text in tiles of
-// 256 threads x 16 bytes: count record starts per tile; exclusive scan of the tile counts (one CTA); rank the starts, and
-// the thread that owns start number r < POINTS parses the record into xyz[r].
+// ASCII.  A byte is a RECORD START when it begins a line that holds at least one token.  Three passes over the data sections
+// of all ASCII files of a batch, in tiles of 256 threads x 16 bytes; each section starts a new tile (tile_file: tile -> file):
+// count record starts per tile; exclusive scan of the tile counts over the whole batch (one CTA); rank the starts -- the
+// rank within a file is the batch rank minus the scan value at the file's first tile -- and the thread that owns start number
+// r < POINTS of its file parses the record into point out_begin + r.
 // ---------------------------------------------------------------------------------------------------------------------
 #define HAF_PCD_TILE_THREADS 256
 #define HAF_PCD_BYTES_PER_THREAD 16
+struct AsciiFile {
+    unsigned long long begin, len;           // data section in the device copy of the batch
+    unsigned long long n_points, out_begin;  // POINTS, first output point
+    int tile_begin, tile_end;                // tiles [tile_begin, tile_end)
+    int tok[3];                              // token numbers of x, y, z inside a record (COUNT-aware)
+    int pad;
+};
 __device__ __forceinline__ bool is_blank(unsigned char c) { return c == ' ' || c == '\t' || c == '\r'; }
+// t: one file's data section of n bytes (its first byte is a line start, the scan stops at its end)
 __device__ __forceinline__ bool record_starts_at(const unsigned char* __restrict__ t, size_t n, size_t i) {
     if (i > 0 && t[i - 1] != '\n') return false;
     for (size_t k = i; k < n; k++) {     // a line of blanks only is no record
@@ -144,17 +168,27 @@ __device__ __forceinline__ unsigned block_exclusive_scan(unsigned v, unsigned* s
     *total = all;
     return before + incl - v;
 }
-__global__ void __launch_bounds__(HAF_PCD_TILE_THREADS) ascii_count_kernel(const unsigned char* __restrict__ text, size_t n, unsigned* __restrict__ tile_count) {
-    __shared__ unsigned s_warp[HAF_PCD_TILE_THREADS / 32];
-    const size_t b0 = ((size_t)blockIdx.x * HAF_PCD_TILE_THREADS + threadIdx.x) * HAF_PCD_BYTES_PER_THREAD;
-    unsigned c = 0;
+// record-start bit mask of this thread's 16 bytes of tile blockIdx.x
+__device__ __forceinline__ unsigned tile_starts(const unsigned char* __restrict__ raw, const AsciiFile& F, size_t* b0_out) {
+    const unsigned char* text = raw + F.begin;
+    const size_t b0 = ((size_t)(blockIdx.x - F.tile_begin) * HAF_PCD_TILE_THREADS + threadIdx.x) * HAF_PCD_BYTES_PER_THREAD;
+    unsigned mask = 0;
     for (int k = 0; k < HAF_PCD_BYTES_PER_THREAD; k++)
-        if (b0 + k < n && record_starts_at(text, n, b0 + k)) c++;
+        if (b0 + k < F.len && record_starts_at(text, F.len, b0 + k)) mask |= 1u << k;
+    *b0_out = b0;
+    return mask;
+}
+__global__ void __launch_bounds__(HAF_PCD_TILE_THREADS) ascii_count_kernel(const unsigned char* __restrict__ raw, const AsciiFile* __restrict__ files,
+                                                                           const int* __restrict__ tile_file, unsigned* __restrict__ tile_count) {
+    __shared__ unsigned s_warp[HAF_PCD_TILE_THREADS / 32];
+    const AsciiFile F = files[tile_file[blockIdx.x]];
+    size_t b0;
+    const unsigned c = __popc(tile_starts(raw, F, &b0));
     unsigned total;
     block_exclusive_scan(c, s_warp, &total);
     if (threadIdx.x == 0) tile_count[blockIdx.x] = total;
 }
-// in place: tile_count -> exclusive offsets (64-bit totals are not needed: POINTS < 2^32); total[0] = number of records
+// in place: tile_count -> exclusive offsets (the host keeps the records of a batch below 2^32); total[0] = number of records
 __global__ void __launch_bounds__(1024) ascii_scan_kernel(unsigned* __restrict__ tile_count, unsigned n_tiles, unsigned long long* __restrict__ total) {
     __shared__ unsigned s_warp[32];
     __shared__ unsigned long long s_carry;
@@ -182,25 +216,32 @@ __global__ void __launch_bounds__(1024) ascii_scan_kernel(unsigned* __restrict__
     }
     if (threadIdx.x == 0) *total = s_carry;
 }
-// tok_x / tok_y / tok_z: token numbers of the three fields inside a record (COUNT-aware).  flags[0]: a record had fewer
-// tokens than that; flags[1]: a token outside what the conversion reproduces exactly (> 19 digits next to a rounding boundary)
-__global__ void __launch_bounds__(HAF_PCD_TILE_THREADS) ascii_parse_kernel(const unsigned char* __restrict__ text, size_t n,
-                                                                           const unsigned* __restrict__ tile_offset, unsigned long long n_points,
-                                                                           int tok_x, int tok_y, int tok_z, float* __restrict__ xyz,
-                                                                           int* __restrict__ flags) {
+// Per ASCII file a: count[a] = its records (the first tile's CTA writes it: scan value at the next file's first tile, or the
+// batch total, minus the scan value at its own); flags[2a]: a record had fewer tokens than the three fields need;
+// flags[2a + 1]: a token outside what the conversion reproduces exactly (> 19 digits next to a rounding boundary)
+__global__ void __launch_bounds__(HAF_PCD_TILE_THREADS) ascii_parse_kernel(const unsigned char* __restrict__ raw, const AsciiFile* __restrict__ files,
+                                                                           const int* __restrict__ tile_file, const unsigned* __restrict__ tile_offset,
+                                                                           unsigned n_tiles, const unsigned long long* __restrict__ total,
+                                                                           float* __restrict__ xyz, unsigned* __restrict__ count, int* __restrict__ flags) {
     __shared__ unsigned s_warp[HAF_PCD_TILE_THREADS / 32];
-    const size_t b0 = ((size_t)blockIdx.x * HAF_PCD_TILE_THREADS + threadIdx.x) * HAF_PCD_BYTES_PER_THREAD;
-    unsigned mask = 0;
-    for (int k = 0; k < HAF_PCD_BYTES_PER_THREAD; k++)
-        if (b0 + k < n && record_starts_at(text, n, b0 + k)) mask |= 1u << k;
-    unsigned total;
-    unsigned long long rank = (unsigned long long)tile_offset[blockIdx.x] + block_exclusive_scan(__popc(mask), s_warp, &total);
+    const int a = tile_file[blockIdx.x];
+    const AsciiFile F = files[a];
+    const unsigned base = tile_offset[F.tile_begin];
+    if (blockIdx.x == (unsigned)F.tile_begin && threadIdx.x == 0)
+        count[a] = ((unsigned)F.tile_end < n_tiles ? tile_offset[F.tile_end] : (unsigned)*total) - base;
+    const unsigned char* text = raw + F.begin;
+    const size_t n = F.len;
+    size_t b0;
+    unsigned mask = tile_starts(raw, F, &b0);
+    unsigned tile_total;
+    unsigned long long rank = (unsigned long long)(tile_offset[blockIdx.x] - base) + block_exclusive_scan(__popc(mask), s_warp, &tile_total);
+    const int tok_x = F.tok[0], tok_y = F.tok[1], tok_z = F.tok[2];
     const int tmax = max(tok_x, max(tok_y, tok_z));
     while (mask) {
         const int k = __ffs(mask) - 1;
         mask &= mask - 1;
         const unsigned long long r = rank++;
-        if (r >= n_points) break;      // exactly POINTS records; further lines are ignored
+        if (r >= F.n_points) break;      // exactly POINTS records; further lines are ignored
         size_t p = b0 + k;
         float v[3] = {0.0f, 0.0f, 0.0f};
         int tok = 0;
@@ -219,9 +260,10 @@ __global__ void __launch_bounds__(HAF_PCD_TILE_THREADS) ascii_parse_kernel(const
             tok++;
             p = e;
         }
-        if (tok <= tmax) flags[0] = 1;
-        if (uns) flags[1] = 1;
-        xyz[3 * r] = v[0]; xyz[3 * r + 1] = v[1]; xyz[3 * r + 2] = v[2];
+        if (tok <= tmax) flags[2 * a] = 1;
+        if (uns) flags[2 * a + 1] = 1;
+        const unsigned long long o = 3 * (F.out_begin + r);
+        xyz[o] = v[0]; xyz[o + 1] = v[1]; xyz[o + 2] = v[2];
     }
 }
 

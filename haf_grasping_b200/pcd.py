@@ -63,6 +63,31 @@ def read_pcd(path: str) -> np.ndarray:
         return read_pcd_bytes(fh.read(), path)
 
 
+def header_points(raw) -> int:
+    """the point count a PCD header declares: POINTS, else WIDTH * HEIGHT (HEIGHT defaults to 1).  raw: bytes-like; only the
+    header is read."""
+    mv = memoryview(raw).cast("B")
+    n = 4096
+    while True:
+        head = bytes(mv[:n])
+        hdr = {}
+        lines = head.split(b"\n")
+        complete = lines if n >= len(mv) else lines[:-1]
+        for ln in complete:
+            toks = ln.split()
+            if not toks or toks[0].startswith(b"#"):
+                continue
+            hdr[toks[0]] = toks[1:]
+            if toks[0] == b"DATA":
+                break
+        if b"DATA" in hdr or n >= len(mv):
+            break
+        n *= 4
+    if b"POINTS" in hdr:
+        return int(hdr[b"POINTS"][0])
+    return int(hdr.get(b"WIDTH", [b"0"])[0]) * int(hdr.get(b"HEIGHT", [b"1"])[0])
+
+
 def read_pcd_bytes(raw: bytes, path: str = "<bytes>") -> np.ndarray:
     pos = 0
     hdr = {}

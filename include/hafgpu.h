@@ -254,9 +254,35 @@ int haf_pcd_decode(haf_ctx* ctx, const void* file_bytes, size_t n_bytes, const f
 int haf_search_pcd(haf_ctx* ctx, const void* file_bytes, size_t n_bytes, const haf_request* reqs, int n_requests, haf_best* best,
                    haf_best* best_per_request, float* graspseval, unsigned char* mask, float* heights, int* per_roll_top);
 /* sensor_msgs/PointCloud2 -> packed xyz on the device (pcl::fromROSMsg for PointXYZ): n_points records of point_step bytes
- * (host or device memory), x / y / z float32 at byte offsets off_x / off_y / off_z (any alignment). */
+ * (host or device memory), x / y / z float32 at byte offsets off_x / off_y / off_z (any alignment).  The batch of one of
+ * haf_pointcloud2_batch_to_xyz. */
 int haf_pointcloud2_to_xyz(haf_ctx* ctx, const void* data_hostdev, size_t n_points, size_t point_step, int off_x, int off_y, int off_z,
                            const float** d_xyz);
+
+/* ---- batches of PCD files and PointCloud2 buffers --------------------------------------------------------------------
+ * files: n_files PCD files concatenated in HOST memory (pinned or pageable); file f = bytes [file_offsets[f], file_offsets[f+1]).
+ * Kinds may be mixed; POINTS 0 is an empty cloud.  *d_xyz: packed xyz of every cloud in DEVICE memory owned by the context
+ * (valid until the next ingest call); point_offsets [n_files+1] (out) from the headers' POINTS.  Every cloud is decoded as
+ * haf_pcd_decode decodes one file (haf_pcd_decode is this call with one file); the number of kernel launches does not grow
+ * with the number of files: per data kind present one sequence over all its files (ASCII: count, scan, parse; binary_compressed:
+ * one LZF launch with one CTA per file; binary and binary_compressed: one gather), then one stream sync.  Pinned input is copied
+ * in one cudaMemcpyAsync; pageable input of 4 MB and more goes through the library's staging thread in pieces cut on file
+ * boundaries.  Errors: the single-file code and text, prefixed "PCD file <i>: ".  Header and size checks run on the host
+ * before any device work (the lowest such file is named); otherwise the lowest file the decode flags is named.  On error
+ * nothing is written.  ASCII data of a batch is limited to 2^32 records and 2^31 tiles of 4 KB (HAF_ERR_UNSUPPORTED).
+ * Multi-GPU context: the decode runs on its first GPU. */
+int haf_pcd_decode_batch(haf_ctx* ctx, const void* files, const size_t* file_offsets, int n_files,
+                         const float** d_xyz, size_t* point_offsets);
+/* haf_pcd_decode_batch + haf_search_batch_requests on the decoded clouds; arguments and outputs as there */
+int haf_search_batch_pcd(haf_ctx* ctx, const void* files, const size_t* file_offsets, int n_files,
+                         const haf_request* reqs, const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request,
+                         int* per_roll_top, haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll);
+/* PointCloud2 data of n_clouds clouds (host or device): cloud c = bytes [byte_offsets[c], byte_offsets[c+1]), a whole number of
+ * records of layouts[c][0] bytes with x / y / z float32 at byte offsets layouts[c][1..3]; rows without padding
+ * (row_step = width * point_step).  One gather launch for the whole batch.  *d_xyz and point_offsets [n_clouds+1] (out) as
+ * in haf_pcd_decode_batch; HAF_ERR_ARG naming the cloud for an offset + 4 > step or a span that is not a multiple of the step. */
+int haf_pointcloud2_batch_to_xyz(haf_ctx* ctx, const void* data_hostdev, const size_t* byte_offsets, int n_clouds,
+                                 const int* layouts, const float** d_xyz, size_t* point_offsets);
 
 /* ---- libsvm-compatible front ends (SURVEY 8f-3) ----------------------------------------------------------------
  * The reference classifies by running two child processes per roll on text files (server.cpp:775-776, :786-792):
@@ -351,7 +377,8 @@ int haf_debug_cell_indices(haf_ctx* ctx, const float* xyz_hostdev, size_t n_poin
 int haf_debug_text_roundtrip(haf_ctx* ctx, const float* in4, int n4, double* out4, const double* in6, int n6,
                              double* out6);
 
-/* packed xyz of the last haf_pcd_decode / haf_pointcloud2_to_xyz, copied to host memory (n_points records) */
+/* packed xyz of the last ingest call (haf_pcd_decode[_batch], haf_pointcloud2[_batch]_to_xyz; all clouds of a batch: total
+ * points), copied to host memory (n_points records) */
 int haf_debug_pcd_xyz(haf_ctx* ctx, float* xyz_host, size_t n_points);
 
 /* cycle counters of the role threads of the last X-resident tensor kernel launch made under HAF_TC_DEBUG=32 (timing
