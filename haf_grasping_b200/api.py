@@ -59,6 +59,16 @@ class haf_grasp(C.Structure):
                         list(self.approachVector) + [self.roll], np.float64)
 
 
+class haf_rank_params(C.Structure):
+    """parameters of haf_search_batch_candidates (include/hafgpu.h)"""
+    _fields_ = [("k", C.c_int), ("per_unit", C.c_int), ("min_distance", C.c_double), ("reserved", C.c_int * 4)]
+
+
+class haf_candidate(C.Structure):
+    """one ranked grasp candidate: the full haf_grasp, the graspseval value of its cell and its request within the cloud"""
+    _fields_ = [("grasp", haf_grasp), ("score", C.c_float), ("request", C.c_int)]
+
+
 class haf_info(C.Structure):
     _fields_ = [("n_features", C.c_int), ("n_dims", C.c_int), ("n_sv", C.c_int), ("n_rolls", C.c_int), ("grid", C.c_int),
                 ("label0", C.c_int), ("label1", C.c_int), ("sm_count", C.c_int), ("gamma", C.c_double),
@@ -76,7 +86,7 @@ class haf_timing(C.Structure):
 
 EXPORTS = ["haf_create", "haf_destroy", "haf_last_error", "haf_get_info", "haf_set_stream", "haf_set_profiling",
            "haf_get_timing", "haf_launch_count", "haf_set_debug", "haf_search", "haf_search_batch", "haf_search_batch_packed",
-           "haf_search_grasps", "haf_search_batch_packed_grasps", "haf_search_batch_requests", "haf_debug_unit_params", "haf_debug_chunk_copy_waits", "haf_debug_heights", "haf_build_transform", "haf_build_transform_wcs", "haf_best_key", "haf_pack_best_records", "haf_debug_window_count", "haf_debug_windows", "haf_debug_features",
+           "haf_search_grasps", "haf_search_batch_packed_grasps", "haf_search_batch_requests", "haf_search_batch_candidates", "haf_debug_unit_params", "haf_debug_chunk_copy_waits", "haf_debug_heights", "haf_build_transform", "haf_build_transform_wcs", "haf_best_key", "haf_pack_best_records", "haf_debug_window_count", "haf_debug_windows", "haf_debug_features",
            "haf_debug_decisions", "haf_debug_tensor_inputs", "haf_debug_integral", "haf_debug_cell_indices", "haf_debug_text_roundtrip", "haf_debug_tc_probe",
            "haf_version", "haf_pcd_decode", "haf_search_pcd", "haf_pointcloud2_to_xyz", "haf_debug_pcd_xyz",
            "haf_pcd_decode_batch", "haf_search_batch_pcd", "haf_pointcloud2_batch_to_xyz", "haf_svm_create", "haf_svm_create_config", "haf_svm_destroy", "haf_svm_predict", "haf_svm_predict_probability", "haf_svm_check_probability_model", "haf_scale_minmax", "haf_scale_apply"]
@@ -121,6 +131,8 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
                                                  C.POINTER(haf_grasp), C.POINTER(haf_grasp)]
     L.haf_search_batch_requests.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(haf_request), C.POINTER(ci), C.POINTER(haf_best),
                                             C.POINTER(haf_best), vp, C.POINTER(haf_grasp), C.POINTER(haf_grasp), C.POINTER(haf_grasp)]
+    L.haf_search_batch_candidates.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(haf_request), C.POINTER(ci), C.POINTER(haf_rank_params),
+                                              C.POINTER(haf_best), C.POINTER(haf_grasp), C.POINTER(haf_candidate), vp]
     L.haf_debug_unit_params.argtypes = [vp, vp, vp, vp, ci]
     L.haf_debug_chunk_copy_waits.argtypes = [vp, vp, ci]
     L.haf_debug_heights.argtypes = [vp, vp, cs]
@@ -411,6 +423,39 @@ class GraspSearch:
         if top is not None:
             out["per_roll_top"] = top
         return out
+
+    def search_batch_candidates(self, xyz_all, point_offsets, requests, request_offsets=None, k=16, per_unit=0, min_distance=0.0,
+                                rank_params=None):
+        """The k best distinct grasps of every cloud (haf_search_batch_candidates), inputs as ``search_batch_requests``.  Returns a
+        dict: ``best`` and ``grasp`` per cloud, ``candidates`` (haf_candidate array [n_clouds * k], cloud c at [c * k, c * k +
+        n_candidates[c])) and ``n_candidates`` (int32 [n_clouds]).  rank_params: a haf_rank_params to pass as it is (overrides k,
+        per_unit and min_distance)."""
+        if not isinstance(requests, C.Array):
+            requests = (haf_request * len(requests))(*requests)
+        rp = rank_params
+        if rp is None:
+            rp = haf_rank_params()
+            rp.k, rp.per_unit, rp.min_distance = int(k), int(per_unit), float(min_distance)
+        n_clouds = len(point_offsets) - 1
+        off = (C.c_size_t * len(point_offsets))(*[int(o) for o in point_offsets])
+        roff = None if request_offsets is None else (C.c_int * len(request_offsets))(*[int(o) for o in request_offsets])
+        best, grasp = (haf_best * n_clouds)(), (haf_grasp * n_clouds)()
+        cand = (haf_candidate * (n_clouds * max(int(rp.k), 1)))()
+        ncand = np.zeros(n_clouds, np.int32)
+        if isinstance(xyz_all, np.ndarray):
+            xyz_all = np.ascontiguousarray(xyz_all, np.float32)
+        self._check(self.L.haf_search_batch_candidates(self.h, _ptr(xyz_all), off, n_clouds, requests, roff, C.byref(rp), best, grasp,
+                                                       cand, _ptr(ncand)))
+        return {"best": best, "grasp": grasp, "candidates": cand, "n_candidates": ncand}
+
+    def search_candidates(self, xyz, requests=None, k=16, per_unit=0, min_distance=0.0):
+        """``search_batch_candidates`` for one cloud (packed float32 [n, 3], host array or CUDA tensor) and its requests."""
+        if requests is None:
+            requests = [make_request()]
+        if isinstance(requests, haf_request):
+            requests = [requests]
+        return self.search_batch_candidates(xyz, [0, len(xyz)], requests, [0, len(requests)], k=k, per_unit=per_unit,
+                                            min_distance=min_distance)
 
     def debug_unit_params(self, n_units, poses=True):
         """unit parameters of the last search (haf_debug_unit_params): (M [U, 16], mask [U, 10], Minv [U, 16] or None)"""

@@ -166,6 +166,7 @@ struct haf_ctx {
         DevBuf<signed char> d_labelgrid;
         DevBuf<int2> d_win;
         DevBuf<int> d_guardlist, d_guardlist2;
+        DevBuf<uint2> d_rank_tiles;
     } alt[3];
     cudaStream_t chunk_stream2[3] = {nullptr, nullptr, nullptr};
     cudaEvent_t ev_dual[4];             // [0] head of the call done on the main stream, [1 + k] extra stream k drained
@@ -197,6 +198,7 @@ struct haf_ctx {
     struct GraphKey {
         unsigned long long epoch; const void* xyz; size_t stride, wcap; long long pts_bucket; int n_jobs, n_clouds, flags, tc_passes;
         const void *o_evals, *o_mask, *o_heights; unsigned long long rolls_hash; cudaStream_t st;
+        int rank_k, rank_p; double rank_md2;   // candidate ranking (0 when off)
         bool operator==(const GraphKey& o) const { return memcmp(this, &o, sizeof *this) == 0; }
     };
     // a few graphs per context, least recently used out: a goal sharded over ranks alternates between two or three shapes
@@ -238,6 +240,16 @@ struct haf_ctx {
     DevBuf<UnitParams> d_dev_units;      // [U]
     DevBuf<UnitPose> d_dev_pose;         // [U] one pose per unit
     PinBuf<float> h_best_M;              // [n_jobs][16] matrix of each job's winning roll (written by reduce_rolls_kernel, UVA)
+
+    // ranked candidates (haf_search_batch_candidates, kernels.cuh rank_*_kernel); set for one call by RankScope.  rank_k 0 = off.
+    int rank_k = 0, rank_p = 0;          // candidates per cloud, list depth per unit
+    double rank_md2 = -1.0;              // min_distance^2; -1 = no suppression
+    DevBuf<CandRec> d_rank_entries;      // [U][P] unit lists (call-wide, written chunk by chunk)
+    DevBuf<RankCompact> d_rank_compact;  // [U][P]
+    DevBuf<float> d_rank_top_score;      // [U] graspseval value of each unit's top cell
+    DevBuf<uint2> d_rank_tiles;          // [Uc][tiles][P] per-tile selections (G > 90)
+    PinBuf<CandRec> h_cand;              // [n_clouds][k], written by rank_cloud_kernel (UVA)
+    PinBuf<int> h_ncand;                 // [n_clouds]
     // where the unit parameters of the last call live, whichever path built them (haf_debug_unit_params); units 0 = none
     const UnitParams* last_up_units = nullptr;
     const UnitPose* last_up_pose = nullptr;   // NULL: the call built no poses
@@ -301,7 +313,7 @@ static void swap_chunk_ws(haf_ctx* c, int k = 0) {
     HAF_SWAP(d_Xh); HAF_SWAP(d_Xl); HAF_SWAP(d_asum); HAF_SWAP(d_integral); HAF_SWAP(d_evals); HAF_SWAP(d_X); HAF_SWAP(d_xn); HAF_SWAP(d_probgrid);
     HAF_SWAP(d_dec_tc); HAF_SWAP(d_rowscan); HAF_SWAP(d_dec); HAF_SWAP(d_kscratch); HAF_SWAP(d_Xg); HAF_SWAP(d_g2accum); HAF_SWAP(d_xn64);
     HAF_SWAP(d_keys); HAF_SWAP(d_g2tickets); HAF_SWAP(d_mask); HAF_SWAP(d_guardflag); HAF_SWAP(d_labelgrid); HAF_SWAP(d_win);
-    HAF_SWAP(d_guardlist); HAF_SWAP(d_guardlist2);
+    HAF_SWAP(d_guardlist); HAF_SWAP(d_guardlist2); HAF_SWAP(d_rank_tiles);
 #undef HAF_SWAP
 }
 
@@ -1041,12 +1053,13 @@ extern "C" void haf_destroy(haf_ctx* ctx) {
     ctx->d_svn64.release(); ctx->d_Xg.release(); ctx->d_xn64.release(); ctx->d_g2accum.release(); ctx->d_g2tickets.release(); ctx->d_guardlist2.release();
     ctx->d_SVh.release(); ctx->d_SVl.release(); ctx->d_Xh.release(); ctx->d_Xl.release(); ctx->d_svcoef.release(); ctx->d_dec_tc.release(); ctx->d_asum.release(); ctx->d_dimfeat.release(); ctx->d_round4.release();
     ctx->d_params.release(); ctx->d_counters.release(); ctx->h_stage.release(); ctx->h_results.release(); ctx->h_per_roll_top.release(); ctx->h_counters.release(); ctx->h_unit_windows.release();
+    ctx->d_rank_tiles.release();
     for (int k = 0; k < 3; k++) {
     swap_chunk_ws(ctx, k);   // the further sets of per-chunk buffers (host-staged batches, one per extra stream)
     ctx->d_keys.release(); ctx->d_integral.release(); ctx->d_rowscan.release(); ctx->d_mask.release(); ctx->d_labelgrid.release(); ctx->d_evals.release();
     ctx->d_win.release(); ctx->d_X.release(); ctx->d_xn.release(); ctx->d_dec.release(); ctx->d_guardflag.release(); ctx->d_guardlist.release(); ctx->d_kscratch.release();
     ctx->d_probgrid.release(); ctx->d_Xg.release(); ctx->d_xn64.release(); ctx->d_g2accum.release(); ctx->d_g2tickets.release(); ctx->d_guardlist2.release();
-    ctx->d_Xh.release(); ctx->d_Xl.release(); ctx->d_dec_tc.release(); ctx->d_asum.release();
+    ctx->d_Xh.release(); ctx->d_Xl.release(); ctx->d_dec_tc.release(); ctx->d_asum.release(); ctx->d_rank_tiles.release();
     if (ctx->chunk_stream2[k]) cudaStreamDestroy(ctx->chunk_stream2[k]);
     }
     if (ctx->ev_dual_ok) for (int k = 0; k < 4; k++) cudaEventDestroy(ctx->ev_dual[k]);
@@ -1054,6 +1067,7 @@ extern "C" void haf_destroy(haf_ctx* ctx) {
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
     ctx->h_out_evals.release(); ctx->h_out_heights.release(); ctx->h_out_mask.release(); ctx->h_ring.release();
     ctx->d_unit_grasp.release(); ctx->h_unit_grasp.release(); ctx->h_job_grasp.release();
+    ctx->d_rank_entries.release(); ctx->d_rank_compact.release(); ctx->d_rank_top_score.release(); ctx->h_cand.release(); ctx->h_ncand.release();
     if (ctx->ev_ok) for (int i = 0; i < 10; i++) cudaEventDestroy(ctx->ev[i]);
     for (size_t i = 0; i < ctx->ev_pool.size(); i++) cudaEventDestroy(ctx->ev_pool[i]);
     for (size_t i = 0; i < ctx->copy_ev.size(); i++) cudaEventDestroy(ctx->copy_ev[i]);
@@ -1346,6 +1360,7 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
     ctx->last_up_n = 0;
     ctx->last_chunk_waits.clear();
     const bool grasp = ctx->grasp_mode > 0;
+    const bool rank = ctx->rank_k > 0;   // (RankScope: only with grasp poses)
     if (dev_units) {   // distinct approach vectors (bitwise), in order of first occurrence
         ctx->approach_trig.clear(); ctx->approach_index.clear(); ctx->job_approach.resize(n_jobs);
         for (int j = 0; j < n_jobs; j++) {
@@ -1507,6 +1522,16 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
         ENSURE(ctx, ctx->d_unit_grasp, U); ENSURE(ctx, ctx->h_job_grasp, n_jobs);
         if (ctx->grasp_mode > 1) ENSURE(ctx, ctx->h_unit_grasp, U);
     }
+    const int rank_P = ctx->rank_p;
+    // one CTA per unit selects from the grid itself up to HAF_RANK_TILE cells, tiles of that many cells above
+    const int rank_tiles = rank && G * G > HAF_RANK_TILE ? (G * G + HAF_RANK_TILE - 1) / HAF_RANK_TILE : 0;
+    int rank_cap = 0;   // entries of the largest cloud's lists walked in shared memory (larger clouds: in place)
+    if (rank) {
+        ENSURE(ctx, ctx->d_rank_entries, (size_t)U * rank_P); ENSURE(ctx, ctx->d_rank_compact, (size_t)U * rank_P);
+        ENSURE(ctx, ctx->d_rank_top_score, U); ENSURE(ctx, ctx->h_cand, (size_t)n_clouds * ctx->rank_k); ENSURE(ctx, ctx->h_ncand, n_clouds);
+        for (int c = 0; c < n_clouds; c++) rank_cap = std::max(rank_cap, (hub[c + 1] - hub[c]) * rank_P);
+        rank_cap = std::min(rank_cap, (int)((46 * 1024) / sizeof(RankCompact)));
+    }
     ENSURE(ctx, ctx->d_unit_block, (size_t)2 * U + (U + 1) / 2);
     unsigned long long* const d_unit_top = ctx->d_unit_block.p;
     unsigned long long* const d_unit_run = d_unit_top + U;
@@ -1559,6 +1584,7 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
         // (grasp poses: the two pose kernels, the record copies and the size of the parameter block belong to the graph too)
         gkey.flags = (prob ? 1 : 0) | (keep_debug_state ? 2 : 0) | (avg_points_all >= 8 * (long long)GG ? 4 : 0) | (ctx->cfg.emulate_text_roundtrip ? 8 : 0) |
                      (ctx->grasp_mode << 4) | (dev_units ? 64 : 0) | ((dev_units ? n_approach : n_pose_sets) << 8);
+        if (rank) { gkey.rank_k = ctx->rank_k; gkey.rank_p = rank_P; gkey.rank_md2 = ctx->rank_md2; }
         gkey.tc_passes = ctx->tc_passes; gkey.o_evals = dst_evals; gkey.o_mask = dst_mask; gkey.o_heights = dst_heights; gkey.rolls_hash = hsh; gkey.st = st;
         for (size_t i = 0; i < ctx->graphs.size() && gmode == 0; i++)
             if (ctx->graphs[i].key == gkey) { gmode = 2; graph_slot = (int)i; }
@@ -1791,6 +1817,22 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
                                                                R, ctx->cfg.roll_step_deg, ctx->d_unit_grasp.p + ubase);
             LAUNCHED(ctx);
         }
+        if (rank) {   // each unit's candidate list, while evals / mask / heights of the chunk are resident
+            if (rank_tiles) {
+                ENSURE(ctx, ctx->d_rank_tiles, (size_t)Uc * rank_tiles * rank_P);
+                rank_tile_kernel<<<dim3(rank_tiles, Uc), HAF_RANK_THREADS, 0, st>>>(ctx->d_evals.p, ctx->d_mask.p, G, units_c, d_jobs, d_unit_top, R,
+                                                                                   rank_P, ctx->d_rank_tiles.p);
+                LAUNCHED(ctx);
+                rank_unit_kernel<true><<<Uc, HAF_RANK_THREADS, 0, st>>>(ctx->d_evals.p, ctx->d_mask.p, ctx->d_keys.p, G, units_c, d_jobs, d_unit_top, d_unit_run,
+                                                                        ubase, R, d_pose, d_jpose, ctx->cfg.roll_step_deg, rank_P, ctx->d_rank_tiles.p,
+                                                                        rank_tiles, ctx->d_rank_entries.p, ctx->d_rank_compact.p, ctx->d_rank_top_score.p);
+            } else {
+                rank_unit_kernel<false><<<Uc, HAF_RANK_THREADS, 0, st>>>(ctx->d_evals.p, ctx->d_mask.p, ctx->d_keys.p, G, units_c, d_jobs, d_unit_top, d_unit_run,
+                                                                         ubase, R, d_pose, d_jpose, ctx->cfg.roll_step_deg, rank_P, nullptr, 0,
+                                                                         ctx->d_rank_entries.p, ctx->d_rank_compact.p, ctx->d_rank_top_score.p);
+            }
+            LAUNCHED(ctx);
+        }
         if (prof) CUDA_TRY(ctx, cudaEventRecord(ctx->ev_pool[ci * 8 + 7], st));
 
         // bookkeeping per chunk: window / guard counts accumulate on the device ([8] windows, [9] guard), no host sync
@@ -1829,6 +1871,13 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
         grasp_gather_kernel<<<(n_jobs + 127) / 128, 128, 0, st>>>(ctx->d_results.p, n_jobs, d_units, d_pose, d_jpose, R, G, ctx->cfg.roll_step_deg,
                                                                  ctx->d_unit_grasp.p, ctx->h_job_grasp.p);
         LAUNCHED(ctx);
+        if (rank) {   // the ranked candidates of every cloud, straight into pinned host memory as well
+            rank_cloud_kernel<<<n_clouds, 256, (size_t)rank_cap * sizeof(RankCompact), st>>>(ctx->d_results.p, d_cloud_ubegin, R, G, ctx->d_unit_grasp.p,
+                                                                                            ctx->d_rank_top_score.p, ctx->d_rank_entries.p,
+                                                                                            ctx->d_rank_compact.p, rank_P, ctx->rank_k, ctx->rank_md2,
+                                                                                            rank_cap, ctx->h_cand.p, ctx->h_ncand.p);
+            LAUNCHED(ctx);
+        }
         if (ctx->grasp_mode > 1)
             CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_unit_grasp.p, ctx->d_unit_grasp.p, (size_t)U * sizeof(GraspRec), cudaMemcpyDeviceToHost, st));
     }
@@ -2010,6 +2059,22 @@ struct DeviceUnitsScope {
     explicit DeviceUnitsScope(haf_ctx* ctx) : c(ctx) { c->device_units = true; }
     ~DeviceUnitsScope() { c->device_units = false; }
 };
+// ranked candidates for the length of one call (haf_search_batch_candidates): the parameters, checked, and where the records go
+struct RankOut {
+    int k, per_unit;
+    double md2;                       // min_distance^2, -1 = no suppression
+    haf_candidate* candidates;        // [n_clouds][k]
+    int* n_candidates;                // [n_clouds]
+};
+static_assert(sizeof(haf_candidate) == sizeof(CandRec) && offsetof(haf_candidate, score) == offsetof(CandRec, score) &&
+              offsetof(haf_candidate, request) == offsetof(CandRec, request), "haf_candidate and CandRec must share their layout");
+struct RankScope {
+    haf_ctx* c;
+    RankScope(haf_ctx* ctx, const RankOut* ro) : c(ctx) {
+        c->rank_k = ro ? ro->k : 0; c->rank_p = ro ? ro->per_unit : 0; c->rank_md2 = ro ? ro->md2 : -1.0;
+    }
+    ~RankScope() { c->rank_k = 0; c->rank_p = 0; c->rank_md2 = -1.0; }
+};
 // per-roll records of the evaluated rolls of each job: h_unit_grasp -> out [n_jobs][R] (the other rolls are left untouched)
 static void copy_roll_grasps(const haf_ctx* ctx, const std::vector<Job>& jobs, haf_grasp* out) {
     const int R = ctx->R;
@@ -2026,7 +2091,7 @@ static int group_batch_packed(haf_ctx* ctx, const float* xyz_all, const size_t* 
                               haf_best* best_per_cloud, const GraspOut* go = nullptr);
 static int group_batch_requests(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
                                 const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
-                                haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll);
+                                haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll, const RankOut* rank = nullptr);
 static void group_timing(haf_ctx* ctx);
 
 // one GPU: the context itself (also what each member of a multi-GPU group runs -- group[0] IS the head context, so the
@@ -2038,7 +2103,7 @@ static int batch_packed_single(haf_ctx* ctx, const float* xyz_all, const size_t*
                                haf_best* best_per_cloud, const GraspOut* go = nullptr);
 static int batch_requests_single(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
                                  const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
-                                 haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll);
+                                 haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll, const RankOut* rank = nullptr);
 static int batch_single(haf_ctx* ctx, const float* const* clouds, const size_t* n_points, int n_clouds, const haf_request* req,
                         haf_best* best_per_cloud);
 
@@ -2243,6 +2308,9 @@ static int batch_packed_single(haf_ctx* ctx, const float* xyz_all, const size_t*
     return HAF_OK;
 }
 
+static int batch_requests_entry(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
+                                const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
+                                haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll, const RankOut* rank);
 extern "C" int haf_search_batch_requests(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
                                          const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
                                          haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll) {
@@ -2250,6 +2318,33 @@ extern "C" int haf_search_batch_requests(haf_ctx* ctx, const float* xyz_all, con
     if (!point_offsets || n_clouds < 1 || !reqs || !best_per_cloud) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_requests: bad arguments");
     if (!grasp_per_cloud && (grasp_per_request || grasp_per_roll))
         return ctx->fail(HAF_ERR_ARG, "haf_search_batch_requests: grasp_per_request / grasp_per_roll need grasp_per_cloud");
+    return batch_requests_entry(ctx, xyz_all, point_offsets, n_clouds, reqs, request_offsets, best_per_cloud, best_per_request, per_roll_top,
+                                grasp_per_cloud, grasp_per_request, grasp_per_roll, nullptr);
+}
+extern "C" int haf_search_batch_candidates(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
+                                           const int* request_offsets, const haf_rank_params* rp, haf_best* best_per_cloud,
+                                           haf_grasp* grasp_per_cloud, haf_candidate* candidates, int* n_candidates) {
+    if (!ctx) return HAF_ERR_ARG;
+    if (!point_offsets || n_clouds < 1 || !reqs || !rp || !best_per_cloud || !grasp_per_cloud || !candidates || !n_candidates)
+        return ctx->fail(HAF_ERR_ARG, "haf_search_batch_candidates: bad arguments");
+    if (rp->k < 1 || rp->k > 256) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_candidates: k = %d outside 1..256", rp->k);
+    const int per_unit = rp->per_unit == 0 ? std::max(rp->k, 64) : rp->per_unit;
+    if (per_unit < rp->k || per_unit > 1024)
+        return ctx->fail(HAF_ERR_ARG, "haf_search_batch_candidates: per_unit = %d outside k..1024 (0 = max(k, 64))", rp->per_unit);
+    if (std::isnan(rp->min_distance)) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_candidates: min_distance is NaN");
+    for (int i = 0; i < 4; i++)
+        if (rp->reserved[i]) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_candidates: reserved[%d] must be 0", i);
+    RankOut ro;
+    ro.k = rp->k; ro.per_unit = per_unit;
+    ro.md2 = rp->min_distance > 0 ? rp->min_distance * rp->min_distance : -1.0;
+    ro.candidates = candidates; ro.n_candidates = n_candidates;
+    return batch_requests_entry(ctx, xyz_all, point_offsets, n_clouds, reqs, request_offsets, best_per_cloud, nullptr, nullptr,
+                                grasp_per_cloud, nullptr, nullptr, &ro);
+}
+// arguments checked above, request_offsets aside
+static int batch_requests_entry(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
+                                const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
+                                haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll, const RankOut* rank) {
     std::vector<int> one_each;
     if (!request_offsets) {
         one_each.resize(n_clouds + 1);
@@ -2261,16 +2356,18 @@ extern "C" int haf_search_batch_requests(haf_ctx* ctx, const float* xyz_all, con
         if (request_offsets[c + 1] <= request_offsets[c])
             return ctx->fail(HAF_ERR_ARG, "haf_search_batch_requests: cloud %d has no request (request_offsets must increase)", c);
     if ((long long)request_offsets[n_clouds] * ctx->R > 0x7fffffffLL) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_requests: too many requests");
+    if (rank && (long long)request_offsets[n_clouds] * ctx->R * rank->per_unit > 0x7fffffffLL)
+        return ctx->fail(HAF_ERR_ARG, "haf_search_batch_candidates: requests x rolls x per_unit above 2^31");
     if (ctx->group.size() > 1)
         return group_batch_requests(ctx, xyz_all, point_offsets, n_clouds, reqs, request_offsets, best_per_cloud, best_per_request, per_roll_top,
-                                    grasp_per_cloud, grasp_per_request, grasp_per_roll);
+                                    grasp_per_cloud, grasp_per_request, grasp_per_roll, rank);
     return batch_requests_single(ctx, xyz_all, point_offsets, n_clouds, reqs, request_offsets, best_per_cloud, best_per_request, per_roll_top,
-                                 grasp_per_cloud, grasp_per_request, grasp_per_roll);
+                                 grasp_per_cloud, grasp_per_request, grasp_per_roll, rank);
 }
 // request_offsets: checked, request_offsets[0] = 0
 static int batch_requests_single(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
                                  const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
-                                 haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll) {
+                                 haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll, const RankOut* rank) {
     CloudSet cs;
     { const int rc = prepare_batch(ctx, xyz_all, point_offsets, n_clouds, cs); if (rc) return rc; }
     StagerJoin stager_join{ctx};
@@ -2285,6 +2382,7 @@ static int batch_requests_single(haf_ctx* ctx, const float* xyz_all, const size_
         go.per_roll = grasp_per_roll;
         GraspScope gs(ctx, grasp_per_cloud ? &go : nullptr);
         DeviceUnitsScope ds(ctx);
+        RankScope rs(ctx, rank);
         rc = run_jobs(ctx, cs, jobs, nullptr, nullptr, nullptr, ctx->debug_keep_batch);
     }
     ctx->copy_pieces = 0;
@@ -2312,6 +2410,14 @@ static int batch_requests_single(haf_ctx* ctx, const float* xyz_all, const size_
     if (per_roll_top) memcpy(per_roll_top, ctx->h_per_roll_top.p, (size_t)n_reqs * R * 3 * sizeof(int));
     if (grasp_per_request) memcpy(grasp_per_request, ctx->h_job_grasp.p, (size_t)n_reqs * sizeof(haf_grasp));
     if (grasp_per_roll) copy_roll_grasps(ctx, jobs, grasp_per_roll);
+    if (rank)   // the slots after a cloud's n_candidates are zeroed
+        for (int c = 0; c < n_clouds; c++) {
+            const int nc = ctx->h_ncand.p[c];
+            rank->n_candidates[c] = nc;
+            haf_candidate* dst = rank->candidates + (size_t)c * rank->k;
+            memcpy(dst, ctx->h_cand.p + (size_t)c * rank->k, (size_t)nc * sizeof(haf_candidate));
+            memset(dst + nc, 0, (size_t)(rank->k - nc) * sizeof(haf_candidate));
+        }
     return HAF_OK;
 }
 
@@ -2911,7 +3017,7 @@ static int group_batch_packed(haf_ctx* ctx, const float* xyz_all, const size_t* 
 // (requests x R); each member writes its records straight into the caller's arrays.
 static int group_batch_requests(haf_ctx* ctx, const float* xyz_all, const size_t* point_offsets, int n_clouds, const haf_request* reqs,
                                 const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
-                                haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll) {
+                                haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll, const RankOut* rank) {
     const int n = (int)ctx->group.size(), R = ctx->R;
     const int* ro = request_offsets;
     std::vector<int> cb(n + 1, n_clouds);   // member k: clouds [cb[k], cb[k + 1])
@@ -2932,11 +3038,13 @@ static int group_batch_requests(haf_ctx* ctx, const float* xyz_all, const size_t
             const float* src = xyz_all + point_offsets[c0] * 3;
             const void* use = src;
             int rc = member_input(m, src, off[c1 - c0] * 12, &use);
+            RankOut mro;   // this member's clouds' candidates go straight to their place in the caller's arrays
+            if (rank) { mro = *rank; mro.candidates = rank->candidates + (size_t)c0 * rank->k; mro.n_candidates = rank->n_candidates + c0; }
             if (rc == HAF_OK)
                 rc = batch_requests_single(m, (const float*)use, off.data(), c1 - c0, reqs + r0, rof.data(), best_per_cloud + c0,
                                            best_per_request ? best_per_request + r0 : nullptr, per_roll_top ? per_roll_top + r0 * R * 3 : nullptr,
                                            grasp_per_cloud ? grasp_per_cloud + c0 : nullptr, grasp_per_request ? grasp_per_request + r0 : nullptr,
-                                           grasp_per_roll ? grasp_per_roll + r0 * R : nullptr);
+                                           grasp_per_roll ? grasp_per_roll + r0 * R : nullptr, rank ? &mro : nullptr);
             rcs[k] = rc;
         });
     }

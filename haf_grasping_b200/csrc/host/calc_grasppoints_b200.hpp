@@ -165,6 +165,25 @@ public:
         return out;
     }
 
+    // the goal's request on every file of a batch, decoded on the device (haf_pcd_decode_batch), then the ranked candidates of every
+    // cloud (haf_search_batch_candidates): cand [n][rp.k], ncand [n]
+    void rank_pcds_cb(const GraspInput& goal, const void* files, const size_t* file_offsets, int n, const haf_rank_params& rp,
+                      std::vector<haf_candidate>& cand, std::vector<int>& ncand) {
+        set_goal(goal);
+        const std::vector<haf_request> reqs(n, request(0));
+        std::vector<size_t> point_offsets(n + 1);
+        const float* d_xyz = NULL;
+        int rc = haf_pcd_decode_batch(ctx_, files, file_offsets, n, &d_xyz, point_offsets.data());
+        std::vector<haf_best> best_c(n);
+        std::vector<haf_grasp> grasp_c(n);
+        cand.assign((size_t)n * rp.k, haf_candidate());
+        ncand.assign(n, 0);
+        if (rc == HAF_OK)
+            rc = haf_search_batch_candidates(ctx_, d_xyz, point_offsets.data(), n, reqs.data(), NULL, &rp, best_c.data(), grasp_c.data(),
+                                             cand.data(), ncand.data());
+        if (rc != HAF_OK) throw std::runtime_error(std::string("hafgpu: ") + haf_last_error(ctx_));
+    }
+
     haf_ctx* ctx() { return ctx_; }
 
 private:

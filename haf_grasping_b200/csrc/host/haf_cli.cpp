@@ -5,6 +5,8 @@
 // --pcd may be repeated: the files are searched with the same goal in ONE batch call (haf_search_batch_pcd, or with --host-pcd
 // haf_search_batch_requests on the host-decoded clouds), one output line per file in argument order, each what a run on that
 // file alone prints.
+// --top K [--min-distance m] [--per-unit P]: after each file's line, the file's K best distinct grasps (haf_search_batch_candidates
+// on the files decoded by haf_pcd_decode_batch): one line per candidate, or with --json one object {"candidates": [...]}.
 //   haf_cli --pcd cloud.pcd --dump-pcd          (parse only, no GPU)
 #include <cstdio>
 #include <cstdlib>
@@ -23,6 +25,30 @@ static bool read_file(const std::string& path, std::vector<unsigned char>& out) 
     while ((nr = fread(buf, 1, sizeof buf, fp)) > 0) out.insert(out.end(), buf, buf + nr);
     fclose(fp);
     return true;
+}
+
+static void print_candidates(bool json, const haf_candidate* cand, int n) {
+    if (json) {
+        printf("{\"candidates\": [");
+        for (int i = 0; i < n; i++) {
+            const haf_candidate& c = cand[i];
+            const haf_grasp& g = c.grasp;
+            printf("%s{\"rank\": %d, \"eval\": %d, \"score\": %.9g, \"request\": %d, \"row\": %d, \"col\": %d, \"roll_index\": %d, \"roll\": %.9g, "
+                   "\"graspPoint1\": [%.17g, %.17g, %.17g], \"graspPoint2\": [%.17g, %.17g, %.17g], \"averagedGraspPoint\": [%.17g, %.17g, %.17g], "
+                   "\"approachVector\": [%.17g, %.17g, %.17g]}",
+                   i ? ", " : "", i, g.eval, (double)c.score, c.request, g.row, g.col, g.roll_index, (double)g.roll, g.graspPoint1[0], g.graspPoint1[1],
+                   g.graspPoint1[2], g.graspPoint2[0], g.graspPoint2[1], g.graspPoint2[2], g.averagedGraspPoint[0], g.averagedGraspPoint[1],
+                   g.averagedGraspPoint[2], g.approachVector[0], g.approachVector[1], g.approachVector[2]);
+        }
+        printf("]}\n");
+    } else {   // rank, then the fields of the line above, then score, row, col
+        for (int i = 0; i < n; i++) {
+            const haf_grasp& g = cand[i].grasp;
+            printf("top %d: %d %g %g %g %g %g %g %g %g %g %g %g %g %d %g %d %d\n", i, g.eval, g.graspPoint1[0], g.graspPoint1[1], g.graspPoint1[2],
+                   g.graspPoint2[0], g.graspPoint2[1], g.graspPoint2[2], g.approachVector[0], g.approachVector[1], g.approachVector[2],
+                   g.averagedGraspPoint[0], g.averagedGraspPoint[1], g.averagedGraspPoint[2], g.roll_index * 15, (double)cand[i].score, g.row, g.col);
+        }
+    }
 }
 
 static void print_result(bool json, size_t n_points, const haf_best& best, const haf_b200::GraspOutput& g, const int* per_roll_top, int R,
@@ -51,6 +77,8 @@ int main(int argc, char** argv) {
     haf_b200::GraspInput goal;
     int grid = 56, svm_mode = HAF_SVM_TENSOR_GUARD;
     bool json = false, dump_pcd = false, host_pcd = false;
+    haf_rank_params rank;
+    memset(&rank, 0, sizeof rank);
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i];
         auto need = [&](int n) { if (i + n >= argc) { fprintf(stderr, "haf_cli: %s needs %d value(s)\n", a.c_str(), n); exit(2); } };
@@ -68,6 +96,9 @@ int main(int argc, char** argv) {
         else if (a == "--json") json = true;
         else if (a == "--dump-pcd") dump_pcd = true;
         else if (a == "--host-pcd") host_pcd = true;
+        else if (a == "--top") { need(1); rank.k = atoi(argv[++i]); }
+        else if (a == "--min-distance") { need(1); rank.min_distance = atof(argv[++i]); }
+        else if (a == "--per-unit") { need(1); rank.per_unit = atoi(argv[++i]); }
         else { fprintf(stderr, "haf_cli: unknown argument %s\n", a.c_str()); return 2; }
     }
     if (dump_pcd && !pcd.empty()) {  // parse only (no GPU): point count + FNV-1a of the packed xyz bytes
@@ -84,6 +115,16 @@ int main(int argc, char** argv) {
         fprintf(stderr, "usage: haf_cli --features F --range R --model M --pcd cloud.pcd [--center x y z] [--area lx ly] [--approach x y z] [--width n] [--only-best] [--grid G] [--svm-mode m] [--json]\n");
         return 2;
     }
+    // --top: every file's bytes, for the candidate pass
+    std::vector<unsigned char> rank_files;
+    std::vector<size_t> rank_offsets(1, 0);
+    if (rank.k != 0)
+        for (size_t f = 0; f < pcds.size(); f++) {
+            if (!read_file(pcds[f], rank_files)) { fprintf(stderr, "haf_cli: cannot open %s\n", pcds[f].c_str()); return 1; }
+            rank_offsets.push_back(rank_files.size());
+        }
+    std::vector<haf_candidate> cand;
+    std::vector<int> ncand;
     if (pcds.size() > 1) {   // one batch call for all files
         std::vector<float> xyz_all;
         std::vector<unsigned char> files;
@@ -105,8 +146,11 @@ int main(int argc, char** argv) {
             const int n = (int)pcds.size();
             const std::vector<haf_b200::CCalc_Grasppoints_B200::CloudResult> res =
                 host_pcd ? server.read_pcs_cb(goal, xyz_all.data(), offsets.data(), n) : server.open_pcds_and_trig_get_grasps_cb(goal, files.data(), offsets.data(), n);
-            for (int f = 0; f < n; f++)
+            if (rank.k != 0) server.rank_pcds_cb(goal, rank_files.data(), rank_offsets.data(), n, rank, cand, ncand);
+            for (int f = 0; f < n; f++) {
                 print_result(json, res[f].n_points, res[f].best, res[f].gp_result, res[f].per_roll_top.data(), server.R, res[f].published_per_roll.size());
+                if (rank.k != 0) print_candidates(json, cand.data() + (size_t)f * rank.k, ncand[f]);
+            }
         } catch (const std::exception& e) {
             fprintf(stderr, "haf_cli: %s\n", e.what());
             return 1;
@@ -127,6 +171,10 @@ int main(int argc, char** argv) {
         if (host_pcd) server.read_pc_cb(goal, xyz.data(), n_points, 12);
         else n_points = server.open_pcd_and_trig_get_grasp_cb(goal, file_bytes.data(), file_bytes.size());
         print_result(json, n_points, server.best, server.gp_result, server.per_roll_top.data(), server.R, server.published_per_roll.size());
+        if (rank.k != 0) {
+            server.rank_pcds_cb(goal, rank_files.data(), rank_offsets.data(), 1, rank, cand, ncand);
+            print_candidates(json, cand.data(), ncand[0]);
+        }
     } catch (const std::exception& e) {
         fprintf(stderr, "haf_cli: %s\n", e.what());
         return 1;

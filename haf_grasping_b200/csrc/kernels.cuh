@@ -1701,6 +1701,17 @@ __device__ __forceinline__ int unit_top_cell(const unsigned long long* __restric
     return val;
 }
 
+// rolls [jp.roll_begin, end) of job j are the ones loop_control evaluates: the early exit of return_only_best (:362-365) replayed
+// on the unit tops (strict >, :953).  Shared by reduce_rolls_kernel and the candidate ranking (rank_unit_kernel).
+__device__ __forceinline__ int job_rolls_end(const unsigned long long* __restrict__ unit_top, const JobParams& jp, int j, int R) {
+    int best = -1000, roll = jp.roll_begin;
+    for (; roll < jp.n_rolls_active; roll++) {
+        if (jp.return_only_best && best >= jp.graspval_top) break;
+        best = max(best, (int)(unsigned)(unit_top[j * R + roll] >> 32) - (1 << 20));
+    }
+    return roll;
+}
+
 // per-unit tops (after the tie rule) + a15 cross-roll reduction with the loop_control rules
 // (server.cpp:362-365 early exit, :953-960 strict >).  One thread per job.  best_M (optional, pinned host memory [n_jobs][16]):
 // mat_transform of each job's winning roll, taken from units (jobs whose unit parameters were built on the device).
@@ -1720,8 +1731,8 @@ __global__ void reduce_rolls_kernel(const unsigned long long* __restrict__ unit_
         per_roll_top[(j * R + roll) * 3 + 1] = col;
         per_roll_top[(j * R + roll) * 3 + 2] = val;
     }
-    for (int roll = jp.roll_begin; roll < jp.n_rolls_active; roll++) {
-        if (jp.return_only_best && best >= jp.graspval_top) break;  // :362-365
+    const int roll_end = job_rolls_end(unit_top, jp, j, R);
+    for (int roll = jp.roll_begin; roll < roll_end; roll++) {
         const int u = j * R + roll;
         const int val = per_roll_top[u * 3 + 2];
         if (val > best) { best = val; brow = per_roll_top[u * 3]; bcol = per_roll_top[u * 3 + 1]; broll = roll; }  // :953
@@ -1820,6 +1831,324 @@ __global__ void grasp_gather_kernel(const JobResult* __restrict__ results, int n
     } else {
         grasp_pose(poses[job_pose[j] * R].Minv, units[j * R].M + 8, nullptr, G, r.row, r.col, -1, roll_step_deg, r.topval - 20, job_grasp + j);
     }
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Ranked grasp candidates (haf_search_batch_candidates).  Order of the cells of a cloud: score (graspseval) descending, then unit
+// u = job * R + roll ascending (request, then roll), then cell ascending.  Per chunk, while evals / mask / heights are resident,
+// rank_unit_kernel keeps each eligible unit's first P cells in that order (its "list") with their poses; a unit of more than
+// HAF_RANK_TILE cells is split over rank_tile_kernel CTAs first (each keeps the first P cells of its tile, in cell order; the unit's first P cells
+// are among them).  Per call, rank_cloud_kernel seeds rank 0 with the cloud's best grasp and walks the lists greedily.
+// The selection is a radix select on fkey(score) (4 passes of 8 bits over a block histogram) followed by an ordered compaction:
+// every cell above the threshold key and the first ones equal to it -- linear in the cells, no sort.
+// ---------------------------------------------------------------------------------------------------
+struct CandRec {       // = haf_candidate (include/hafgpu.h); in the [U][P] lists `request` holds the job index
+    GraspRec g;
+    float score;
+    int request;
+};
+static_assert(sizeof(CandRec) == 128, "CandRec layout");
+struct RankCompact {   // what the cloud walk reads of a list entry; cell < 0: empty slot, taken or suppressed
+    double avg[3];
+    unsigned key;      // fkey(score)
+    int cell;
+};
+static_assert(sizeof(RankCompact) == 32, "RankCompact layout");
+#define HAF_RANK_THREADS 512
+#define HAF_RANK_TILE 8192   // cells of one selection held in shared memory: one CTA per unit up to G = 90, tiles above
+
+struct RankSelectSmem {
+    unsigned hist[256];
+    unsigned wsum[HAF_RANK_THREADS / 32];
+    unsigned digit, remaining, all;
+};
+
+// exclusive count of p over the block, in thread order; total: the block's count
+__device__ __forceinline__ unsigned rank_block_scan(bool p, unsigned* wsum, unsigned& total) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned b = __ballot_sync(0xffffffffu, p);
+    if (lane == 0) wsum[warp] = __popc(b);
+    __syncthreads();
+    unsigned before = 0, tot = 0;
+    for (int w = 0; w < HAF_RANK_THREADS / 32; w++) {
+        const unsigned v = wsum[w];
+        before += w < warp ? v : 0u;
+        tot += v;
+    }
+    __syncthreads();
+    total = tot;
+    return before + __popc(b & ((1u << lane) - 1u));
+}
+
+// keyat(i), i < n: 0 = not eligible, else fkey(score).  Emits the first P eligible positions in (key descending, position ascending)
+// order -- every key above the P-th key and the first `remaining` equal to it -- as emit(i, key, slot), slots 0.. in position order.
+// Returns the number emitted (min(P, eligible)).  Block-uniform; every thread of the block calls it.
+template <class KeyAt, class Emit>
+__device__ int rank_block_select(KeyAt keyat, int n, int P, RankSelectSmem& sh, Emit emit) {
+    const int tid = threadIdx.x, lane = tid & 31;
+    unsigned prefix = 0, pmask = 0, remaining = (unsigned)P;
+    bool all = false;
+    for (int pass = 0; pass < 4 && !all; pass++) {
+        const int shift = 24 - 8 * pass;
+        for (int i = tid; i < 256; i += HAF_RANK_THREADS) sh.hist[i] = 0;
+        __syncthreads();
+        // warp-aggregated: label scores take few distinct values, so most lanes of a warp hit the same bin
+        for (int i0 = 0; i0 < n; i0 += HAF_RANK_THREADS) {
+            const int i = i0 + tid;
+            const unsigned k = i < n ? keyat(i) : 0u;
+            const unsigned bin = (k && (k & pmask) == prefix) ? ((k >> shift) & 255u) : 256u;
+            const unsigned same = __match_any_sync(0xffffffffu, bin);
+            if (bin < 256u && lane == __ffs(same) - 1) atomicAdd(&sh.hist[bin], (unsigned)__popc(same));
+        }
+        __syncthreads();
+        if (tid < 32) {   // lane l holds digits 255 - 8l .. 248 - 8l, descending
+            unsigned c[8], s = 0;
+#pragma unroll
+            for (int b = 0; b < 8; b++) { c[b] = sh.hist[255 - 8 * lane - b]; s += c[b]; }
+            unsigned incl = s;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const unsigned t = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o) incl += t;
+            }
+            const unsigned total = __shfl_sync(0xffffffffu, incl, 31);
+            if (lane == 0) sh.all = (pass == 0 && total <= (unsigned)P) ? 1u : 0u;
+            const unsigned excl = incl - s;
+            if (excl < remaining && remaining <= incl) {
+                unsigned acc = excl;
+                for (int b = 0; b < 8; b++) {
+                    if (acc + c[b] >= remaining) { sh.digit = 255u - 8u * lane - b; sh.remaining = remaining - acc; break; }
+                    acc += c[b];
+                }
+            }
+        }
+        __syncthreads();
+        all = sh.all != 0;
+        if (!all) {
+            prefix |= sh.digit << shift;
+            pmask |= 0xFFu << shift;
+            remaining = sh.remaining;
+            // every key of the threshold's bin is taken: the remaining digits cannot split it (T - 1 with nothing equal)
+            if (pass < 3 && sh.hist[sh.digit] == remaining) { prefix = prefix ? prefix - 1u : 0u; remaining = 0u; all = true; }
+        }
+        __syncthreads();   // (hist and digit are rewritten by the next pass)
+    }
+    // all: every key > prefix is taken (prefix 0 after pass 0: fewer eligible cells than P)
+    const unsigned T = prefix, take_eq = all ? 0u : remaining;
+    unsigned eq_base = 0, out_base = 0;
+    for (int i0 = 0; i0 < n && out_base < (unsigned)P; i0 += HAF_RANK_THREADS) {
+        const int i = i0 + tid;
+        const unsigned k = i < n ? keyat(i) : 0u;
+        const bool eq = k != 0u && k == T;
+        unsigned eq_total, take_total;
+        const unsigned eq_rank = eq_base + rank_block_scan(eq, sh.wsum, eq_total);
+        const bool take = k > T || (eq && eq_rank < take_eq);
+        const unsigned slot = out_base + rank_block_scan(take, sh.wsum, take_total);
+        if (take) emit(i, k, (int)slot);
+        eq_base += eq_total;
+        out_base += take_total;
+    }
+    return (int)out_base;
+}
+
+// unit u (global) is ranked: an active roll among the ones the reference loop evaluated for its job
+__device__ __forceinline__ bool rank_unit_eligible(const UnitParams& up, const JobParams* __restrict__ jobs,
+                                                   const unsigned long long* __restrict__ unit_top, int R) {
+    return up.cloud >= 0 && up.roll < job_rolls_end(unit_top, jobs[up.job], up.job, R);
+}
+__device__ __forceinline__ unsigned rank_cell_key(const float* __restrict__ evals, const unsigned char* __restrict__ mask, size_t idx) {
+    return mask[idx] == 1 ? fkey(evals[idx]) : 0u;
+}
+
+// grid (tiles per unit, units of the chunk): the first P eligible cells of each tile of HAF_RANK_TILE cells, in cell order, as
+// (key, cell) into tiles [Uc][n_tiles * P] (unused slots key 0)
+__global__ void __launch_bounds__(HAF_RANK_THREADS) rank_tile_kernel(const float* __restrict__ evals, const unsigned char* __restrict__ mask,
+                                                                     int G, const UnitParams* __restrict__ units, const JobParams* __restrict__ jobs,
+                                                                     const unsigned long long* __restrict__ unit_top, int R, int P,
+                                                                     uint2* __restrict__ tiles) {
+    __shared__ unsigned s_keys[HAF_RANK_TILE];
+    __shared__ RankSelectSmem sh;
+    const int u = blockIdx.y, tile = blockIdx.x, GG = G * G;
+    uint2* out = tiles + ((size_t)u * gridDim.x + tile) * P;
+    int n = 0;
+    if (rank_unit_eligible(units[u], jobs, unit_top, R)) {
+        const int c0 = tile * HAF_RANK_TILE;
+        n = min(HAF_RANK_TILE, GG - c0);
+        const size_t base = (size_t)u * GG + c0;
+        for (int i = threadIdx.x; i < n; i += HAF_RANK_THREADS) s_keys[i] = rank_cell_key(evals, mask, base + i);
+        __syncthreads();
+        n = rank_block_select([&](int i) { return s_keys[i]; }, n, P, sh,
+                              [&](int i, unsigned k, int slot) { out[slot] = make_uint2(k, (unsigned)(c0 + i)); });
+    }
+    for (int s = n + threadIdx.x; s < P; s += HAF_RANK_THREADS) out[s] = make_uint2(0u, 0u);
+}
+
+// one CTA per unit of the chunk: the unit's list -- its first P eligible cells with their poses (grasp_pose with the unit's heights,
+// eval = (int)score - 20) into entries / compact [U][P] (call-wide, so they outlive the chunk's buffers), the empty slots marked, and
+// the graspseval value of the unit's top cell into top_score [U].  FROM_TILES: the candidates are rank_tile_kernel's output.
+template <bool FROM_TILES>
+__global__ void __launch_bounds__(HAF_RANK_THREADS) rank_unit_kernel(const float* __restrict__ evals, const unsigned char* __restrict__ mask,
+                                                                     const unsigned* __restrict__ keys_heights, int G,
+                                                                     const UnitParams* __restrict__ units, const JobParams* __restrict__ jobs,
+                                                                     const unsigned long long* __restrict__ unit_top,
+                                                                     const unsigned long long* __restrict__ unit_run, int ubase, int R,
+                                                                     const UnitPose* __restrict__ poses, const int* __restrict__ job_pose,
+                                                                     int roll_step_deg, int P, const uint2* __restrict__ tiles, int n_tiles,
+                                                                     CandRec* __restrict__ entries, RankCompact* __restrict__ compact,
+                                                                     float* __restrict__ top_score) {
+    __shared__ unsigned s_keys[HAF_RANK_TILE];
+    __shared__ uint2 s_sel[1024];   // (key, cell) of the list's slots
+    __shared__ RankSelectSmem sh;
+    const int uc = blockIdx.x, u = ubase + uc, GG = G * G;
+    const UnitParams up = units[uc];
+    CandRec* ent = entries + (size_t)u * P;
+    RankCompact* cmp = compact + (size_t)u * P;
+    int n = 0;
+    if (rank_unit_eligible(up, jobs, unit_top, R)) {
+        const float* E = evals + (size_t)uc * GG;
+        const float* H = reinterpret_cast<const float*>(keys_heights) + (size_t)uc * GG;
+        if (threadIdx.x == 0) {
+            int row, col;
+            unit_top_cell(unit_top, unit_run, u, G, &row, &col);
+            top_score[u] = E[row * G + col];
+        }
+        // the selection only records (key, cell) per slot; the poses are built after it, all slots at once
+        auto emit = [&](int cell, unsigned k, int slot) { s_sel[slot] = make_uint2(k, (unsigned)cell); };
+        if (!FROM_TILES) {
+            for (int i = threadIdx.x; i < GG; i += HAF_RANK_THREADS) s_keys[i] = rank_cell_key(E, mask + (size_t)uc * GG, i);
+            __syncthreads();
+            n = rank_block_select([&](int i) { return s_keys[i]; }, GG, P, sh, [&](int i, unsigned k, int slot) { emit(i, k, slot); });
+        } else {
+            const uint2* T = tiles + (size_t)uc * n_tiles * P;
+            const int nt = n_tiles * P;
+            if (nt <= HAF_RANK_TILE) {
+                for (int i = threadIdx.x; i < nt; i += HAF_RANK_THREADS) s_keys[i] = T[i].x;
+                __syncthreads();
+                n = rank_block_select([&](int i) { return s_keys[i]; }, nt, P, sh, [&](int i, unsigned k, int slot) { emit((int)T[i].y, k, slot); });
+            } else {
+                n = rank_block_select([&](int i) { return T[i].x; }, nt, P, sh, [&](int i, unsigned k, int slot) { emit((int)T[i].y, k, slot); });
+            }
+        }
+        __syncthreads();
+        const float* Minv = poses[job_pose[up.job] * R + up.roll].Minv;
+        for (int s = threadIdx.x; s < n; s += HAF_RANK_THREADS) {
+            const unsigned k = s_sel[s].x;
+            const int cell = (int)s_sel[s].y;
+            CandRec c;
+            c.score = fkey_inv(k);
+            c.request = up.job;
+            grasp_pose(Minv, up.M + 8, H, G, cell / G, cell % G, up.roll, roll_step_deg, (int)c.score - 20, &c.g);
+            ent[s] = c;
+            RankCompact rc;
+            rc.avg[0] = c.g.avg[0]; rc.avg[1] = c.g.avg[1]; rc.avg[2] = c.g.avg[2];
+            rc.key = k; rc.cell = cell;
+            cmp[s] = rc;
+        }
+    }
+    for (int s = n + threadIdx.x; s < P; s += HAF_RANK_THREADS) {
+        RankCompact rc;
+        rc.avg[0] = rc.avg[1] = rc.avg[2] = 0.0; rc.key = 0u; rc.cell = -1;
+        cmp[s] = rc;
+    }
+}
+
+// one CTA per cloud, after grasp_gather_kernel.  Rank 0: the cloud's best grasp (winning request: strict >, earliest; its record of
+// grasp_gather_kernel, eval = topval - 20); its cell leaves the lists.  Then at most k - 1 times: the block-wide maximum of the order
+// key over the live entries of the cloud's lists, after every entry within min_distance of the last accepted candidate has been
+// suppressed (d2 = (dx dx + dy dy) + dz dz in double, no FMA; d2 < md2).  cand [n_clouds][k] / n_cand [n_clouds]: pinned host memory
+// (UVA).  The compact records are walked in shared memory when the cloud's n_units * P fit in cap entries, in place otherwise.
+__global__ void __launch_bounds__(256) rank_cloud_kernel(const JobResult* __restrict__ results, const int* __restrict__ cloud_ubegin, int R,
+                                                         int G, const GraspRec* __restrict__ unit_grasp, const float* __restrict__ top_score,
+                                                         const CandRec* __restrict__ entries, RankCompact* __restrict__ compact, int P,
+                                                         int k, double md2, int cap, CandRec* __restrict__ cand, int* __restrict__ n_cand) {
+    extern __shared__ RankCompact s_cmp[];
+    __shared__ unsigned long long s_hi[8];
+    __shared__ unsigned s_lo[8];
+    __shared__ int s_idx[8];
+    __shared__ double s_avg[3];
+    __shared__ int s_win;
+    __shared__ int s_taken[256];   // list index of candidate n (1 .. k - 1)
+    const int c = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int ub0 = cloud_ubegin[c], ub1 = cloud_ubegin[c + 1];
+    const int jb0 = ub0 / R, jb1 = ub1 / R;
+    CandRec* out = cand + (size_t)c * k;
+    int win = -1, wtop = -1000;
+    for (int j = jb0; j < jb1; j++)
+        if (results[j].topval > wtop) { wtop = results[j].topval; win = j; }
+    if (win < 0 || results[win].roll < 0) {   // no roll evaluated
+        if (tid == 0) n_cand[c] = 0;
+        return;
+    }
+    const JobResult rw = results[win];
+    const int uw_rel = win * R + rw.roll - ub0, cell_w = rw.row * G + rw.col;
+    const GraspRec* g0 = unit_grasp + win * R + rw.roll;
+    if (tid < 32) {   // rank 0, one 32-bit word per lane: words 0 eval, 30 score, 31 request
+        unsigned w = lane < 30 ? reinterpret_cast<const unsigned*>(g0)[lane] : 0u;
+        if (lane == 0) w = (unsigned)(rw.topval - 20);
+        if (lane == 30) w = __float_as_uint(top_score[win * R + rw.roll]);
+        if (lane == 31) w = (unsigned)(win - jb0);
+        reinterpret_cast<unsigned*>(out)[lane] = w;
+        if (tid == 0) { s_avg[0] = g0->avg[0]; s_avg[1] = g0->avg[1]; s_avg[2] = g0->avg[2]; }
+    }
+    const int N = (ub1 - ub0) * P;
+    RankCompact* cr = compact + (size_t)ub0 * P;
+    if (N <= cap) {
+        for (int i = tid; i < N; i += 256) s_cmp[i] = cr[i];
+        cr = s_cmp;
+    }
+    __syncthreads();
+    int n = 1;
+    for (; n < k; n++) {
+        const double ax = s_avg[0], ay = s_avg[1], az = s_avg[2];
+        unsigned long long bhi = 0ull;
+        unsigned blo = 0u;
+        int bidx = -1;
+        for (int i = tid; i < N; i += 256) {
+            const RankCompact e = cr[i];
+            if (e.cell < 0) continue;
+            const int urel = i / P;
+            bool drop = urel == uw_rel && e.cell == cell_w;
+            if (!drop) {
+                const double dx = __dsub_rn(e.avg[0], ax), dy = __dsub_rn(e.avg[1], ay), dz = __dsub_rn(e.avg[2], az);
+                const double d2 = __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
+                drop = d2 < md2;
+            }
+            if (drop) { cr[i].cell = -1; continue; }
+            const unsigned long long hi = ((unsigned long long)e.key << 32) | (unsigned long long)(0xFFFFFFFFu - (unsigned)urel);
+            const unsigned lo = 0xFFFFFFFFu - (unsigned)e.cell;
+            if (hi > bhi || (hi == bhi && lo > blo)) { bhi = hi; blo = lo; bidx = i; }
+        }
+#pragma unroll
+        for (int o = 16; o >= 1; o >>= 1) {
+            const unsigned long long ohi = __shfl_xor_sync(0xffffffffu, bhi, o);
+            const unsigned olo = __shfl_xor_sync(0xffffffffu, blo, o);
+            const int oidx = __shfl_xor_sync(0xffffffffu, bidx, o);
+            if (ohi > bhi || (ohi == bhi && olo > blo)) { bhi = ohi; blo = olo; bidx = oidx; }
+        }
+        if (lane == 0) { s_hi[warp] = bhi; s_lo[warp] = blo; s_idx[warp] = bidx; }
+        __syncthreads();
+        if (tid == 0) {
+            for (int w = 1; w < 8; w++)
+                if (s_hi[w] > bhi || (s_hi[w] == bhi && s_lo[w] > blo)) { bhi = s_hi[w]; blo = s_lo[w]; bidx = s_idx[w]; }
+            s_win = bidx;
+            if (bidx >= 0) {
+                const RankCompact e = cr[bidx];
+                s_avg[0] = e.avg[0]; s_avg[1] = e.avg[1]; s_avg[2] = e.avg[2];
+                cr[bidx].cell = -1;
+            }
+        }
+        __syncthreads();
+        const int wi = s_win;
+        if (wi < 0) break;
+        if (tid == 0) s_taken[n] = wi;
+    }
+    __syncthreads();
+    for (int i = 1 + warp; i < n; i += 8) {   // the records, one warp each; word 31: the job index -> the request index within the cloud
+        unsigned w = reinterpret_cast<const unsigned*>(entries + (size_t)ub0 * P + s_taken[i])[lane];
+        if (lane == 31) w -= (unsigned)jb0;
+        reinterpret_cast<unsigned*>(out + i)[lane] = w;
+    }
+    if (tid == 0) n_cand[c] = n;
 }
 
 // ---------------------------------------------------------------------------------------------------

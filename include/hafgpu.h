@@ -240,6 +240,40 @@ int haf_search_batch_requests(haf_ctx* ctx, const float* xyz_all_hostdev, const 
                               const haf_request* reqs, const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request,
                               int* per_roll_top, haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll);
 
+/* ---- ranked grasp candidates: the k best distinct grasps of every cloud ----------------------------------------------------
+ * What a pick pipeline asks for when IK or collision checking rejects the best grasp.  For cloud c, a cell (request q, roll r, row,
+ * col) is eligible when r is one of the rolls the reference loop evaluated for q ([roll_begin, roll_begin + rolls_done), the early
+ * exit of return_only_best included) and mask == 1 there; its score is its graspseval value.  Cells are ordered by score descending,
+ * then q, r, row, col ascending.  Each unit (q, r) contributes its first per_unit eligible cells in that order (its list).  Rank 0 is
+ * the cloud's best grasp, exactly grasp_per_cloud (tie rule cell, eval = topval - 20); its cell leaves the lists.  The union of the
+ * lists is then walked in order, and a cell is accepted unless an accepted candidate of the cloud lies within min_distance:
+ * d2 = (dx dx + dy dy) + dz dz between averagedGraspPoints in double, suppressed iff d2 < min_distance^2 (min_distance <= 0: no
+ * suppression), up to k candidates.  With min_distance <= 0 and per_unit >= k the list is the global top k of the eligible cells
+ * after rank 0.  Every candidate carries a full haf_grasp record, eval = (int)score - 20: transform_gp_in_wcs_and_publish of its cell
+ * with its roll's heights, bit-equal to the reference's arithmetic. */
+typedef struct {
+    int k;                 /* candidates per cloud, 1..256 */
+    int per_unit;          /* eligible cells each (request, roll) contributes, k..1024; 0 = max(k, 64) */
+    double min_distance;   /* metres between averagedGraspPoints of two candidates of one cloud; <= 0: no suppression */
+    int reserved[4];       /* must be 0 */
+} haf_rank_params;
+typedef struct {
+    haf_grasp grasp;       /* eval = (int)score - 20; row / col / roll_index = the cell */
+    float score;           /* graspseval value of the cell */
+    int request;           /* index within the cloud's request list */
+} haf_candidate;           /* 128 bytes */
+/* haf_search_batch_requests (same inputs, staging, chunking, streams, CUDA graphs, multi-GPU sharding; a single goal is n_clouds = 1)
+ * plus the ranked candidates: candidates [n_clouds][k], n_candidates [n_clouds] (<= k; the slots after them are zeroed).  A cloud with
+ * no evaluated roll gets 0 candidates (its grasp_per_cloud is the roll -1 record); one whose evaluated rolls have no eligible cell gets
+ * 1 (the best).  best_per_cloud / grasp_per_cloud as in haf_search_batch_requests.  All outputs in host memory.  Each chunk's units
+ * select their lists on the device with a radix select on the score and an ordered compaction (rank_unit_kernel; rank_tile_kernel
+ * first where G > 90); one CTA per cloud walks them (rank_cloud_kernel).  HAF_ERR_ARG: k, per_unit out of range, NaN min_distance,
+ * nonzero reserved, requests x R x per_unit above 2^31. */
+int haf_search_batch_candidates(haf_ctx* ctx, const float* xyz_all_hostdev, const size_t* point_offsets, int n_clouds,
+                                const haf_request* reqs, const int* request_offsets, const haf_rank_params* rp,
+                                haf_best* best_per_cloud, haf_grasp* grasp_per_cloud,
+                                haf_candidate* candidates /* [n_clouds][k] */, int* n_candidates /* [n_clouds] */);
+
 /* ---- PCD / PointCloud2 ingest on the device (SURVEY 8f-2) -----------------------------------------------------------
  * What the reference does on the CPU before the hot path starts: the client's pcl::io::loadPCDFile<pcl::PointXYZ>
  * (src/calc_grasppoints_action_client.cpp:137-157) and the server's pcl::fromROSMsg (src/calc_grasppoints_action_server.cpp
