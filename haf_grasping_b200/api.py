@@ -69,6 +69,17 @@ class haf_candidate(C.Structure):
     _fields_ = [("grasp", haf_grasp), ("score", C.c_float), ("request", C.c_int)]
 
 
+HAF_DEPTH_U16 = 1   # 16UC1 / mono16, 0 = no return
+HAF_DEPTH_F32 = 2   # 32FC1 metres, non-finite = no return
+
+
+class haf_depth_image(C.Structure):
+    """one depth image of haf_depth_to_xyz_batch (include/hafgpu.h): size, encoding, row step, intrinsics, scale and pose"""
+    _fields_ = [("width", C.c_int), ("height", C.c_int), ("encoding", C.c_int), ("has_pose", C.c_int), ("step", C.c_longlong),
+                ("fx", C.c_double), ("fy", C.c_double), ("cx", C.c_double), ("cy", C.c_double), ("depth_scale", C.c_float),
+                ("camera_to_base", C.c_float * 16), ("reserved", C.c_int * 3)]
+
+
 class haf_info(C.Structure):
     _fields_ = [("n_features", C.c_int), ("n_dims", C.c_int), ("n_sv", C.c_int), ("n_rolls", C.c_int), ("grid", C.c_int),
                 ("label0", C.c_int), ("label1", C.c_int), ("sm_count", C.c_int), ("gamma", C.c_double),
@@ -89,7 +100,7 @@ EXPORTS = ["haf_create", "haf_destroy", "haf_last_error", "haf_get_info", "haf_s
            "haf_search_grasps", "haf_search_batch_packed_grasps", "haf_search_batch_requests", "haf_search_batch_candidates", "haf_debug_unit_params", "haf_debug_chunk_copy_waits", "haf_debug_heights", "haf_build_transform", "haf_build_transform_wcs", "haf_best_key", "haf_pack_best_records", "haf_debug_window_count", "haf_debug_windows", "haf_debug_features",
            "haf_debug_decisions", "haf_debug_tensor_inputs", "haf_debug_integral", "haf_debug_cell_indices", "haf_debug_text_roundtrip", "haf_debug_tc_probe",
            "haf_version", "haf_pcd_decode", "haf_search_pcd", "haf_pointcloud2_to_xyz", "haf_debug_pcd_xyz",
-           "haf_pcd_decode_batch", "haf_search_batch_pcd", "haf_pointcloud2_batch_to_xyz", "haf_svm_create", "haf_svm_create_config", "haf_svm_destroy", "haf_svm_predict", "haf_svm_predict_probability", "haf_svm_check_probability_model", "haf_scale_minmax", "haf_scale_apply"]
+           "haf_pcd_decode_batch", "haf_search_batch_pcd", "haf_pointcloud2_batch_to_xyz", "haf_depth_to_xyz_batch", "haf_search_batch_depth", "haf_svm_create", "haf_svm_create_config", "haf_svm_destroy", "haf_svm_predict", "haf_svm_predict_probability", "haf_svm_check_probability_model", "haf_scale_minmax", "haf_scale_apply"]
 
 _lib = None
 
@@ -159,6 +170,9 @@ def load_library(build_if_missing: bool = True) -> C.CDLL:
     L.haf_search_batch_pcd.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(haf_request), C.POINTER(ci), C.POINTER(haf_best),
                                        C.POINTER(haf_best), vp, C.POINTER(haf_grasp), C.POINTER(haf_grasp), C.POINTER(haf_grasp)]
     L.haf_pointcloud2_batch_to_xyz.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(ci), C.POINTER(vp), C.POINTER(cs)]
+    L.haf_depth_to_xyz_batch.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(haf_depth_image), C.POINTER(vp), C.POINTER(cs)]
+    L.haf_search_batch_depth.argtypes = [vp, vp, C.POINTER(cs), ci, C.POINTER(haf_depth_image), C.POINTER(haf_request), C.POINTER(ci),
+                                         C.POINTER(haf_best), C.POINTER(haf_best), vp, C.POINTER(haf_grasp), C.POINTER(haf_grasp), C.POINTER(haf_grasp)]
     L.haf_svm_create.argtypes = [C.POINTER(vp), C.c_char_p, ci, ci, ci, C.c_float]
     L.haf_svm_create_config.argtypes = [C.POINTER(vp), C.POINTER(haf_config), ci]
     L.haf_svm_destroy.argtypes = [vp]
@@ -606,6 +620,115 @@ class GraspSearch:
         po = (C.c_size_t * (n + 1))()
         self._check(self.L.haf_pointcloud2_batch_to_xyz(self.h, _ptr(data), off, n, lay.ctypes.data_as(C.POINTER(C.c_int)), C.byref(d), po))
         return (d.value or 0), np.array(po[:], np.int64)
+
+    # ---- batches of depth images: back-projection and the camera -> base transform on the device ----
+    @staticmethod
+    def _depth_batch(images, intrinsics, poses, depth_scale):
+        """(data, byte_offsets, haf_depth_image array, n) of a batch.  images: a list of 2-D uint16 / float32 numpy arrays (row
+        stride may exceed the row: the step keeps it), one (N, H, W) numpy array or torch tensor (host, pinned or not, or CUDA; made
+        contiguous), or (data, byte_offsets, records) passed as they are.  intrinsics: (fx, fy, cx, cy) or one per image; poses:
+        None, one 4x4 camera -> base matrix or one per image (None entries: no pose); depth_scale: one value or one per image."""
+        if isinstance(images, tuple):
+            data, offs, recs = images
+            if not isinstance(recs, C.Array):
+                recs = (haf_depth_image * len(recs))(*recs)
+            return data, (C.c_size_t * len(offs))(*[int(o) for o in offs]), recs, len(recs)
+        if isinstance(images, list):
+            n = len(images)
+            shapes, encs, steps, bufs = [], [], [], []
+            for im in images:
+                if im.ndim != 2 or im.dtype not in (np.uint16, np.float32):
+                    raise ValueError("a depth image is a 2-D uint16 or float32 array")
+                h, w = im.shape
+                isz = im.itemsize
+                step = im.strides[0] if (im.strides[1] == isz and im.strides[0] >= w * isz) else w * isz
+                rows = np.zeros((h, step), np.uint8)
+                if h and w:
+                    rows[:, :w * isz] = np.ascontiguousarray(im).astype(im.dtype.newbyteorder("<"), copy=False).view(np.uint8).reshape(h, w * isz)
+                shapes.append((h, w)); encs.append(HAF_DEPTH_U16 if im.dtype == np.uint16 else HAF_DEPTH_F32); steps.append(step)
+                bufs.append(rows.reshape(-1))
+            data = np.concatenate(bufs) if bufs else np.zeros(0, np.uint8)
+            offs = [0] + np.cumsum([len(b) for b in bufs], dtype=np.int64).tolist()
+        else:
+            if len(images.shape) != 3:
+                raise ValueError("a stack of depth images is (N, H, W)")
+            n, h, w = (int(v) for v in images.shape)
+            if isinstance(images, np.ndarray):
+                if images.dtype not in (np.uint16, np.float32):
+                    raise ValueError("depth images are uint16 or float32")
+                images = np.ascontiguousarray(images)
+                isz, u16 = images.itemsize, images.dtype == np.uint16
+            else:
+                import torch
+                if images.dtype not in (torch.uint16, torch.float32, torch.int16):
+                    raise ValueError("depth images are uint16 or float32")
+                images = images.contiguous()
+                isz, u16 = images.element_size(), images.dtype != torch.float32
+            data, row = images, w * isz
+            shapes, encs, steps = [(h, w)] * n, [HAF_DEPTH_U16 if u16 else HAF_DEPTH_F32] * n, [row] * n
+            offs = [k * h * row for k in range(n + 1)]
+        recs = (haf_depth_image * n)()
+        names = [f[0] for f in haf_depth_image._fields_]
+        rec = np.frombuffer(recs, np.dtype({"names": names,
+                                            "formats": [np.int32] * 4 + [np.int64] + [np.float64] * 4 + [np.float32, (np.float32, 16), (np.int32, 3)],
+                                            "offsets": [getattr(haf_depth_image, f).offset for f in names],
+                                            "itemsize": C.sizeof(haf_depth_image)}))
+        if n:
+            rec["height"], rec["width"] = np.asarray(shapes, np.int32).reshape(n, 2).T
+            rec["encoding"], rec["step"] = encs, steps
+            K = np.broadcast_to(np.asarray(intrinsics, np.float64), (n, 4))
+            rec["fx"], rec["fy"], rec["cx"], rec["cy"] = K.T
+            rec["depth_scale"] = np.broadcast_to(np.asarray(depth_scale, np.float32), (n,))
+            if poses is not None and not isinstance(poses, (list, tuple)) and np.asarray(poses).ndim == 2:
+                rec["has_pose"], rec["camera_to_base"] = 1, np.asarray(poses, np.float32).reshape(16)
+            elif poses is not None:
+                for i, m in enumerate(poses):
+                    if m is not None:
+                        rec["has_pose"][i], rec["camera_to_base"][i] = 1, np.asarray(m, np.float32).reshape(16)
+        return data, (C.c_size_t * len(offs))(*[int(o) for o in offs]), recs, n
+
+    def depth_to_xyz_batch(self, images, intrinsics=None, poses=None, depth_scale=0.0):
+        """haf_depth_to_xyz_batch: depth images (see _depth_batch) -> (device pointer of the packed xyz of every cloud, point_offsets
+        int64 [n_images + 1]); image i gives width x height points in row-major pixel order, invalid pixels as NaN points.  The buffer
+        belongs to the context (valid until the next ingest call)."""
+        data, off, recs, n = self._depth_batch(images, intrinsics, poses, depth_scale)
+        d = C.c_void_p()
+        po = (C.c_size_t * (n + 1))()
+        self._check(self.L.haf_depth_to_xyz_batch(self.h, _ptr(data), off, n, recs, C.byref(d), po))
+        return (d.value or 0), np.array(po[:], np.int64)
+
+    def depth_to_xyz_batch_to_host(self, images, intrinsics=None, poses=None, depth_scale=0.0):
+        """back-project on the device, then copy back: a list of float32 [width * height, 3] arrays"""
+        _, po = self.depth_to_xyz_batch(images, intrinsics, poses, depth_scale)
+        xyz = self.debug_pcd_xyz(int(po[-1]))
+        return [xyz[po[i]:po[i + 1]] for i in range(len(po) - 1)]
+
+    def search_batch_depth(self, images, intrinsics=None, poses=None, depth_scale=0.0, requests=None, request_offsets=None, grasps=True,
+                           per_roll=False, per_roll_top=False):
+        """haf_search_batch_depth: back-project every image on the device, then ``search_batch_requests`` on the clouds.
+        requests=None: ``make_request()`` for every image.  Returns the dict of ``search_batch_pcd``."""
+        data, off, recs, n = self._depth_batch(images, intrinsics, poses, depth_scale)
+        if requests is None:
+            requests = make_requests(n)
+        elif not isinstance(requests, C.Array):
+            requests = (haf_request * len(requests))(*requests)
+        nreq = len(requests)
+        roff = None if request_offsets is None else (C.c_int * len(request_offsets))(*[int(o) for o in request_offsets])
+        best, bpr = (haf_best * n)(), (haf_best * nreq)()
+        grasp = (haf_grasp * n)() if grasps else None
+        gpr = (haf_grasp * nreq)() if grasps else None
+        groll = (haf_grasp * (nreq * self.R))() if grasps and per_roll else None
+        top = np.full((nreq, self.R, 3), -1, np.int32) if per_roll_top else None
+        self._check(self.L.haf_search_batch_depth(self.h, _ptr(data), off, n, recs, requests, roff, best, bpr, _ptr(top), grasp, gpr, groll))
+        out = {"best": best, "best_per_request": bpr}
+        if grasps:
+            out["grasp"], out["grasp_per_request"] = grasp, gpr
+        if groll is not None:
+            out["grasp_per_roll"] = groll
+        if top is not None:
+            out["per_roll_top"] = top
+        out["point_offsets"] = np.cumsum([0] + [recs[i].width * recs[i].height for i in range(n)]).astype(np.int64)
+        return out
 
     def debug_windows(self):
         W = self._check(self.L.haf_debug_window_count(self.h))

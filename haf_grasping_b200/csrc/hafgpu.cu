@@ -2825,6 +2825,102 @@ extern "C" int haf_search_batch_pcd(haf_ctx* ctx, const void* files, const size_
                                      per_roll_top, grasp_per_cloud, grasp_per_request, grasp_per_roll);
 }
 
+// Depth images -> packed xyz in ctx->d_pcd_xyz (hafpcdk::depth_project_kernel; the contract is in hafgpu.h).  Every image is
+// checked on the host first; then one upload (host input), one parameter block and one launch over every non-empty image, no sync.
+extern "C" int haf_depth_to_xyz_batch(haf_ctx* ctx, const void* data, const size_t* byte_offsets, int n_images, const haf_depth_image* images,
+                                      const float** d_xyz, size_t* point_offsets) {
+    if (!ctx) return HAF_ERR_ARG;
+    if (!d_xyz || !byte_offsets || n_images < 1 || !images || !point_offsets) return ctx->fail(HAF_ERR_ARG, "haf_depth_to_xyz_batch: bad arguments");
+    std::vector<size_t> pts(n_images + 1, 0);
+    std::vector<hafpcdk::DepthImage> imgs;
+    std::vector<unsigned> tile_begin(1, 0);
+    std::vector<size_t> cuts;
+    const size_t base = byte_offsets[0];
+    for (int i = 0; i < n_images; i++) {
+        const haf_depth_image& I = images[i];
+        auto bad = [&](const char* what) { return ctx->fail(HAF_ERR_ARG, "depth image %d: %s", i, what); };
+        if (I.width < 0 || I.width >= (1 << 24) || I.height < 0 || I.height >= (1 << 24)) return bad("width and height must lie in [0, 2^24)");
+        if (I.encoding != HAF_DEPTH_U16 && I.encoding != HAF_DEPTH_F32) return bad("unknown encoding");
+        const long long esz = I.encoding == HAF_DEPTH_U16 ? 2 : 4;
+        if (I.step < (long long)I.width * esz || I.step % esz) return bad("step must be a multiple of the element size and at least width x element size");
+        const unsigned long long span = byte_offsets[i + 1] - byte_offsets[i];
+        if (byte_offsets[i + 1] < byte_offsets[i] || (I.height && (unsigned long long)I.step > span / (unsigned long long)I.height) ||
+            (unsigned long long)I.height * (unsigned long long)I.step != span)
+            return bad("the byte span must be height x step");
+        if (!std::isfinite(I.fx) || !std::isfinite(I.fy) || !std::isfinite(I.cx) || !std::isfinite(I.cy) || I.fx == 0.0 || I.fy == 0.0)
+            return bad("fx, fy, cx, cy must be finite and fx, fy nonzero");
+        if (!(I.depth_scale >= 0.0f && I.depth_scale <= 1.0f)) return bad("depth_scale must lie in [0, 1]");
+        if (I.has_pose != 0 && I.has_pose != 1) return bad("has_pose must be 0 or 1");
+        if (I.has_pose)
+            for (int k = 0; k < 16; k++)
+                if (!std::isfinite(I.camera_to_base[k])) return bad("camera_to_base has a non-finite entry");
+        if (I.reserved[0] || I.reserved[1] || I.reserved[2]) return bad("reserved fields must be 0");
+        const unsigned long long npix = (unsigned long long)I.width * (unsigned long long)I.height;
+        pts[i + 1] = pts[i] + npix;
+        cuts.push_back(byte_offsets[i + 1] - base);
+        if (npix == 0) continue;
+        const unsigned long long tiles = (npix + HAF_DEPTH_TILE - 1) / HAF_DEPTH_TILE;
+        if (tile_begin.back() + tiles > 0x7fffffffull) return bad("the batch has more than 2^31 tiles of pixels");
+        hafpcdk::DepthImage d;
+        memset(&d, 0, sizeof d);
+        d.src = reinterpret_cast<const unsigned char*>(byte_offsets[i] - base);   // offset until the source is known
+        d.step = (unsigned long long)I.step;
+        d.n_pixels = npix;
+        d.out_begin = pts[i];
+        d.width = I.width;
+        d.encoding = I.encoding;
+        d.has_pose = I.has_pose;
+        const float s = I.depth_scale != 0.0f ? I.depth_scale : (I.encoding == HAF_DEPTH_U16 ? 0.001f : 1.0f);
+        d.s = s;
+        d.kx = (float)((double)s / I.fx);
+        d.ky = (float)((double)s / I.fy);
+        d.cxf = (float)I.cx;
+        d.cyf = (float)I.cy;
+        for (int k = 0; k < 12; k++) d.m[k] = I.camera_to_base[k];
+        imgs.push_back(d);
+        tile_begin.push_back((unsigned)(tile_begin.back() + tiles));
+    }
+    const size_t bytes = byte_offsets[n_images] - base, total = pts[n_images];
+    if (total > 0) {
+        if (!data) return ctx->fail(HAF_ERR_ARG, "haf_depth_to_xyz_batch: data is null");
+        CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+        const unsigned char* src = reinterpret_cast<const unsigned char*>(data) + base;
+        if (!is_device_ptr(data)) {
+            ENSURE(ctx, ctx->d_pcd_raw, bytes + 16);
+            const int rc = upload_host_bytes(ctx, ctx->d_pcd_raw.p, src, bytes, cuts);
+            if (rc) return rc;
+            src = ctx->d_pcd_raw.p;
+        }
+        ENSURE(ctx, ctx->d_pcd_xyz, total * 3);
+        for (size_t k = 0; k < imgs.size(); k++) imgs[k].src = src + reinterpret_cast<size_t>(imgs[k].src);
+        IngestParams P(ctx);
+        const size_t o_imgs = P.add(imgs.size() * sizeof(hafpcdk::DepthImage)), o_tiles = P.add(tile_begin.size() * sizeof(unsigned));
+        { const int rc = P.open(); if (rc) return rc; }
+        memcpy(P.h<hafpcdk::DepthImage>(o_imgs), imgs.data(), imgs.size() * sizeof(hafpcdk::DepthImage));
+        memcpy(P.h<unsigned>(o_tiles), tile_begin.data(), tile_begin.size() * sizeof(unsigned));
+        { const int rc = P.send(); if (rc) return rc; }
+        hafpcdk::depth_project_kernel<<<tile_begin.back(), HAF_DEPTH_THREADS, 0, ctx->stream>>>(P.d<hafpcdk::DepthImage>(o_imgs), P.d<unsigned>(o_tiles),
+                                                                                              (int)imgs.size(), ctx->d_pcd_xyz.p);
+        LAUNCHED(ctx);
+    }
+    for (int i = 0; i <= n_images; i++) point_offsets[i] = pts[i];
+    *d_xyz = total ? ctx->d_pcd_xyz.p : nullptr;
+    return HAF_OK;
+}
+
+extern "C" int haf_search_batch_depth(haf_ctx* ctx, const void* data, const size_t* byte_offsets, int n_images, const haf_depth_image* images,
+                                      const haf_request* reqs, const int* request_offsets, haf_best* best_per_cloud, haf_best* best_per_request,
+                                      int* per_roll_top, haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll) {
+    if (!ctx) return HAF_ERR_ARG;
+    if (n_images < 1) return ctx->fail(HAF_ERR_ARG, "haf_search_batch_depth: bad arguments");
+    std::vector<size_t> point_offsets(n_images + 1);
+    const float* d_xyz = nullptr;
+    const int rc = haf_depth_to_xyz_batch(ctx, data, byte_offsets, n_images, images, &d_xyz, point_offsets.data());
+    if (rc != HAF_OK) return rc;
+    return haf_search_batch_requests(ctx, d_xyz, point_offsets.data(), n_images, reqs, request_offsets, best_per_cloud, best_per_request,
+                                     per_roll_top, grasp_per_cloud, grasp_per_request, grasp_per_roll);
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // several GPUs behind one context (haf_config.n_devices > 1, SURVEY 8b / 8e)
 // ------------------------------------------------------------------------------------------------------------

@@ -118,6 +118,13 @@ public:
         return batch_control(goal, NULL, NULL, xyz_all, point_offsets, n_clouds);
     }
 
+    // depth images back to back in host memory (image i = bytes [byte_offsets[i], byte_offsets[i+1]), described by images[i]),
+    // back-projected and moved into the base frame on the device in one call (haf_search_batch_depth)
+    std::vector<CloudResult> depth_images_cb(const GraspInput& goal, const void* data, const size_t* byte_offsets, int n_images,
+                                             const haf_depth_image* images) {
+        return batch_control(goal, data, byte_offsets, NULL, NULL, n_images, images);
+    }
+
     // goal -> members (:258-326)
     void set_goal(const GraspInput& goal) {
         graspsearchcenter = goal.grasp_area_center;                              // :258-260
@@ -167,13 +174,15 @@ public:
 
     // the goal's request on every file of a batch, decoded on the device (haf_pcd_decode_batch), then the ranked candidates of every
     // cloud (haf_search_batch_candidates): cand [n][rp.k], ncand [n]
+    // (images: depth images back to back, as in depth_images_cb, back-projected by haf_depth_to_xyz_batch)
     void rank_pcds_cb(const GraspInput& goal, const void* files, const size_t* file_offsets, int n, const haf_rank_params& rp,
-                      std::vector<haf_candidate>& cand, std::vector<int>& ncand) {
+                      std::vector<haf_candidate>& cand, std::vector<int>& ncand, const haf_depth_image* images = NULL) {
         set_goal(goal);
         const std::vector<haf_request> reqs(n, request(0));
         std::vector<size_t> point_offsets(n + 1);
         const float* d_xyz = NULL;
-        int rc = haf_pcd_decode_batch(ctx_, files, file_offsets, n, &d_xyz, point_offsets.data());
+        int rc = images ? haf_depth_to_xyz_batch(ctx_, files, file_offsets, n, images, &d_xyz, point_offsets.data())
+                        : haf_pcd_decode_batch(ctx_, files, file_offsets, n, &d_xyz, point_offsets.data());
         std::vector<haf_best> best_c(n);
         std::vector<haf_grasp> grasp_c(n);
         cand.assign((size_t)n * rp.k, haf_candidate());
@@ -207,21 +216,26 @@ private:
             if (!return_only_best_gp && top[roll * 3 + 2] > graspval_th) out.push_back(to_grasp_output(grasp_per_roll[roll]));
         return out;
     }
-    // one haf_search_batch_pcd (files) or haf_search_batch_requests (xyz_all) call with the goal's request for every cloud
+    // one haf_search_batch_pcd (files), haf_search_batch_depth (files with images) or haf_search_batch_requests (xyz_all) call with
+    // the goal's request for every cloud
     std::vector<CloudResult> batch_control(const GraspInput& goal, const void* files, const size_t* file_offsets, const float* xyz_all,
-                                           const size_t* point_offsets, int n) {
+                                           const size_t* point_offsets, int n, const haf_depth_image* images = NULL) {
         set_goal(goal);
         const std::vector<haf_request> reqs(n, request(0));
         std::vector<haf_best> best_c(n);
         std::vector<int> top((size_t)n * R * 3, -1);
         std::vector<haf_grasp> grasp_c(n), grasp_r((size_t)n * R);
-        const int rc = files ? haf_search_batch_pcd(ctx_, files, file_offsets, n, reqs.data(), NULL, best_c.data(), NULL, top.data(), grasp_c.data(),
+        const int rc = images ? haf_search_batch_depth(ctx_, files, file_offsets, n, images, reqs.data(), NULL, best_c.data(), NULL, top.data(),
+                                                       grasp_c.data(), NULL, grasp_r.data())
+                     : files ? haf_search_batch_pcd(ctx_, files, file_offsets, n, reqs.data(), NULL, best_c.data(), NULL, top.data(), grasp_c.data(),
                                                     NULL, grasp_r.data())
                              : haf_search_batch_requests(ctx_, xyz_all, point_offsets, n, reqs.data(), NULL, best_c.data(), NULL, top.data(),
                                                          grasp_c.data(), NULL, grasp_r.data());
         if (rc != HAF_OK) throw std::runtime_error(std::string("hafgpu: ") + haf_last_error(ctx_));
         std::vector<size_t> pts(n + 1, 0);
-        if (files) {   // the clouds' sizes: the headers' POINTS (the call above has parsed every header)
+        if (images) {  // an image's cloud has width x height points
+            for (int c = 0; c < n; c++) pts[c + 1] = pts[c] + (size_t)images[c].width * (size_t)images[c].height;
+        } else if (files) {   // the clouds' sizes: the headers' POINTS (the call above has parsed every header)
             for (int c = 0; c < n; c++) {
                 hafpcd::PcdHeader hd;
                 hafpcd::parse_pcd_header(static_cast<const unsigned char*>(files) + file_offsets[c], file_offsets[c + 1] - file_offsets[c], hd, NULL);

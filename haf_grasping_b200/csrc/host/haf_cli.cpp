@@ -7,7 +7,11 @@
 // file alone prints.
 // --top K [--min-distance m] [--per-unit P]: after each file's line, the file's K best distinct grasps (haf_search_batch_candidates
 // on the files decoded by haf_pcd_decode_batch): one line per candidate, or with --json one object {"candidates": [...]}.
+// --depth img.pgm (repeatable) --camera fx fy cx cy [--camera-pose m00 .. m33] [--depth-scale s]: 16-bit binary PGM depth images
+// (P5, big-endian samples, swapped here) back-projected and moved into the base frame on the device, all in ONE batch call
+// (haf_search_batch_depth), one output line per image in the --pcd format; --top works as with --pcd.
 //   haf_cli --pcd cloud.pcd --dump-pcd          (parse only, no GPU)
+#include <cctype>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -24,6 +28,38 @@ static bool read_file(const std::string& path, std::vector<unsigned char>& out) 
     size_t nr;
     while ((nr = fread(buf, 1, sizeof buf, fp)) > 0) out.insert(out.end(), buf, buf + nr);
     fclose(fp);
+    return true;
+}
+
+// 16-bit binary PGM (P5, maxval 256..65535) -> little-endian u16 rows appended to out
+static bool read_pgm16(const std::string& path, std::vector<unsigned char>& out, int* w, int* h, std::string* err) {
+    std::vector<unsigned char> b;
+    if (!read_file(path, b)) { *err = "cannot open " + path; return false; }
+    size_t p = 0;
+    long vals[3];
+    auto token = [&](long* v) {
+        for (;;) {
+            while (p < b.size() && isspace(b[p])) p++;
+            if (p < b.size() && b[p] == '#') { while (p < b.size() && b[p] != '\n') p++; continue; }
+            break;
+        }
+        if (p >= b.size() || !isdigit(b[p])) return false;
+        *v = 0;
+        while (p < b.size() && isdigit(b[p]) && *v < 100000000) *v = *v * 10 + (b[p++] - '0');
+        return true;
+    };
+    if (b.size() < 2 || b[0] != 'P' || b[1] != '5') { *err = path + ": not a binary PGM (P5)"; return false; }
+    p = 2;
+    for (int k = 0; k < 3; k++)
+        if (!token(&vals[k])) { *err = path + ": bad PGM header"; return false; }
+    if (vals[2] < 256 || vals[2] > 65535) { *err = path + ": not a 16-bit PGM"; return false; }
+    if (p >= b.size() || !isspace(b[p])) { *err = path + ": bad PGM header"; return false; }
+    p++;
+    const size_t n = (size_t)vals[0] * (size_t)vals[1];
+    if (b.size() - p < 2 * n) { *err = path + ": PGM data truncated"; return false; }
+    for (size_t i = 0; i < n; i++) { out.push_back(b[p + 2 * i + 1]); out.push_back(b[p + 2 * i]); }
+    *w = (int)vals[0];
+    *h = (int)vals[1];
     return true;
 }
 
@@ -73,7 +109,11 @@ static void print_result(bool json, size_t n_points, const haf_best& best, const
 
 int main(int argc, char** argv) {
     std::string features, range, model, pcd;
-    std::vector<std::string> pcds;
+    std::vector<std::string> pcds, depths;
+    haf_depth_image cam;
+    memset(&cam, 0, sizeof cam);
+    cam.encoding = HAF_DEPTH_U16;
+    bool have_camera = false;
     haf_b200::GraspInput goal;
     int grid = 56, svm_mode = HAF_SVM_TENSOR_GUARD;
     bool json = false, dump_pcd = false, host_pcd = false;
@@ -86,6 +126,10 @@ int main(int argc, char** argv) {
         else if (a == "--range") { need(1); range = argv[++i]; }
         else if (a == "--model") { need(1); model = argv[++i]; }
         else if (a == "--pcd") { need(1); pcd = argv[++i]; pcds.push_back(pcd); }
+        else if (a == "--depth") { need(1); depths.push_back(argv[++i]); }
+        else if (a == "--camera") { need(4); cam.fx = atof(argv[++i]); cam.fy = atof(argv[++i]); cam.cx = atof(argv[++i]); cam.cy = atof(argv[++i]); have_camera = true; }
+        else if (a == "--camera-pose") { need(16); cam.has_pose = 1; for (int k = 0; k < 16; k++) cam.camera_to_base[k] = (float)atof(argv[++i]); }
+        else if (a == "--depth-scale") { need(1); cam.depth_scale = (float)atof(argv[++i]); }
         else if (a == "--center") { need(3); goal.grasp_area_center.x = atof(argv[++i]); goal.grasp_area_center.y = atof(argv[++i]); goal.grasp_area_center.z = atof(argv[++i]); }
         else if (a == "--area") { need(2); goal.grasp_area_length_x = (float)atof(argv[++i]); goal.grasp_area_length_y = (float)atof(argv[++i]); }
         else if (a == "--approach") { need(3); goal.approach_vector.x = atof(argv[++i]); goal.approach_vector.y = atof(argv[++i]); goal.approach_vector.z = atof(argv[++i]); }
@@ -109,6 +153,39 @@ int main(int argc, char** argv) {
         const unsigned char* b = reinterpret_cast<const unsigned char*>(pts.data());
         for (size_t k = 0; k < pts.size() * 4; k++) { h ^= b[k]; h *= 1099511628211ull; }
         printf("%zu %llu\n", pts.size() / 3, h);
+        return 0;
+    }
+    if (!depths.empty()) {   // depth images: one batch call for all of them
+        if (features.empty() || range.empty() || model.empty() || !have_camera || !pcds.empty()) {
+            fprintf(stderr, "usage: haf_cli --features F --range R --model M --depth img.pgm [--depth img.pgm ...] --camera fx fy cx cy [--camera-pose m00 .. m33] [--depth-scale s] [goal options]\n");
+            return 2;
+        }
+        std::vector<unsigned char> data;
+        std::vector<size_t> offsets(1, 0);
+        std::vector<haf_depth_image> images;
+        for (size_t f = 0; f < depths.size(); f++) {
+            haf_depth_image im = cam;
+            std::string err;
+            if (!read_pgm16(depths[f], data, &im.width, &im.height, &err)) { fprintf(stderr, "haf_cli: %s\n", err.c_str()); return 1; }
+            im.step = 2LL * im.width;
+            images.push_back(im);
+            offsets.push_back(data.size());
+        }
+        try {
+            haf_b200::CCalc_Grasppoints_B200 server(features, range, model, 302, grid, 15, 190, 0, svm_mode);
+            const int n = (int)depths.size();
+            const std::vector<haf_b200::CCalc_Grasppoints_B200::CloudResult> res = server.depth_images_cb(goal, data.data(), offsets.data(), n, images.data());
+            std::vector<haf_candidate> cand;
+            std::vector<int> ncand;
+            if (rank.k != 0) server.rank_pcds_cb(goal, data.data(), offsets.data(), n, rank, cand, ncand, images.data());
+            for (int f = 0; f < n; f++) {
+                print_result(json, res[f].n_points, res[f].best, res[f].gp_result, res[f].per_roll_top.data(), server.R, res[f].published_per_roll.size());
+                if (rank.k != 0) print_candidates(json, cand.data() + (size_t)f * rank.k, ncand[f]);
+            }
+        } catch (const std::exception& e) {
+            fprintf(stderr, "haf_cli: %s\n", e.what());
+            return 1;
+        }
         return 0;
     }
     if (features.empty() || range.empty() || model.empty() || pcd.empty()) {

@@ -267,4 +267,92 @@ __global__ void __launch_bounds__(HAF_PCD_TILE_THREADS) ascii_parse_kernel(const
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Depth images (haf_depth_to_xyz_batch; the arithmetic is the contract in hafgpu.h, restated from depth_image_proc's convert()
+// and PCL 1.7's transformPointCloud of a non-dense cloud).  Every non-empty image of a call is cut into tiles of
+// HAF_DEPTH_TILE pixels in row-major order; tile_begin [n_images + 1] is the exclusive prefix of the images' tile counts and a
+// CTA finds its image by binary search.  Rows are only element-aligned, so each pixel is one 2- or 4-byte load.  A CTA stages
+// its 12-byte points in shared memory and stores them with 16-byte stores, scalar stores for the unaligned head and tail.
+// ---------------------------------------------------------------------------------------------------------------------
+#define HAF_DEPTH_THREADS 256
+#define HAF_DEPTH_PIX_PER_THREAD 4
+#define HAF_DEPTH_TILE (HAF_DEPTH_THREADS * HAF_DEPTH_PIX_PER_THREAD)
+struct DepthImage {
+    const unsigned char* src;            // first row
+    unsigned long long step;             // bytes per row
+    unsigned long long n_pixels;         // width * height
+    unsigned long long out_begin;        // first output point
+    int width, encoding, has_pose, pad;  // encoding: HAF_DEPTH_U16 / HAF_DEPTH_F32
+    float kx, ky, cxf, cyf, s;
+    float m[12];                         // rows 0..2 of camera_to_base
+};
+__device__ __forceinline__ bool depth_fin(float x) { return fabsf(x) <= 3.402823466e38f; }   // false for +-inf and NaN
+__global__ void __launch_bounds__(HAF_DEPTH_THREADS) depth_project_kernel(const DepthImage* __restrict__ imgs, const unsigned* __restrict__ tile_begin,
+                                                                          int n_imgs, float* __restrict__ xyz) {
+    __shared__ float s_out[3 * HAF_DEPTH_TILE];
+    int lo = 0, hi = n_imgs - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (tile_begin[mid] <= blockIdx.x) lo = mid; else hi = mid - 1;
+    }
+    const DepthImage& I = imgs[lo];
+    const unsigned long long p0 = (unsigned long long)(blockIdx.x - tile_begin[lo]) * HAF_DEPTH_TILE;
+    const unsigned n = (unsigned)min((unsigned long long)HAF_DEPTH_TILE, I.n_pixels - p0);
+    const unsigned w = (unsigned)I.width;
+    const unsigned long long v0 = p0 / w;
+    const unsigned u0 = (unsigned)(p0 - v0 * w);
+    const bool f32 = I.encoding == 2;                    // HAF_DEPTH_F32
+    const float kx = I.kx, ky = I.ky, cxf = I.cxf, cyf = I.cyf, s = I.s;
+#pragma unroll
+    for (int k = 0; k < HAF_DEPTH_PIX_PER_THREAD; k++) {
+        const unsigned j = threadIdx.x + k * HAF_DEPTH_THREADS;
+        if (j >= n) break;
+        const unsigned uu = u0 + j;                      // < 2^24 + 2^10
+        const unsigned u = uu % w;
+        const unsigned long long v = v0 + uu / w;
+        const unsigned char* p = I.src + v * I.step + (unsigned long long)u * (f32 ? 4u : 2u);
+        float D;
+        bool valid;
+        if (f32) {
+            D = load_f32_any(p);
+            valid = depth_fin(D);
+        } else {
+            const unsigned d = (reinterpret_cast<uintptr_t>(p) & 1) ? ((unsigned)p[0] | ((unsigned)p[1] << 8))
+                                                                     : (unsigned)*reinterpret_cast<const unsigned short*>(p);
+            D = (float)d;
+            valid = d != 0;
+        }
+        float x, y, z;
+        if (valid) {
+            x = __fmul_rn(__fmul_rn(__fsub_rn((float)u, cxf), D), kx);
+            y = __fmul_rn(__fmul_rn(__fsub_rn((float)v, cyf), D), ky);
+            z = __fmul_rn(D, s);
+            if (I.has_pose && depth_fin(x) && depth_fin(y) && depth_fin(z)) {
+                const float* m = I.m;
+                const float X = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[0], x), __fmul_rn(m[1], y)), __fmul_rn(m[2], z)), m[3]);
+                const float Y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[4], x), __fmul_rn(m[5], y)), __fmul_rn(m[6], z)), m[7]);
+                const float Z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[8], x), __fmul_rn(m[9], y)), __fmul_rn(m[10], z)), m[11]);
+                x = X; y = Y; z = Z;
+            }
+        } else {
+            x = y = z = __uint_as_float(0x7fc00000u);
+        }
+        s_out[3 * j] = x; s_out[3 * j + 1] = y; s_out[3 * j + 2] = z;
+    }
+    __syncthreads();
+    // floats [g0, g0 + 3n) of the output: scalar head up to a 16-byte boundary, float4 body, scalar tail
+    const unsigned long long g0 = 3 * (I.out_begin + p0);
+    const unsigned nf = 3 * n;
+    const unsigned head = min((unsigned)((4 - (g0 & 3)) & 3), nf);
+    const unsigned nb = (nf - head) >> 2;
+    if (threadIdx.x < head) xyz[g0 + threadIdx.x] = s_out[threadIdx.x];
+    float4* body = reinterpret_cast<float4*>(xyz + g0 + head);
+    for (unsigned q = threadIdx.x; q < nb; q += HAF_DEPTH_THREADS) {
+        const float* a = s_out + head + 4 * q;
+        body[q] = make_float4(a[0], a[1], a[2], a[3]);
+    }
+    const unsigned t0 = head + 4 * nb;
+    if (t0 + threadIdx.x < nf) xyz[g0 + t0 + threadIdx.x] = s_out[t0 + threadIdx.x];
+}
+
 }  // namespace hafpcdk

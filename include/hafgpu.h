@@ -318,6 +318,48 @@ int haf_search_batch_pcd(haf_ctx* ctx, const void* files, const size_t* file_off
 int haf_pointcloud2_batch_to_xyz(haf_ctx* ctx, const void* data_hostdev, const size_t* byte_offsets, int n_clouds,
                                  const int* layouts, const float** d_xyz, size_t* point_offsets);
 
+/* ---- batches of depth images: back-projection (and the camera -> base transform) on the device -----------------------
+ * What a camera-fed server otherwise does on the CPU before a search: depth_image_proc's point_cloud_xyz (convert() of
+ * depth_conversions.h for 16UC1 and 32FC1, range_max = 0, no lens distortion), then pcl_ros::transformPointCloud into the base
+ * frame (server.cpp:316).  Image i = height rows of step bytes, little-endian, bytes [byte_offsets[i], byte_offsets[i+1]) of
+ * data (host, pinned or pageable, or device); its cloud is the organized cloud of width x height points in row-major pixel
+ * order, invalid pixels kept as NaN points.
+ * Per image, on the host in double, stored as float: s = depth_scale (0: 0.001f for U16, 1.0f for F32), kx = s / fx,
+ * ky = s / fy, cxf = cx, cyf = cy.  Pixel (u, v) with raw value d is valid when d != 0 (U16) or isfinite(d) (F32, negative
+ * depths included); then D = (float)d and, one float rounding per operation, left to right, no FMA:
+ *     x = ((float)u - cxf) * D * kx,   y = ((float)v - cyf) * D * ky,   z = D * s.
+ * An invalid pixel is x = y = z = quiet NaN 0x7fc00000.  has_pose = 1: a point whose three coordinates are finite becomes
+ * x' = ((m00 x + m01 y) + m02 z) + m03 (and so on per row; float, left to right, no FMA), any other point stays as it is (PCL
+ * 1.7's transformPointCloud of a non-dense cloud).  has_pose = 0: no arithmetic at all (an identity pose would turn -0 into +0).
+ * With depth_scale <= 1 every valid pixel has a finite z, so a point with a non-finite coordinate has a non-finite x or y and
+ * fails the search's box test whatever its pose.
+ * HAF_ERR_ARG "depth image <i>: ..." names the lowest bad image, checked on the host before any device work (nothing is
+ * written): width or height outside [0, 2^24), unknown encoding, step not a multiple of the element size or below width x
+ * element size, byte span != height x step, non-finite fx / fy / cx / cy or fx / fy = 0, depth_scale outside [0, 1] or NaN,
+ * has_pose not 0 / 1, a non-finite camera_to_base entry with has_pose = 1, nonzero reserved. */
+#define HAF_DEPTH_U16 1        /* 16UC1 / mono16; 0 = no return */
+#define HAF_DEPTH_F32 2        /* 32FC1 metres; non-finite = no return */
+typedef struct {
+    int width, height, encoding, has_pose;
+    long long step;            /* sensor_msgs/Image.step */
+    double fx, fy, cx, cy;     /* CameraInfo K[0], K[4], K[2], K[5] */
+    float depth_scale;         /* metres per unit, 0 = per-encoding default, <= 1 */
+    float camera_to_base[16];  /* row-major, what pcl_ros::transformAsMatrix gives */
+    int reserved[3];           /* must be 0 */
+} haf_depth_image;             /* 136 bytes */
+/* n_images images -> packed xyz of every cloud in ctx's ingest buffer: *d_xyz and point_offsets [n_images+1] (out) as in
+ * haf_pcd_decode_batch (valid until the next ingest call; accepted by every search entry point as xyz_hostdev).  One kernel
+ * launch covers every non-empty image (none when all are empty); no stream sync.  Device input is read in place, pinned input
+ * is copied with one cudaMemcpyAsync, pageable input of 4 MB and more goes through the staging thread in pieces cut on image
+ * boundaries.  Multi-GPU context: runs on its first GPU. */
+int haf_depth_to_xyz_batch(haf_ctx* ctx, const void* data_hostdev, const size_t* byte_offsets, int n_images,
+                           const haf_depth_image* images, const float** d_xyz, size_t* point_offsets);
+/* haf_depth_to_xyz_batch + haf_search_batch_requests on the clouds, on the same stream; arguments and outputs as there */
+int haf_search_batch_depth(haf_ctx* ctx, const void* data_hostdev, const size_t* byte_offsets, int n_images,
+                           const haf_depth_image* images, const haf_request* reqs, const int* request_offsets,
+                           haf_best* best_per_cloud, haf_best* best_per_request, int* per_roll_top,
+                           haf_grasp* grasp_per_cloud, haf_grasp* grasp_per_request, haf_grasp* grasp_per_roll);
+
 /* ---- libsvm-compatible front ends (SURVEY 8f-3) ----------------------------------------------------------------
  * The reference classifies by running two child processes per roll on text files (server.cpp:775-776, :786-792):
  *     svm-scale -r <range> /tmp/features.txt > /tmp/features.txt.scale      (libsvm-3.12/svm-scale.c)
@@ -411,7 +453,7 @@ int haf_debug_cell_indices(haf_ctx* ctx, const float* xyz_hostdev, size_t n_poin
 int haf_debug_text_roundtrip(haf_ctx* ctx, const float* in4, int n4, double* out4, const double* in6, int n6,
                              double* out6);
 
-/* packed xyz of the last ingest call (haf_pcd_decode[_batch], haf_pointcloud2[_batch]_to_xyz; all clouds of a batch: total
+/* packed xyz of the last ingest call (haf_pcd_decode[_batch], haf_pointcloud2[_batch]_to_xyz, haf_depth_to_xyz_batch; all clouds of a batch: total
  * points), copied to host memory (n_points records) */
 int haf_debug_pcd_xyz(haf_ctx* ctx, float* xyz_host, size_t n_points);
 
