@@ -35,6 +35,26 @@ inline bool lzf_decompress(const unsigned char* ip, size_t in_len, unsigned char
     return o == out_len;
 }
 
+// The tokens of one line of an ASCII DATA section: fields are separated by runs of blank, tab and CR only (PCL's boost::split
+// on "\t\r "); vertical tab and form feed are token characters, as on the device (csrc/pcd_ingest.cuh, is_blank).
+inline void ascii_tokens(const std::string& line, std::vector<std::string>& toks) {
+    size_t p = 0;
+    const size_t n = line.size();
+    while (p < n) {
+        while (p < n && (line[p] == ' ' || line[p] == '\t' || line[p] == '\r')) p++;
+        size_t e = p;
+        while (e < n && line[e] != ' ' && line[e] != '\t' && line[e] != '\r') e++;
+        if (e > p) toks.push_back(line.substr(p, e - p));
+        p = e;
+    }
+}
+// A FLOAT32 token: strtof of its longest numeric prefix.  strtof would skip a leading vertical tab or form feed; those are
+// token characters here, so such a token has no numeric prefix and reads 0, as on the device.
+inline float ascii_token_value(const std::string& tok) {
+    if (!tok.empty() && (tok[0] == '\v' || tok[0] == '\f')) return 0.0f;
+    return strtof(tok.c_str(), NULL);
+}
+
 // The text header of a PCD v0.7 file, up to and including its DATA line (what pcl::PCDReader::readHeader takes from it for
 // an xyz cloud).  Also used by the device ingest (csrc/pcd_ingest.cuh, haf_pcd_decode): the header stays host-side text.
 struct PcdHeader {
@@ -104,13 +124,11 @@ inline bool read_pcd(const std::string& path, std::vector<float>& xyz, std::stri
             std::string line((const char*)&raw[pos], nl - pos);
             pos = nl + 1;
             std::vector<std::string> toks;
-            std::istringstream ss(line);
-            std::string tok;
-            while (ss >> tok) toks.push_back(tok);
+            ascii_tokens(line, toks);
             if (toks.empty()) continue;
             for (int a = 0; a < 3; a++) {
                 if (tokoff[idx[a]] >= (int)toks.size()) { if (err) *err = "short ASCII record in " + path; return false; }
-                xyz[rec * 3 + a] = strtof(toks[tokoff[idx[a]]].c_str(), NULL);
+                xyz[rec * 3 + a] = ascii_token_value(toks[tokoff[idx[a]]]);
             }
             rec++;
         }

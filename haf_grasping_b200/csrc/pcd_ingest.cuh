@@ -5,7 +5,8 @@
 // and ships a PointCloud2; the server turns it back into points with pcl::fromROSMsg (src/calc_grasppoints_action_server.cpp
 // :313-316).  PCL is a dependency of the reference, not vendored in it (ROS hydro / indigo: PCL 1.7); what is restated here is
 // its published reader (io/src/pcd_io.cpp, PCDReader::read):
-//   * ascii             -- one record per non-empty line, fields split on blank / tab / CR, FLOAT32 fields through
+//   * ascii             -- one record per non-empty line, fields split on blank / tab / CR only (vertical tab and form feed
+//                          are token characters here and in both host readers), FLOAT32 fields through
 //                          `istringstream >> float` (= strtof: correctly rounded, hafdec::parse_float_token); exactly POINTS
 //                          records are taken, further lines are ignored (pcd4 / pcd5 carry 208 lines for POINTS 200);
 //   * binary            -- POINTS records of the header's layout;

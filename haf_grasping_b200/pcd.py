@@ -25,8 +25,22 @@ def _strtof(tok: bytes) -> float:
     return _libc.strtof(tok, None)
 
 
+def ascii_tokens(line: bytes) -> list:
+    """the tokens of one line of an ASCII DATA section: fields are separated by runs of blank, tab and CR only (PCL's
+    boost::split on "\\t\\r "); vertical tab and form feed are token characters, as on the device (csrc/pcd_ingest.cuh)"""
+    return [t for t in line.replace(b"\t", b" ").replace(b"\r", b" ").split(b" ") if t]
+
+
+def ascii_token_value(tok: bytes) -> float:
+    """a FLOAT32 token: strtof of its longest numeric prefix.  strtof would skip a leading vertical tab or form feed; those
+    are token characters here, so such a token has no numeric prefix and reads 0, as on the device."""
+    return 0.0 if tok[:1] in (b"\v", b"\f") else _strtof(tok)
+
+
 def lzf_decompress(src: bytes, out_len: int) -> bytes:
-    """liblzf stream decoder (the codec PCL embeds for DATA binary_compressed)."""
+    """liblzf stream decoder (the codec PCL embeds for DATA binary_compressed).  Rejects, with ValueError("corrupt LZF
+    stream ..."), exactly the streams the C++ reader (csrc/host/pcd_io.hpp) and the device kernel reject: a token cut off
+    by the end of the input, a reference before the start of the output, a token past out_len, a stream short of out_len."""
     out = bytearray(out_len)
     ip, op, n = 0, 0, len(src)
     while ip < n:
@@ -34,19 +48,25 @@ def lzf_decompress(src: bytes, out_len: int) -> bytes:
         ip += 1
         if ctrl < 32:  # literal run of ctrl+1 bytes
             ln = ctrl + 1
+            if op + ln > out_len or ip + ln > n:
+                raise ValueError("corrupt LZF stream: literal run past the end of the input or the output")
             out[op:op + ln] = src[ip:ip + ln]
             ip += ln
             op += ln
         else:  # back reference
             ln = ctrl >> 5
             if ln == 7:
+                if ip >= n:
+                    raise ValueError("corrupt LZF stream: no length byte")
                 ln += src[ip]
                 ip += 1
+            if ip >= n:
+                raise ValueError("corrupt LZF stream: no distance byte")
             ref = op - ((ctrl & 0x1F) << 8) - src[ip] - 1
             ip += 1
             ln += 2
             if ref < 0 or op + ln > out_len:
-                raise ValueError("corrupt LZF stream")
+                raise ValueError("corrupt LZF stream: reference before the start or past the end of the output")
             if ref + ln <= op:
                 out[op:op + ln] = out[ref:ref + ln]
             else:  # overlapping copy, byte by byte
@@ -54,7 +74,7 @@ def lzf_decompress(src: bytes, out_len: int) -> bytes:
                     out[op + k] = out[ref + k]
             op += ln
     if op != out_len:
-        raise ValueError(f"LZF stream decoded to {op} bytes, expected {out_len}")
+        raise ValueError(f"corrupt LZF stream: decoded to {op} bytes, expected {out_len}")
     return bytes(out)
 
 
@@ -120,12 +140,14 @@ def read_pcd_bytes(raw: bytes, path: str = "<bytes>") -> np.ndarray:
         for ln in raw[pos:].split(b"\n"):
             if idx >= npts:
                 break
-            toks = ln.split()
+            toks = ascii_tokens(ln)
             if not toks:
                 continue
+            if len(toks) <= max(cols):
+                raise ValueError(f"PCD {path}: short ASCII record")
             for k, c in enumerate(cols):
                 t = toks[c]
-                out[idx, k] = np.float32("nan") if t.lower() == b"nan" else _strtof(t)
+                out[idx, k] = np.float32("nan") if t.lower() == b"nan" else ascii_token_value(t)
             idx += 1
         if idx != npts:
             raise ValueError(f"PCD {path}: {idx} records, header says {npts}")
@@ -138,6 +160,8 @@ def read_pcd_bytes(raw: bytes, path: str = "<bytes>") -> np.ndarray:
         return np.stack([rec[ax][:, 0].astype(np.float32) for ax in "xyz"], axis=1)
     if data_kind == "binary_compressed":
         comp, uncomp = struct.unpack_from("<II", raw, pos)
+        if pos + 8 + comp > len(raw):
+            raise ValueError(f"PCD {path}: compressed PCD truncated")
         blob = lzf_decompress(raw[pos + 8:pos + 8 + comp], uncomp)
         out = np.empty((npts, 3), np.float32)
         off = 0
