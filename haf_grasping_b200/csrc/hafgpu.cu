@@ -412,10 +412,6 @@ static void calibrate_tensor_passes(const hafhost::Model& model, int Dsv, double
         rel[2] = std::max(rel[2], fabs(dec2 - dec) / E);
     }
 }
-// "%.4g" tables of the fast feature tier (kernels.cuh, Round4Tab): powers of ten 10^(i-48)
-static void make_round4_table(Round4Tab& tab) {
-    for (int i = 0; i < 96; i++) { tab.pwd[i] = pow(10.0, i - 48); tab.pwf[i] = (float)tab.pwd[i]; }
-}
 // Operand tensor in the k-block tiled layout (kernels.cuh, kt_off): seen by TMA as [n_tiles * 128 rows][64 fp16], pitch 128 B
 // = fully contiguous; one box = 64 x 128 = one 16 KB tile (row tile, k-block), 128B swizzle.  rows is a multiple of 128.
 static bool make_tensor_map(CUtensorMap* m, void* base, int KB, uint64_t rows) {
@@ -765,9 +761,11 @@ static int create_impl(haf_ctx** out, const haf_config* cfg, bool svm_only, int 
         CREATE_TRY(cudaFuncSetAttribute(haftc::svm_rbf_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, haftc::SMEM2_BYTES + haftc::TAB_SMEM_MAX * 4));
         CREATE_TRY(cudaFuncSetAttribute(haftc::svm_rbf_tc3_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, haftc::TC3_SMEM_LIMIT));
         CREATE_TRY(cudaFuncSetAttribute(haftc::svm_rbf_tc3_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, haftc::TC3_SMEM_LIMIT));
-        CREATE_TRY(cudaFuncSetAttribute(features_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ft_smem_layout(G, 2)));
+        CREATE_TRY(cudaFuncSetAttribute(features_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ft_smem_layout(G, 1)));
+        CREATE_TRY(cudaFuncSetAttribute(features_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ft_smem_layout(G, 2)));
         // 4 CTAs x ~49 KB: ask for just that much shared memory so that the rest of the SM's 256 KB stays L1 (the corner-offset table)
-        CREATE_TRY(cudaFuncSetAttribute(features_tc_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 90));
+        CREATE_TRY(cudaFuncSetAttribute(features_tc_kernel<false>, cudaFuncAttributePreferredSharedMemoryCarveout, 90));
+        CREATE_TRY(cudaFuncSetAttribute(features_tc_kernel<true>, cudaFuncAttributePreferredSharedMemoryCarveout, 90));
     }
     for (int i = 0; i < 10; i++) CREATE_TRY(cudaEventCreate(&ctx->ev[i]));
     ctx->ev_ok = true;
@@ -1778,9 +1776,10 @@ static int run_jobs_once(haf_ctx* ctx, const CloudSet& cs, std::vector<Job>& job
         const unsigned wblocks32 = (unsigned)((Wcap + 31) / 32);
         if (tc) {
             const unsigned fblocks = (unsigned)((Wcap + 32 * HAF_FT_WT - 1) / (32 * HAF_FT_WT));
-            features_tc_kernel<<<fblocks, 256, ft_smem_bytes(ctx), st>>>(ctx->d_integral.p, ctx->d_win.p, cnt + 0, G, ubase, ctx->d_dimfeat.p, ctx->D,
-                                                                      ctx->Krow, (float)ctx->lower, ctx->cfg.emulate_text_roundtrip, ctx->d_round4.p, ctx->d_Xh.p,
-                                                                      ctx->tc_passes >= 3 ? ctx->d_Xl.p : nullptr, ctx->d_xn.p, ctx->Dsv, ctx->KB, ctx->d_dec.p, ctx->d_asum.p);
+            (ctx->tc_passes >= 3 ? features_tc_kernel<true> : features_tc_kernel<false>)<<<fblocks, 256, ft_smem_bytes(ctx), st>>>(
+                ctx->d_integral.p, ctx->d_win.p, cnt + 0, G, ubase, ctx->d_dimfeat.p, ctx->D, ctx->Krow, (float)ctx->lower,
+                ctx->cfg.emulate_text_roundtrip, ctx->d_round4.p, ctx->d_Xh.p, ctx->tc_passes >= 3 ? ctx->d_Xl.p : nullptr, ctx->d_xn.p,
+                ctx->Dsv, ctx->KB, ctx->d_dec.p, ctx->d_asum.p);
             LAUNCHED(ctx);
         } else if (ctx->cfg.svm_mode != HAF_SVM_FP64_EXACT && !prob) {
             features_kernel<false><<<wblocks32, 256, 0, st>>>(ctx->d_integral.p, ctx->d_win.p, cnt + 0, G, ubase, ctx->d_feats.p, ctx->d_dims.p,

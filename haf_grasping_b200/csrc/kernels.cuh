@@ -17,6 +17,7 @@
 
 #include "decimal_round.cuh"
 #include "haf_host.hpp"
+#include "round4_table.hpp"
 
 namespace hafk {
 
@@ -569,20 +570,27 @@ __device__ __forceinline__ FastTab load_fast_tab(const DimFeat* __restrict__ tab
     f.fmin = __uint_as_float(t4.x); f.slope = __uint_as_float(t4.y); f.cval = __uint_as_float(t4.z);
     return f;
 }
-// same record from the copy the CTA staged in shared memory: five broadcast LDS.128 = five wavefronts, where the same
-// loads from global memory returned 16 B to each of 32 lanes = twenty (the kernel is bound by the LSU data pipe)
+// same record from the copy the CTA staged in shared memory: broadcast LDS.128 = one wavefront each, where the same
+// loads from global memory returned 16 B to each of 32 lanes = four (the kernel is bound by the LSU data pipe).  The
+// third region's offsets are loaded only when the record has one (flags & 0x4, 28 of 323 features): off[8..11] stay
+// unset otherwise.
+__device__ __forceinline__ uint4 lds_v4(uint32_t addr) {
+    uint4 t;
+    asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(t.x), "=r"(t.y), "=r"(t.z), "=r"(t.w) : "r"(addr));
+    return t;
+}
 __device__ __forceinline__ FastTab load_fast_tab_smem(uint32_t rec_addr) {
-    uint4 t[5];
-#pragma unroll
-    for (int k = 0; k < 5; k++)
-        asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(t[k].x), "=r"(t[k].y), "=r"(t[k].z), "=r"(t[k].w) : "r"(rec_addr + 16u * k));
+    const uint4 t0 = lds_v4(rec_addr), t1 = lds_v4(rec_addr + 16u), t3 = lds_v4(rec_addr + 48u), t4 = lds_v4(rec_addr + 64u);
     FastTab f;
-    f.off[0] = (int)t[0].x; f.off[1] = (int)t[0].y; f.off[2] = (int)t[0].z; f.off[3] = (int)t[0].w;
-    f.off[4] = (int)t[1].x; f.off[5] = (int)t[1].y; f.off[6] = (int)t[1].z; f.off[7] = (int)t[1].w;
-    f.off[8] = (int)t[2].x; f.off[9] = (int)t[2].y; f.off[10] = (int)t[2].z; f.off[11] = (int)t[2].w;
-    f.w[0] = __uint_as_float(t[3].x); f.w[1] = __uint_as_float(t[3].y); f.w[2] = __uint_as_float(t[3].z);
-    f.flags = (int)t[3].w;
-    f.fmin = __uint_as_float(t[4].x); f.slope = __uint_as_float(t[4].y); f.cval = __uint_as_float(t[4].z);
+    f.off[0] = (int)t0.x; f.off[1] = (int)t0.y; f.off[2] = (int)t0.z; f.off[3] = (int)t0.w;
+    f.off[4] = (int)t1.x; f.off[5] = (int)t1.y; f.off[6] = (int)t1.z; f.off[7] = (int)t1.w;
+    f.w[0] = __uint_as_float(t3.x); f.w[1] = __uint_as_float(t3.y); f.w[2] = __uint_as_float(t3.z);
+    f.flags = (int)t3.w;
+    f.fmin = __uint_as_float(t4.x); f.slope = __uint_as_float(t4.y); f.cval = __uint_as_float(t4.z);
+    if (f.flags & 0x4) {
+        const uint4 t2 = lds_v4(rec_addr + 32u);
+        f.off[8] = (int)t2.x; f.off[9] = (int)t2.y; f.off[10] = (int)t2.z; f.off[11] = (int)t2.w;
+    }
     return f;
 }
 struct SmemRows { uint32_t base; };  // 32-bit shared-window byte address of the staged integral rows
@@ -594,18 +602,13 @@ __device__ __forceinline__ float load_corner(SmemRows I, int idx0_bytes, int off
     asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(I.base + (uint32_t)(idx0_bytes + off_bytes)));
     return v;
 }
-// "%.4g" of the fast tier: powers of ten 10^(i-48) as double and float (built on the host, staged in shared memory by the
-// kernel -- as global loads they cost more LSU wavefronts than the instructions they saved).
-struct Round4Tab {
-    double pwd[96];
-    float pwf[96];
-};
-static_assert(sizeof(Round4Tab) == 96 * 8 + 96 * 4, "Round4Tab layout");
-struct Round4Smem { uint32_t pwd, pwf; };   // 32-bit shared-window addresses of the staged tables
-// idx0: element index of the window's patch origin for global rows, BYTE offset for staged rows; f.off[] are byte offsets
+// "%.4g" of the fast tier: the decision table of round4_table.hpp, staged in shared memory by the kernel (as global loads
+// its values cost more LSU wavefronts than the instructions they saved).  rt = its 32-bit shared-window address.
+// idx0: element index of the window's patch origin for global rows, BYTE offset for staged rows; f.off[] are byte offsets.
+// Constant (0x200) and dropped (0x400) columns never get here: the kernel writes them under a warp-uniform branch.
 template <typename PtrT>
 __device__ __forceinline__ float fast_tier_value(PtrT I, int idx0, const FastTab& f, float lower, int emulate_text,
-                                                 const Round4Smem rt) {
+                                                 const uint32_t rt) {
     float c[12];
 #pragma unroll
     for (int k = 0; k < 8; k++) c[k] = load_corner(I, idx0, f.off[k]);
@@ -633,22 +636,21 @@ __device__ __forceinline__ float fast_tier_value(PtrT I, int idx0, const FastTab
         // "%.4g": a * 10^(3-E) is formed and rounded in DOUBLE (exact ties stay exact; a mis-decided near-tie needs
         // |frac - 0.5| < 1e-12); everything after the rounding decision only needs float accuracy here.  Branch-free:
         // raw = +-0 runs through the subnormal record and comes out as +-0.
-        // E0 = floor(log10 2^k) = (k * 1233) >> 12 exactly for every float binade k in [-126, 127]; subnormals count as
-        // binade -126.  (a >= 10^(E0+1) as a float rounded to nearest: a value sitting exactly on a rounded-down power of
-        // ten is then scaled by one decade more and still rounds to the same four digits.)
+        // E = E0(b) + (a >= thr[b]) with b the biased exponent byte of raw (round4_table.hpp): one load of the threshold,
+        // then the two scale factors of (b, side).  (a >= 10^(E0+1) as a float rounded to nearest: a value sitting exactly
+        // on a rounded-down power of ten is then scaled by one decade more and still rounds to the same four digits.)
         const float a = fabsf(raw);
-        int E = ((max((int)(__float_as_uint(a) >> 23), 1) - 127) * 1233) >> 12;
+        const uint32_t b = (__float_as_uint(raw) >> 23) & 0xffu;
         float thr;
-        asm volatile("ld.shared.f32 %0, [%1];" : "=f"(thr) : "r"(rt.pwf + (uint32_t)((48 + E + 1) << 2)));
-        E += (a >= thr) ? 1 : 0;
+        asm volatile("ld.shared.f32 %0, [%1];" : "=f"(thr) : "r"(rt + (uint32_t)offsetof(Round4Tab, thr) + (b << 2)));
+        const uint32_t bs = 2u * b + ((a >= thr) ? 1u : 0u);
         double mul; float inv;
-        asm volatile("ld.shared.f64 %0, [%1];" : "=d"(mul) : "r"(rt.pwd + (uint32_t)((48 + 3 - E) << 3)));
-        asm volatile("ld.shared.f32 %0, [%1];" : "=f"(inv) : "r"(rt.pwf + (uint32_t)((48 + E - 3) << 2)));
+        asm volatile("ld.shared.f64 %0, [%1];" : "=d"(mul) : "r"(rt + (uint32_t)offsetof(Round4Tab, mul) + (bs << 3)));
+        asm volatile("ld.shared.f32 %0, [%1];" : "=f"(inv) : "r"(rt + (uint32_t)offsetof(Round4Tab, inv) + (bs << 2)));
         const float r = (float)rint((double)a * mul);
         v = copysignf(r * inv, raw);
     }
-    const float x = fmaf(v - f.fmin, f.slope, lower);  // svm-scale.c:344-346
-    return (f.flags & 0x400) ? 0.0f : ((f.flags & 0x200) ? f.cval : x);
+    return fmaf(v - f.fmin, f.slope, lower);  // svm-scale.c:344-346
 }
 
 // Tensor-core variant: per-dimension values split into two fp16 terms and written K-major in the k-block tiled layout
@@ -656,7 +658,7 @@ __device__ __forceinline__ float fast_tier_value(PtrT I, int idx0, const FastTab
 // 64-window x 96-dimension tile of (hi | lo << 16) words is staged in shared memory so that the global writes are whole
 // 32-byte sectors of the operand rows; the squared norm of the (hi + lo) representation is accumulated on the way.
 // The kernel is bound by the LSU data pipe and the issue rate together (DESIGN.md, "The feature kernel"): hence the
-// bank-conflict-free staging of the image rows, the per-pass copy of the table records and the power-of-ten tables in
+// bank-conflict-free staging of the image rows, the per-pass copy of the table records and the "%.4g" decision table in
 // shared memory, and the warp-uniform branches around the third region and the SHAF rule.
 //
 // FAST TIER.  The values written here are rounded to 22 significant bits (fp16 hi + lo) anyway and every window whose
@@ -694,11 +696,13 @@ __device__ __forceinline__ void write_aug_columns(__half* __restrict__ X, size_t
 __host__ __device__ constexpr size_t ft_smem_layout(int G, int tiles) {
     return sizeof(Round4Tab) + (size_t)tiles * 32 * HAF_FT_WT * HAF_FT_KPASS * 2 + (size_t)HAF_FT_ROWS * (G + 1 + 31) * 4 + 16 + (size_t)HAF_FT_KPASS * 96;
 }
+// LO: the fp16 lo terms are written too (Xl, three products); the one- and two-product builds write Xh only (Xl unused)
+template <bool LO>
 __global__ void __launch_bounds__(256, 4) features_tc_kernel(const float* __restrict__ integral, const int2* __restrict__ win,
                                                              const unsigned* __restrict__ win_count, int G, int unit_base,
                                                              const DimFeat* __restrict__ table, int D, int Krow, float lower,
                                                              int emulate_text, const Round4Tab* __restrict__ rtab,
-                                                             __half* __restrict__ Xh, __half* __restrict__ Xl /*NULL: hi only*/, float* __restrict__ xn,
+                                                             __half* __restrict__ Xh, __half* __restrict__ Xl, float* __restrict__ xn,
                                                              int aug0 /*first of the six extra operand columns (svm_tc.cuh)*/, int KB /*k-blocks of the tiled layout*/,
                                                              double* __restrict__ dec_acc, float* __restrict__ asum_acc /*the contraction's accumulators: zeroed here*/) {
     constexpr int WT = HAF_FT_WT, NW = 32 * WT;
@@ -708,13 +712,12 @@ __global__ void __launch_bounds__(256, 4) features_tc_kernel(const float* __rest
     // reads whole chunks with LDS.128 (16 lanes = the 16 chunks of a row, XOR-permuted = all banks) and writes them with
     // STG.128: 8 dimensions per instruction.  Round 1 kept (hi | lo << 16) words and wrote 2 dimensions per STG after two LDS
     // and a PRMT, with 64-bit kt_off arithmetic per word: a quarter of the kernel's instructions (ncu r2, source view).
-    // dynamic shared memory: the "%.4g" power-of-ten tables first (their addresses are then tile_base - constant: as a static
+    // dynamic shared memory: the "%.4g" decision table first (their addresses are then tile_base - constant: as a static
     // __shared__ object the compiler re-derived the address -- S2R CgaCtaId, MOV, VIADD, LEA -- for every value, ncu r2), then the
     // tile(s) [1 or 2][NW][KPASS] fp16, then float s_int[ROWS][ld .. ld + 31], then the pass's table records
     extern __shared__ __align__(16) uint32_t s_dyn[];
-    static_assert(sizeof(Round4Tab) % 16 == 0, "the tile behind the tables must stay 16-byte aligned");
     uint32_t* const s_words = s_dyn + sizeof(Round4Tab) / 4;
-    const int tiles = Xl ? 2 : 1;
+    constexpr int tiles = LO ? 2 : 1;
     constexpr int TILE_WORDS = NW * HAF_FT_KPASS / 2;
     const unsigned W = *win_count;
     const unsigned w0 = blockIdx.x * NW;
@@ -795,13 +798,11 @@ __global__ void __launch_bounds__(256, 4) features_tc_kernel(const float* __rest
             s_box[7] = cmin - 7; s_box[8] = cmax - cmin + 15;   // columns the patches touch: only these are copied
         }
     }
-    for (int t = threadIdx.x; t < (int)(sizeof(Round4Tab) / 8); t += blockDim.x)
-        reinterpret_cast<uint2*>(s_dyn)[t] = __ldg(reinterpret_cast<const uint2*>(rtab) + t);
+    for (int t = threadIdx.x; t < (int)(sizeof(Round4Tab) / 16); t += blockDim.x)
+        reinterpret_cast<uint4*>(s_dyn)[t] = __ldg(reinterpret_cast<const uint4*>(rtab) + t);
     __syncthreads();
-    Round4Smem rt;
-    rt.pwd = (uint32_t)__cvta_generic_to_shared(s_dyn);                                                  // Round4Tab::pwd at offset 0
-    asm volatile("" : "+r"(rt.pwd));   // opaque: keep the base in a register instead of re-deriving it (S2R CgaCtaId, MOV, VIADD, LEA) per value
-    rt.pwf = rt.pwd + (uint32_t)(96 * sizeof(double));                                                   // Round4Tab::pwf behind it
+    uint32_t rt = (uint32_t)__cvta_generic_to_shared(s_dyn);
+    asm volatile("" : "+r"(rt));   // opaque: keep the base in a register instead of re-deriving it (S2R CgaCtaId, MOV, VIADD, LEA) per value
     const int nrows = s_box[2];
     const int sst = nrows > 0 ? s_box[3] : ld;           // row stride the corner offsets must be built for
     table += (size_t)(sst - ld) * D;                      // stride class
@@ -835,31 +836,42 @@ __global__ void __launch_bounds__(256, 4) features_tc_kernel(const float* __rest
     float nrm[WT];  // squared-norm partials of this lane's windows over the dimensions this warp evaluates
 #pragma unroll
     for (int t = 0; t < WT; t++) nrm[t] = 0.0f;
-    const uint32_t tile_base = rt.pwd + (uint32_t)sizeof(Round4Tab);
+    const uint32_t tile_base = rt + (uint32_t)sizeof(Round4Tab);
     const uint32_t row0 = tile_base + (uint32_t)lane * (HAF_FT_KPASS * 2), row1 = row0 + 32u * (HAF_FT_KPASS * 2);   // windows lane, 32 + lane
     const uint32_t sw = (uint32_t)(((lane & 7) << 2) | ((lane >> 3) & 3));   // swizzle of this lane's two rows (same low five bits)
+    // tile entries of dimension dl: fp16 pairs (low half: window lane, high half: window 32 + lane) of the hi and lo terms
+    auto put = [&](int dl, uint32_t hu, uint32_t lu) {
+        // swizzled byte offset of dimension dl inside a tile row (see TILE above)
+        const uint32_t toff = ((((uint32_t)dl >> 1) ^ sw) << 2) | (((uint32_t)dl & 1u) << 1);
+        asm volatile("st.shared.b16 [%0], %1;" ::"r"(row0 + toff), "h"((unsigned short)(hu & 0xffffu)) : "memory");
+        asm volatile("st.shared.b16 [%0], %1;" ::"r"(row1 + toff), "h"((unsigned short)(hu >> 16)) : "memory");
+        if (LO) {
+            asm volatile("st.shared.b16 [%0], %1;" ::"r"(row0 + TILE_WORDS * 4 + toff), "h"((unsigned short)(lu & 0xffffu)) : "memory");
+            asm volatile("st.shared.b16 [%0], %1;" ::"r"(row1 + TILE_WORDS * 4 + toff), "h"((unsigned short)(lu >> 16)) : "memory");
+        }
+    };
     for (int d0 = 0; d0 < Krow; d0 += HAF_FT_KPASS) {
         const int KP = min(HAF_FT_KPASS, Krow - d0);   // a multiple of 16
+        const int KD = max(0, min(KP, D - d0));        // dimensions of the pass that carry values; KD .. KP - 1 pad the row
         {   // this pass's records of the stride class, coalesced
-            const int nrec = min(KP, D - d0);
             const uint4* src = reinterpret_cast<const uint4*>(table + d0);
-            for (int t = threadIdx.x; t < nrec * 6; t += blockDim.x) s_tab[t] = __ldg(src + t);
+            for (int t = threadIdx.x; t < KD * 6; t += blockDim.x) s_tab[t] = __ldg(src + t);
         }
         __syncthreads();
-        for (int dl = warp; dl < KP; dl += 8) {
-            const int d = d0 + dl;
+        int dl = warp;
+        for (; dl < KD; dl += 8) {
+            const FastTab f = load_fast_tab_smem(tab_base + 96u * dl);
             float xf[WT];
+            if (f.flags & 0x600) {   // constant (0x200) or dropped (0x400) column: warp-uniform, no image reads
+                const float c = (f.flags & 0x400) ? 0.0f : f.cval;
 #pragma unroll
-            for (int t = 0; t < WT; t++) xf[t] = 0.0f;
-            if (d < D) {
-                const FastTab f = load_fast_tab_smem(tab_base + 96u * dl);
-                if (nrows > 0) {
+                for (int t = 0; t < WT; t++) xf[t] = (nrows > 0 || valid[t]) ? c : 0.0f;
+            } else if (nrows > 0) {
 #pragma unroll
-                    for (int t = 0; t < WT; t++) xf[t] = fast_tier_value(srows, idx0[t] * 4, f, lower, emulate_text, rt);
-                } else {
+                for (int t = 0; t < WT; t++) xf[t] = fast_tier_value(srows, idx0[t] * 4, f, lower, emulate_text, rt);
+            } else {
 #pragma unroll
-                    for (int t = 0; t < WT; t++) xf[t] = valid[t] ? fast_tier_value(gI[t], idx0[t], f, lower, emulate_text, rt) : 0.0f;
-                }
+                for (int t = 0; t < WT; t++) xf[t] = valid[t] ? fast_tier_value(gI[t], idx0[t], f, lower, emulate_text, rt) : 0.0f;
             }
             // fp16 hi + fp16 lo = 22 significant bits (absolute floor 2^-25 once lo is subnormal), two windows per conversion.
             // A value beyond the fp16 range becomes hi = +-inf, lo = -+inf: the NaN / inf it produces stays inside this
@@ -874,16 +886,9 @@ __global__ void __launch_bounds__(256, 4) features_tc_kernel(const float* __rest
                 nrm[0] = fmaf(v0, v0, nrm[0]);
                 nrm[1] = fmaf(v1, v1, nrm[1]);
             }
-            const uint32_t hu = *reinterpret_cast<const uint32_t*>(&hi2), lu = *reinterpret_cast<const uint32_t*>(&lo2);
-            // swizzled byte offset of dimension dl inside a tile row (see TILE above)
-            const uint32_t toff = ((((uint32_t)dl >> 1) ^ sw) << 2) | (((uint32_t)dl & 1u) << 1);
-            asm volatile("st.shared.b16 [%0], %1;" ::"r"(row0 + toff), "h"((unsigned short)(hu & 0xffffu)) : "memory");
-            asm volatile("st.shared.b16 [%0], %1;" ::"r"(row1 + toff), "h"((unsigned short)(hu >> 16)) : "memory");
-            if (Xl) {   // three products only
-                asm volatile("st.shared.b16 [%0], %1;" ::"r"(row0 + TILE_WORDS * 4 + toff), "h"((unsigned short)(lu & 0xffffu)) : "memory");
-                asm volatile("st.shared.b16 [%0], %1;" ::"r"(row1 + TILE_WORDS * 4 + toff), "h"((unsigned short)(lu >> 16)) : "memory");
-            }
+            put(dl, *reinterpret_cast<const uint32_t*>(&hi2), *reinterpret_cast<const uint32_t*>(&lo2));
         }
+        for (; dl < KP; dl += 8) put(dl, 0u, 0u);   // padding columns: +0 (adds nothing to the norms)
         __syncthreads();
         {   // write-out: lane = (window of a pair, chunk): 16 lanes x 16 bytes = two whole 128-byte k-block rows of one window
             const int c = lane & 15, nch = KP >> 3;
@@ -899,7 +904,7 @@ __global__ void __launch_bounds__(256, 4) features_tc_kernel(const float* __rest
                     const int kx = (wi >> 3) & 3;   // the row's word permutation: stored word q ^ kx holds dimensions 2q, 2q + 1
 #pragma unroll
                     for (int tl = 0; tl < 2; tl++) {
-                        if (tl == 1 && !Xl) break;
+                        if (tl == 1 && !LO) break;
                         uint4 v;
                         asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a + tl * TILE_WORDS * 4));
                         if (kx & 1) { uint32_t t0 = v.x; v.x = v.y; v.y = t0; t0 = v.z; v.z = v.w; v.w = t0; }
